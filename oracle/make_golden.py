@@ -23,6 +23,7 @@ sys.path.insert(0, ROOT)
 from oracle import ref_harness as RH  # noqa: E402
 from oracle import restate as R  # noqa: E402
 from oracle import weights as W  # noqa: E402
+from oracle.golden import sample_flat  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
 
@@ -174,11 +175,12 @@ def gen_vae_enc(name, ddconfig, B, res, seed):
     save(name + ".pt", out)
 
 
-def gen_sd_traj(name="sd_traj", steps_kept=(0, 12, 25, 37, 49)):
+def gen_sd_traj(name="sd_traj", steps_kept=(0, 12, 25, 37, 49), img_samples=32768):
     """BASELINE config C2 at its own size: the UNMODIFIED reference UNetModel (SD-1.x kwargs) driven by the reference
     DDIMSampler (DDIM/ddim.py) for a full DDIM-50 run at B=1, 64x64x4 latent, 77x768 context, then the reference ldm
     Decoder on z / 0.18215 (ldm/diffusion/ddpm.py:1095) -> 3x512x512.  Stored: (x_t, t, e_t) at five steps of the
-    reference trajectory (teacher-forced eps checks), the final latent and the decoded image (PSNR check).
+    reference trajectory (teacher-forced eps checks), the final latent and the decoded image (PSNR check) as its values
+    at `img_samples` fixed positions (oracle/golden.py sample_index), which keeps the fixture under 1 MB.
     UNet weights = seed 31 (same as unet_sd.pt), VAE weights = seed 51 (same as vae_sd_z16.pt)."""
     import contextlib
     import io
@@ -232,12 +234,14 @@ def gen_sd_traj(name="sd_traj", steps_kept=(0, 12, 25, 37, 49)):
     assert err_img < 2e-5, err_img
     save(name + ".pt", dict(cfg=cfg, ddconfig=R.SD_VAE_DDCONFIG, unet_seed=31, vae_seed=51, unet_key_shapes=ks_u, vae_key_shapes=ks_v,
                             x_T_seed=2, ctx_seed=3, steps=kept, all_t=[r[1] for r in rec], z_ref=z_ref.clone(),
-                            img_ref=img_ref.clone(), restate_err=worst, restate_err_img=err_img, ref_seconds=t_traj))
+                            img_shape=tuple(img_ref.shape), img_ref_s=sample_flat(img_ref, img_samples),
+                            restate_err=worst, restate_err_img=err_img, ref_seconds=t_traj))
 
 
-def gen_vae_full(name="vae_sd_z64"):
+def gen_vae_full(name="vae_sd_z64", img_samples=65536):
     """BASELINE config C3 at its own size (B=1): the reference ldm Decoder on a 64x64x4 latent -> 3x512x512.
-    `img_f64` is the float64 restatement rounded to fp32 for storage (3e-8 relative, against a 1e-5 bound)."""
+    `img_f64` is the float64 restatement rounded to fp32 for storage (3e-8 relative, against a 1e-5 bound).  Both images
+    are stored as their values at `img_samples` fixed positions (oracle/golden.py sample_index: `img_ref_s`, `img_f64_s`)."""
     ddconfig = R.SD_VAE_DDCONFIG
     dec = RH.build_decoder(ddconfig)
     ks = [("decoder." + k, s) for k, s in W.key_shapes_of(dec)] + [("post_quant_conv.weight", (4, 4, 1, 1)), ("post_quant_conv.bias", (4,))]
@@ -253,8 +257,9 @@ def gen_vae_full(name="vae_sd_z64"):
     print("%s: restatement vs reference rel-L2 = %.3e (img std %.3f); fp32 reference vs f64 %.3e"
           % (name, err, float(img_ref.std()), R.rel_l2(img_ref, img64)))
     assert err < 2e-5, err
-    save(name + ".pt", dict(ddconfig=ddconfig, seed=51, z_seed=4, key_shapes=ks, z_shape=(1, 4, 64, 64), img_ref=img_ref.clone(),
-                            img_f64=img64.float().clone(), restate_err=err))
+    save(name + ".pt", dict(ddconfig=ddconfig, seed=51, z_seed=4, key_shapes=ks, z_shape=(1, 4, 64, 64), img_shape=tuple(img_ref.shape),
+                            img_ref_s=sample_flat(img_ref, img_samples), img_f64_s=sample_flat(img64.float(), img_samples),
+                            restate_err=err))
 
 
 def gen_unet_96(name="unet_sd_96"):

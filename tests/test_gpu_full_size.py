@@ -11,7 +11,7 @@ import torch
 from gpu_util import rel
 from oracle import restate as R
 from oracle import weights as W
-from oracle.golden import load_golden
+from oracle.golden import load_golden, sample_flat
 
 pytestmark = pytest.mark.gpu
 
@@ -109,8 +109,10 @@ def test_c2_free_running_ddim50_image_psnr_vs_reference(cuda, mode):
     x_T = W.seeded_randn((1, 4, 64, 64), g["x_T_seed"]).cuda()
     ctx = W.seeded_randn((1, 77, 768), g["ctx_seed"]).cuda()
     z, img = ld.txt2img(ctx, 1, ddim_steps=50, shape=(4, 64, 64), x_T=x_T)
-    psnr = R.psnr_255(img.cpu(), g["img_ref"])
-    ez, ei = rel(z, g["z_ref"]), rel(img, g["img_ref"])
+    assert tuple(img.shape) == tuple(g["img_shape"])
+    img = sample_flat(img, g["img_ref_s"].numel())          # the fixture stores the reference image at these positions
+    psnr = R.psnr_255(img, g["img_ref_s"])
+    ez, ei = rel(z, g["z_ref"]), rel(img, g["img_ref_s"])
     print("C2 free-running DDIM-50 + decode vs reference, %s mode: latent rel-L2 %.3e, image rel-L2 %.3e, PSNR %.1f dB" % (mode, ez, ei, psnr))
     assert psnr >= 40.0
     if mode == "fp32":
@@ -128,12 +130,14 @@ def test_c3_vae_decode_512_vs_reference(cuda):
     vae = vae.cuda()
     z = W.seeded_randn(g["z_shape"], g["z_seed"]).cuda()
     img32 = vae.decode(z)
-    e64, eref = rel(img32, g["img_f64"]), rel(img32, g["img_ref"])
+    assert tuple(img32.shape) == tuple(g["img_shape"])
+    n = g["img_ref_s"].numel()                              # the fixture stores both images at these positions
+    e64, eref = rel(sample_flat(img32, n), g["img_f64_s"]), rel(sample_flat(img32, n), g["img_ref_s"])
     vae.compute_mode = "bf16"
     img16 = vae.decode(z)
-    psnr = R.psnr_255(img16.cpu(), g["img_ref"])
+    psnr = R.psnr_255(sample_flat(img16, n), g["img_ref_s"])
     print("C3 decode 512x512 vs reference: fp32 mode rel-L2 %.3e (vs f64 %.3e), bf16 mode rel-L2 %.3e, PSNR %.1f dB"
-          % (eref, e64, rel(img16, g["img_ref"]), psnr))
+          % (eref, e64, rel(sample_flat(img16, n), g["img_ref_s"]), psnr))
     assert e64 <= 1e-5 and eref <= 1e-5
     assert psnr >= 40.0
     img_b = vae.decode(z.repeat(16, 1, 1, 1))

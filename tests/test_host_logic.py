@@ -197,6 +197,29 @@ def test_bench_reference_arm_line(monkeypatch, capsys):
     assert capsys.readouterr().out.strip() == ""
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float32 .npy per output, whole while they fit the size limit; above it, each output is
+    replaced by the same share of its values at fixed, distinct positions."""
+    import sys
+    import bench
+    from oracle.golden import sample_flat, sample_index
+    z, img = torch.randn(2, 4, 8, 8), torch.randn(2, 3, 16, 16, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "whole"), {"latents": z, "images": img})
+    got = np.load(tmp_path / "whole" / "images.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, img.float().numpy())
+    assert np.array_equal(np.load(tmp_path / "whole" / "latents.npy"), z.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1024)          # 8 KB of outputs -> an eighth of each
+    bench.dump_outputs(str(tmp_path / "sampled"), {"latents": z, "images": img})
+    lat, ims = np.load(tmp_path / "sampled" / "latents.npy"), np.load(tmp_path / "sampled" / "images.npy")
+    assert lat.shape == (64,) and ims.shape == (192,) and (lat.nbytes + ims.nbytes) <= 1024
+    assert np.array_equal(lat, sample_flat(z, 64).numpy()) and np.array_equal(ims, sample_flat(img.float(), 192).numpy())
+    assert sample_index(3 * 512 * 512, 65536).unique().numel() == 65536
+    for argv in (["--config", "c3"], ["--impl", "reference"], ["--steps", "0"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--dump-outputs", str(tmp_path / "x")] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
+
+
 def _tiny_unet():
     from sdb200.openai_model import UNetModel
     return UNetModel(image_size=8, in_channels=4, model_channels=32, out_channels=4, num_res_blocks=1, attention_resolutions=[1],

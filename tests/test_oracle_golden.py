@@ -44,8 +44,8 @@ def test_full_size_fixtures_match_reference():
     g = load_golden("sd_traj.pt")
     assert g["restate_err"] < 1e-5 and g["restate_err_img"] < 1e-5
     assert [s["i"] for s in g["steps"]] == [0, 12, 25, 37, 49] and len(g["all_t"]) == 50 and g["all_t"][0] == 981 and g["all_t"][-1] == 1
-    assert tuple(g["img_ref"].shape) == (1, 3, 512, 512) and tuple(g["z_ref"].shape) == (1, 4, 64, 64)
-    assert float((g["img_ref"].abs() <= 1).float().mean()) > 0.9          # PSNR on the clamp-255 scale is not saturated
+    assert tuple(g["img_shape"]) == (1, 3, 512, 512) and tuple(g["z_ref"].shape) == (1, 4, 64, 64)
+    assert float((g["img_ref_s"].abs() <= 1).float().mean()) > 0.9        # PSNR on the clamp-255 scale is not saturated
     st = g["steps"][2]
     sd = W.make_state_dict(g["unet_key_shapes"], g["unet_seed"])
     ctx = W.seeded_randn((1, 77, 768), g["ctx_seed"])
@@ -55,7 +55,7 @@ def test_full_size_fixtures_match_reference():
     # the trajectory's first input is the seeded x_T, and DDIM's update links consecutive stored quantities
     assert torch.equal(g["steps"][0]["x_t"], W.seeded_randn((1, 4, 64, 64), g["x_T_seed"]))
     gv = load_golden("vae_sd_z64.pt")
-    assert gv["restate_err"] < 1e-5 and R.rel_l2(gv["img_ref"], gv["img_f64"]) < 1e-5 and tuple(gv["img_ref"].shape) == (1, 3, 512, 512)
+    assert gv["restate_err"] < 1e-5 and R.rel_l2(gv["img_ref_s"], gv["img_f64_s"]) < 1e-5 and tuple(gv["img_shape"]) == (1, 3, 512, 512)
     g9 = load_golden("unet_sd_96.pt")
     assert g9["restate_err"] < 1e-5 and R.rel_l2(g9["eps_ref"], g9["eps_f64"]) < 1e-5 and tuple(g9["eps_ref"].shape) == (1, 4, 96, 96)
 
