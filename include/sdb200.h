@@ -172,6 +172,22 @@ int sdb_ddim_step(const float* x, const float* e_cond, const float* e_uncond, fl
  * (the caller replaced it by first_stage_model.quantize(pred_x0)), x_prev = sqrt_aprev*pred_x0 + dir_coef*e + sigma_t*noise*temperature. */
 int sdb_ddim_xprev(const float* pred_x0, const float* e_cond, const float* e_uncond, float cfg_scale, const float* noise,
                    float sqrt_aprev, float dir_coef, float sigma_t, float temperature, float* x_prev, long long n, void* stream);
+/* ---- ancestral (DDPM) update ---------------------------------------------------------------
+ * Replaces LatentDiffusion.p_sample's arithmetic (ldm/diffusion/ddpm.py:1528-1793: predict_start_from_noise,
+ * x_recon.clamp_, q_posterior, `model_mean + nonzero_mask * (0.5 * model_log_variance).exp() * noise`):
+ *   x0     = x0_in != NULL ? x0_in : sqrt_recip[t]*x - sqrt_recipm1[t]*eps
+ *   x0     = clip ? clamp(x0, -1, 1) : x0                  (NaN passes through, like torch.clamp)
+ *   mean   = coef1[t]*x0 + coef2[t]*x
+ *   x_prev = noise != NULL ? mean + ((t != 0) * std[t]) * (noise*temperature) : mean
+ * all fp32, every operation individually rounded (no FMA contraction) in the reference's order.
+ * x / eps / x0_in / noise / x_prev / x0_out [B, per] fp32; t: device int64 [B]; table: device fp32 [5, T] with rows
+ * sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod, posterior_mean_coef1, posterior_mean_coef2 and
+ * posterior_std = exp(0.5 * posterior_log_variance_clipped), gathered per sample inside the kernel.  eps may be NULL
+ * when x0_in is given; x_prev and x0_out are each optional, not both (x0_out only: predict_start_from_noise; no noise:
+ * the posterior mean).  A t[b] outside [0, T) writes NaN into sample b and is never used as an index. */
+int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const float* noise, const long long* t,
+                  const float* table, int T, int clip, float temperature, float* x_prev, float* x0_out, int B, long long per,
+                  void* stream);
 /* Inpainting blend of ddim_sampling (ldm/diffusion/ddim.py:144-149) fused with LatentDiffusion.q_sample
  * (ldm/diffusion/ddpm.py:407-412): img_orig = a[b]*x0 + c[b]*noise; out = img_orig*mask + (1 - mask)*img.
  * x0 / noise / img / out [B,C,HW] fp32, mask [B,Cm,HW] with Cm == 1 (broadcast over channels) or Cm == C; a / c: B per-sample

@@ -350,6 +350,70 @@ ddim_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, con
     }
 }
 
+// ---- ancestral (DDPM) update of LatentDiffusion.p_sample (ldm/diffusion/ddpm.py:1528-1793) -----------------------
+//   x0   = x0_in given ? x0_in : sqrt_recip[t]*x - sqrt_recipm1[t]*eps     (predict_start_from_noise)
+//   x0   = clip ? clamp(x0, -1, 1) : x0                                     (x_recon.clamp_, NaN passes through)
+//   mean = coef1[t]*x0 + coef2[t]*x                                          (q_posterior)
+//   out  = noise ? mean + ((t != 0) * std[t]) * (noise * temperature) : mean
+// Separately rounded fp32 operations in the reference's order.  The per-sample coefficients are gathered from the
+// [5, T] device table by t[b]; a t outside [0, T) makes that sample NaN and is never used as an index.
+__device__ __forceinline__ void ddpm_update_1(float xv, float e, float x0v, bool x0_given, bool clip, bool has_nz, float nzv,
+                                              float sr, float srm1, float c1, float c2, float s, float temperature,
+                                              float& x0, float& xp) {
+    x0 = x0_given ? x0v : __fsub_rn(__fmul_rn(sr, xv), __fmul_rn(srm1, e));
+    if (clip) x0 = x0 < -1.f ? -1.f : (x0 > 1.f ? 1.f : x0);
+    const float mean = __fadd_rn(__fmul_rn(c1, x0), __fmul_rn(c2, xv));
+    xp = has_nz ? __fadd_rn(mean, __fmul_rn(s, __fmul_rn(nzv, temperature))) : mean;
+}
+
+// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, per % 4 == 0, so a vector never straddles two
+// samples), VEC = 1: any alignment.  x_prev / x0_out may each be NULL (not both).
+template <int VEC>
+__global__ void __launch_bounds__(256)
+ddpm_step_kernel(const float* __restrict__ x, const float* __restrict__ eps, const float* __restrict__ x0_in,
+                 const float* __restrict__ noise, const long long* __restrict__ t, const float* __restrict__ table, int T,
+                 int clip, float temperature, float* __restrict__ x_prev, float* __restrict__ x0_out, long long per, long long n) {
+    pdl_trigger();
+    pdl_wait();
+    const long long nv = n / VEC, pv = per / VEC;
+    const bool xg = x0_in != nullptr, cl = clip != 0, hn = noise != nullptr;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+        const long long tb = __ldg(t + i / pv);
+        const bool ok = tb >= 0 && tb < T;
+        const float qnan = __int_as_float(0x7fc00000);
+        float sr = qnan, srm1 = qnan, c1 = qnan, c2 = qnan, s = qnan;
+        if (ok) {
+            sr = __ldg(table + tb);
+            srm1 = __ldg(table + T + tb);
+            c1 = __ldg(table + 2 * (long long)T + tb);
+            c2 = __ldg(table + 3 * (long long)T + tb);
+            s = __fmul_rn(tb != 0 ? 1.f : 0.f, __ldg(table + 4 * (long long)T + tb));   // nonzero_mask * std
+        }
+        if (VEC == 4) {
+            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+            const float4 x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
+            const float4 e4 = xg ? zero : __ldg(reinterpret_cast<const float4*>(eps) + i);
+            const float4 g4 = xg ? __ldg(reinterpret_cast<const float4*>(x0_in) + i) : zero;
+            const float4 n4 = hn ? __ldg(reinterpret_cast<const float4*>(noise) + i) : zero;
+            float4 p4, o4;
+            ddpm_update_1(x4.x, e4.x, g4.x, xg, cl, hn, n4.x, sr, srm1, c1, c2, s, temperature, p4.x, o4.x);
+            ddpm_update_1(x4.y, e4.y, g4.y, xg, cl, hn, n4.y, sr, srm1, c1, c2, s, temperature, p4.y, o4.y);
+            ddpm_update_1(x4.z, e4.z, g4.z, xg, cl, hn, n4.z, sr, srm1, c1, c2, s, temperature, p4.z, o4.z);
+            ddpm_update_1(x4.w, e4.w, g4.w, xg, cl, hn, n4.w, sr, srm1, c1, c2, s, temperature, p4.w, o4.w);
+            if (!ok) p4 = o4 = make_float4(qnan, qnan, qnan, qnan);
+            if (x_prev) reinterpret_cast<float4*>(x_prev)[i] = o4;
+            if (x0_out) reinterpret_cast<float4*>(x0_out)[i] = p4;
+        } else {
+            float p0, xp;
+            ddpm_update_1(x[i], xg ? 0.f : eps[i], xg ? x0_in[i] : 0.f, xg, cl, hn, hn ? noise[i] : 0.f, sr, srm1, c1, c2, s,
+                          temperature, p0, xp);
+            if (!ok) p0 = xp = qnan;
+            if (x_prev) x_prev[i] = xp;
+            if (x0_out) x0_out[i] = p0;
+        }
+    }
+}
+
 // ---- inpainting blend of ddim_sampling (ldm/diffusion/ddim.py:144-149) with q_sample (ldm/diffusion/ddpm.py:407-412) fused:
 //   img_orig = a[b] * x0 + c[b] * noise;   out = img_orig * mask + (1 - mask) * img
 // mask [B, Cm, HW] with Cm in {1, C} (broadcast over channels); separately rounded fp32 operations like the eager reference.
@@ -673,6 +737,26 @@ int sdb_ddim_xprev(const float* pred_x0, const float* e_cond, const float* e_unc
     SDB_REQUIRE(noise || sigma_t == 0.0f, "ddim_xprev: sigma_t != 0 needs a noise tensor");
     return launch_ddim(nullptr, e_cond, e_uncond, cfg_scale, noise, pred_x0, 1.0f, sqrt_aprev, dir_coef, sigma_t, 0.0f,
                        temperature, x_prev, nullptr, n, stream);
+}
+
+int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const float* noise, const long long* t,
+                  const float* table, int T, int clip, float temperature, float* x_prev, float* x0_out, int B, long long per,
+                  void* stream) {
+    SDB_REQUIRE(x && t && table, "ddpm_step: null pointer");
+    SDB_REQUIRE(eps || x0_in, "ddpm_step: needs eps or a given x0");
+    SDB_REQUIRE(x_prev || x0_out, "ddpm_step: no output requested");
+    SDB_REQUIRE(T > 0 && B > 0 && per > 0, "ddpm_step: bad shape B=%d per=%lld T=%d", B, per, T);
+    const long long n = (long long)B * per;
+    const uintptr_t al = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(eps) | reinterpret_cast<uintptr_t>(x0_in) |
+                         reinterpret_cast<uintptr_t>(noise) | reinterpret_cast<uintptr_t>(x_prev) | reinterpret_cast<uintptr_t>(x0_out);
+    if ((al & 15) == 0 && per % 4 == 0) {
+        launch_pdl(ddpm_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream,
+            x, eps, x0_in, noise, t, table, T, clip, temperature, x_prev, x0_out, per, n);
+    } else {
+        launch_pdl(ddpm_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream,
+            x, eps, x0_in, noise, t, table, T, clip, temperature, x_prev, x0_out, per, n);
+    }
+    return check_launch("ddpm_step_kernel");
 }
 
 int sdb_inpaint_blend(const float* x0, const float* noise, const float* a, const float* c, const float* mask, const float* img,

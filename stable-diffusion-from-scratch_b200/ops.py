@@ -293,6 +293,29 @@ def ddim_xprev(pred_x0, e_cond, sqrt_aprev, dir_coef, sigma_t, e_uncond=None, cf
     return x_prev
 
 
+def ddpm_step(x, t, table, eps=None, x0=None, noise=None, clip=False, temperature=1.0, want_x_prev=True, want_x0=False):
+    """One fused ancestral update (LatentDiffusion.p_sample arithmetic, see include/sdb200.h sdb_ddpm_step).
+    x / eps / x0 / noise: contiguous fp32 [B, ...] with x's element count; t: int64 [B] on the device; table: fp32 [5, T]
+    (LatentDiffusion.ddpm_table).  x0 given replaces predict_start_from_noise (eps is then unused).  noise None: x_prev is
+    the posterior mean.  Returns (x_prev or None, x0 or None)."""
+    require_cuda(x, t, table, eps, x0, noise)
+    _f32c("x", x)
+    _f32c("eps", eps, x)
+    _f32c("x0", x0, x)
+    _f32c("noise", noise, x)
+    _f32c("table", table)
+    B = x.shape[0]
+    if t.dtype != torch.int64 or t.numel() != B or not t.is_contiguous():
+        raise _lib.SdbError("t must be a contiguous int64 tensor of %d timesteps (got %s %s)" % (B, t.dtype, tuple(t.shape)))
+    if table.dim() != 2 or table.shape[0] != 5:
+        raise _lib.SdbError("table must be [5, T] (got %s)" % (tuple(table.shape),))
+    x_prev = torch.empty_like(x) if want_x_prev else None
+    x0_out = torch.empty_like(x) if want_x0 else None
+    check(_L().sdb_ddpm_step(ptr(x), ptr(eps), ptr(x0), ptr(noise), ptr(t), ptr(table), table.shape[1], int(bool(clip)),
+                             float(temperature), ptr(x_prev), ptr(x0_out), B, x.numel() // B if B else 0, stream_ptr()), "ddpm_step")
+    return x_prev, x0_out
+
+
 def inpaint_blend(x0, noise, a, c, mask, img):
     """(a[b]*x0 + c[b]*noise) * mask + (1 - mask) * img: q_sample + the mask blend of ddim_sampling in one kernel
     (ldm/diffusion/ddim.py:144-149, ldm/diffusion/ddpm.py:407-412).  x0 / noise / img [B,C,H,W]; mask [B,1,H,W] or [B,C,H,W]."""

@@ -4,11 +4,16 @@
 `decode_first_stage` call sites need (ldm/diffusion/ddpm.py:1326-1448, 1083-1156, 1814-1826):
 schedule buffers, `apply_model(x, t, cond)`, `decode_first_stage(z)`.  It owns a `UNetModel`
 (as `model.diffusion_model`, like DiffusionWrapper, ddpm.py:1992-2034) and an `AutoencoderKL`.
+It also carries the reference's ancestral sampler (`sample` / `p_sample_loop` / `progressive_denoising`,
+ddpm.py:1528-1793), whose per-step update runs as one fused kernel (sdb_ddpm_step).
 """
+import weakref
+
 import numpy as np
 import torch
 from torch import nn
 
+from . import ops
 from .autoencoder import AutoencoderKL
 from .ddim import DDIMSampler
 from .openai_model import UNetModel
@@ -54,7 +59,8 @@ class DiffusionWrapper(nn.Module):
 class LatentDiffusion(nn.Module):
     def __init__(self, unet_config=None, first_stage_config=None, timesteps=1000, linear_start=0.00085, linear_end=0.0120,
                  beta_schedule="linear", scale_factor=0.18215, conditioning_key="crossattn", compute_mode=None,
-                 unet=None, first_stage_model=None, cond_stage_model=None):
+                 unet=None, first_stage_model=None, cond_stage_model=None, v_posterior=0., clip_denoised=True,
+                 log_every_t=100, channels=4, image_size=64):
         super().__init__()
         # optional text conditioner (Diffusion/config.yaml:69-70: FrozenCLIPEmbedder); None = the caller supplies `context` tensors
         self.cond_stage_model = cond_stage_model
@@ -65,6 +71,12 @@ class LatentDiffusion(nn.Module):
         self.first_stage_model = first_stage_model
         self.scale_factor = scale_factor
         self.parameterization = "eps"
+        self.shorten_cond_schedule = False
+        self.v_posterior = v_posterior
+        self.clip_denoised = clip_denoised
+        self.log_every_t = log_every_t
+        self.channels = channels
+        self.image_size = image_size
         self.num_timesteps = int(timesteps)
         betas = make_beta_schedule(beta_schedule, timesteps, linear_start=linear_start, linear_end=linear_end)
         alphas_cumprod = np.cumprod(1. - betas, axis=0)
@@ -75,6 +87,16 @@ class LatentDiffusion(nn.Module):
         self.register_buffer("alphas_cumprod_prev", to_t(alphas_cumprod_prev))
         self.register_buffer("sqrt_alphas_cumprod", to_t(np.sqrt(alphas_cumprod)))           # ldm/diffusion/ddpm.py:212-213
         self.register_buffer("sqrt_one_minus_alphas_cumprod", to_t(np.sqrt(1. - alphas_cumprod)))
+        # the rest of register_schedule (ddpm.py DDPM.register_schedule), float64 numpy cast to fp32, the reference's expressions
+        alphas = 1. - betas
+        self.register_buffer("log_one_minus_alphas_cumprod", to_t(np.log(1. - alphas_cumprod)))
+        self.register_buffer("sqrt_recip_alphas_cumprod", to_t(np.sqrt(1. / alphas_cumprod)))
+        self.register_buffer("sqrt_recipm1_alphas_cumprod", to_t(np.sqrt(1. / alphas_cumprod - 1)))
+        posterior_variance = (1 - self.v_posterior) * betas * (1. - alphas_cumprod_prev) / (1. - alphas_cumprod) + self.v_posterior * betas
+        self.register_buffer("posterior_variance", to_t(posterior_variance))
+        self.register_buffer("posterior_log_variance_clipped", to_t(np.log(np.maximum(posterior_variance, 1e-20))))
+        self.register_buffer("posterior_mean_coef1", to_t(betas * np.sqrt(alphas_cumprod_prev) / (1. - alphas_cumprod)))
+        self.register_buffer("posterior_mean_coef2", to_t((1. - alphas_cumprod_prev) * np.sqrt(alphas) / (1. - alphas_cumprod)))
 
     @property
     def device(self):
@@ -155,8 +177,9 @@ class LatentDiffusion(nn.Module):
 
     @torch.no_grad()
     def sample_log(self, cond, batch_size, ddim=True, ddim_steps=50, shape=(4, 64, 64), **kwargs):
-        """ldm/diffusion/ddpm.py:1814-1826 (DDIM branch)."""
-        assert ddim, "only the DDIM branch is on the hot path"
+        """ldm/diffusion/ddpm.py:1814-1826: DDIM-`ddim_steps`, or (ddim=False) the ancestral sampler with intermediates."""
+        if not ddim:
+            return self.sample(cond=cond, batch_size=batch_size, return_intermediates=True, shape=(batch_size, *shape), **kwargs)
         sampler = DDIMSampler(self)
         return sampler.sample(ddim_steps, batch_size, shape, cond, verbose=False, **kwargs)
 
@@ -168,3 +191,217 @@ class LatentDiffusion(nn.Module):
                                unconditional_guidance_scale=unconditional_guidance_scale,
                                unconditional_conditioning=unconditional_conditioning)
         return z, self.decode_first_stage(z)
+
+    # ---- ancestral sampler (ldm/diffusion/ddpm.py:1528-1793) -------------------------------------------------------------
+    def _ancestral_supported(self):
+        if self.parameterization != "eps":
+            raise NotImplementedError("ancestral sampling is built for parameterization 'eps' only (got %r)" % self.parameterization)
+        if self.shorten_cond_schedule:
+            raise NotImplementedError("shorten_cond_schedule is not supported")
+
+    def _ddpm_cache(self):
+        """(posterior_std [T] on the host, [5, T] device table of sdb_ddpm_step) for the current schedule buffers.  Built once
+        per schedule and rebuilt when any buffer it derives from is replaced (.to(), reassignment) or written in place
+        (load_state_dict): the key holds each buffer's identity, data_ptr and _version."""
+        src = (self.betas, self.sqrt_recip_alphas_cumprod, self.sqrt_recipm1_alphas_cumprod, self.posterior_mean_coef1,
+               self.posterior_mean_coef2, self.posterior_log_variance_clipped)
+        key = tuple((b.data_ptr(), b._version) for b in src)
+        hit = self.__dict__.get("_ddpm_tables")
+        if hit is None or hit[0] != key or any(r() is not b for r, b in zip(hit[1], src)):
+            # (0.5 * model_log_variance).exp() of p_sample, evaluated per element on a [1,1,1,1] fp32 host tensor: torch's CPU
+            # exp is not correctly rounded, and the reference applies it to a [b,1,1,1] tensor, i.e. element by element
+            lv = self.posterior_log_variance_clipped.detach().float().cpu()
+            std = torch.tensor([float((0.5 * torch.full((1, 1, 1, 1), float(v))).exp()) for v in lv], dtype=torch.float32)
+            dev = self.betas.device
+            table = torch.stack([b.detach().float().to(dev) for b in src[1:5]] + [std.to(dev)]).contiguous()
+            hit = (key, tuple(weakref.ref(b) for b in src), std, table)
+            self.__dict__["_ddpm_tables"] = hit
+        return hit[2], hit[3]
+
+    def posterior_std(self):
+        """fp32 [T] host table exp(0.5 * posterior_log_variance_clipped[t]): the std p_sample adds noise with."""
+        return self._ddpm_cache()[0]
+
+    def ddpm_table(self):
+        """[5, T] fp32 device table read by sdb_ddpm_step: sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod,
+        posterior_mean_coef1, posterior_mean_coef2, posterior_std."""
+        return self._ddpm_cache()[1]
+
+    @staticmethod
+    def _f32(t):
+        return t if (t is None or (t.dtype == torch.float32 and t.is_contiguous())) else t.float().contiguous()
+
+    def _timesteps(self, t, x):
+        return t if (t.dtype == torch.long and t.device == x.device and t.is_contiguous()) else t.to(x.device, torch.long).contiguous()
+
+    @staticmethod
+    def _extract(a, t, x_shape):
+        """extract_into_tensor (ldm/modules/diffusionmodules/util.py:96-99)."""
+        return a.gather(-1, t).reshape(t.shape[0], *((1,) * (len(x_shape) - 1)))
+
+    @torch.no_grad()
+    def predict_start_from_noise(self, x_t, t, noise):
+        """sqrt_recip_alphas_cumprod[t] * x_t - sqrt_recipm1_alphas_cumprod[t] * noise, one kernel."""
+        x = self._f32(x_t)
+        _, x0 = ops.ddpm_step(x, self._timesteps(t, x), self.ddpm_table(), eps=self._f32(noise), want_x_prev=False, want_x0=True)
+        return x0
+
+    @torch.no_grad()
+    def q_posterior(self, x_start, x_t, t):
+        """(posterior mean coef1[t] * x_start + coef2[t] * x_t, posterior_variance[t], posterior_log_variance_clipped[t])."""
+        x = self._f32(x_t)
+        t = self._timesteps(t, x)
+        mean, _ = ops.ddpm_step(x, t, self.ddpm_table(), x0=self._f32(x_start))
+        return mean, self._extract(self.posterior_variance, t, x.shape), self._extract(self.posterior_log_variance_clipped, t, x.shape)
+
+    def _model_eps(self, x, c, t, score_corrector, corrector_kwargs):
+        model_out = self.apply_model(x, t, c)
+        if score_corrector is not None:
+            model_out = score_corrector.modify_score(self, model_out, x, t, c, **corrector_kwargs)
+        return self._f32(model_out)
+
+    def _ancestral_update(self, x, t, eps, clip, quantize_denoised, draw=None):
+        """x0 -> (clamp) -> (first_stage_model.quantize) -> posterior mean (+ the noise `draw()` returns, drawn after quantize
+        like the reference).  Returns (x_prev, x0)."""
+        table = self.ddpm_table()
+        if quantize_denoised:
+            _, x0 = ops.ddpm_step(x, t, table, eps=eps, clip=clip, want_x_prev=False, want_x0=True)
+            x0 = self._f32(self.first_stage_model.quantize(x0)[0])
+            noise, temperature = draw() if draw is not None else (None, 1.)
+            x_prev, _ = ops.ddpm_step(x, t, table, x0=x0, noise=noise, temperature=temperature)
+            return x_prev, x0
+        noise, temperature = draw() if draw is not None else (None, 1.)
+        return ops.ddpm_step(x, t, table, eps=eps, noise=noise, clip=clip, temperature=temperature, want_x0=True)
+
+    @torch.no_grad()
+    def p_mean_variance(self, x, c, t, clip_denoised, return_codebook_ids=False, quantize_denoised=False, return_x0=False,
+                        score_corrector=None, corrector_kwargs=None):
+        """(model_mean, posterior_variance, posterior_log_variance[, x_recon]) of one denoising step."""
+        self._ancestral_supported()
+        if return_codebook_ids:
+            raise NotImplementedError("return_codebook_ids is not supported")
+        xf = self._f32(x)
+        t = self._timesteps(t, xf)
+        eps = self._model_eps(x, c, t, score_corrector, corrector_kwargs)
+        mean, x_recon = self._ancestral_update(xf, t, eps, clip_denoised, quantize_denoised)
+        var = self._extract(self.posterior_variance, t, xf.shape)
+        log_var = self._extract(self.posterior_log_variance_clipped, t, xf.shape)
+        return (mean, var, log_var, x_recon) if return_x0 else (mean, var, log_var)
+
+    @torch.no_grad()
+    def p_sample(self, x, c, t, clip_denoised=False, repeat_noise=False, return_codebook_ids=False, quantize_denoised=False,
+                 return_x0=False, temperature=1., noise_dropout=0., score_corrector=None, corrector_kwargs=None):
+        """model_mean + nonzero_mask * (0.5 * model_log_variance).exp() * noise_like(x.shape) * temperature, as one kernel
+        (two with quantize_denoised).  The noise is drawn on every step, t == 0 included, exactly as the reference draws it."""
+        self._ancestral_supported()
+        if return_codebook_ids:
+            raise NotImplementedError("return_codebook_ids is not supported")
+        xf = self._f32(x)
+        t = self._timesteps(t, xf)
+        eps = self._model_eps(x, c, t, score_corrector, corrector_kwargs)
+
+        def draw():
+            if repeat_noise:
+                noise = torch.randn((1, *x.shape[1:]), device=x.device).repeat(x.shape[0], *((1,) * (x.dim() - 1)))
+            else:
+                noise = torch.randn(x.shape, device=x.device)
+            if noise_dropout > 0.:
+                # dropout acts on noise * temperature and draws its own mask: form the product here, the kernel scales by 1
+                return torch.nn.functional.dropout(noise * temperature, p=noise_dropout), 1.
+            return noise, temperature
+
+        x_prev, x0 = self._ancestral_update(xf, t, eps, clip_denoised, quantize_denoised, draw)
+        return (x_prev, x0) if return_x0 else x_prev
+
+    def _inpaint(self, x0, ts, mask, img):
+        """img_orig = self.q_sample(x0, ts); img_orig * mask + (1. - mask) * img, fused (the DDIM sampler's blend)."""
+        return DDIMSampler(self)._inpaint_blend(x0, ts, mask, img)
+
+    @staticmethod
+    def _slice_cond(cond, batch_size):
+        if cond is None:
+            return None
+        if isinstance(cond, dict):
+            return {k: cond[k][:batch_size] if not isinstance(cond[k], list) else [x[:batch_size] for x in cond[k]] for k in cond}
+        return [c[:batch_size] for c in cond] if isinstance(cond, list) else cond[:batch_size]
+
+    @torch.no_grad()
+    def p_sample_loop(self, cond, shape, return_intermediates=False, x_T=None, verbose=True, callback=None, timesteps=None,
+                      quantize_denoised=False, mask=None, x0=None, img_callback=None, start_T=None, log_every_t=None):
+        """Ancestral sampling from t = timesteps - 1 down to 0; intermediates = [x_T] + img every log_every_t steps."""
+        self._ancestral_supported()
+        if not log_every_t:
+            log_every_t = self.log_every_t
+        device = self.betas.device
+        b = shape[0]
+        img = torch.randn(shape, device=device) if x_T is None else x_T
+        intermediates = [img]
+        if timesteps is None:
+            timesteps = self.num_timesteps
+        if start_T is not None:
+            timesteps = min(timesteps, start_T)
+        if mask is not None:
+            assert x0 is not None
+            assert x0.shape[2:3] == mask.shape[2:3]  # spatial size has to match
+        for i in reversed(range(0, timesteps)):
+            ts = torch.full((b,), i, device=device, dtype=torch.long)
+            img = self.p_sample(img, cond, ts, clip_denoised=self.clip_denoised, quantize_denoised=quantize_denoised)
+            if mask is not None:
+                img = self._inpaint(x0, ts, mask, img)
+            if i % log_every_t == 0 or i == timesteps - 1:
+                intermediates.append(img)
+            if callback:
+                callback(i)
+            if img_callback:
+                img_callback(img, i)
+        if return_intermediates:
+            return img, intermediates
+        return img
+
+    @torch.no_grad()
+    def sample(self, cond, batch_size=16, return_intermediates=False, x_T=None, verbose=True, timesteps=None,
+               quantize_denoised=False, mask=None, x0=None, shape=None, **kwargs):
+        """p_sample_loop over (batch_size, channels, image_size, image_size) unless `shape` is given."""
+        if shape is None:
+            shape = (batch_size, self.channels, self.image_size, self.image_size)
+        cond = self._slice_cond(cond, batch_size)
+        return self.p_sample_loop(cond, shape, return_intermediates=return_intermediates, x_T=x_T, verbose=verbose,
+                                  timesteps=timesteps, quantize_denoised=quantize_denoised, mask=mask, x0=x0)
+
+    @torch.no_grad()
+    def progressive_denoising(self, cond, shape, verbose=True, callback=None, quantize_denoised=False, img_callback=None,
+                              mask=None, x0=None, temperature=1., noise_dropout=0., score_corrector=None, corrector_kwargs=None,
+                              batch_size=None, x_T=None, start_T=None, log_every_t=None):
+        """Ancestral sampling that logs the predicted x0 (`x0_partial`) every log_every_t steps; `temperature` is one
+        value or a list indexed by the timestep."""
+        self._ancestral_supported()
+        if not log_every_t:
+            log_every_t = self.log_every_t
+        timesteps = self.num_timesteps
+        if batch_size is not None:
+            b = batch_size
+            shape = [batch_size] + list(shape)
+        else:
+            b = batch_size = shape[0]
+        img = torch.randn(shape, device=self.device) if x_T is None else x_T
+        intermediates = []
+        cond = self._slice_cond(cond, batch_size)
+        if start_T is not None:
+            timesteps = min(timesteps, start_T)
+        if isinstance(temperature, (int, float)):
+            temperature = [float(temperature)] * timesteps
+        for i in reversed(range(0, timesteps)):
+            ts = torch.full((b,), i, device=self.device, dtype=torch.long)
+            img, x0_partial = self.p_sample(img, cond, ts, clip_denoised=self.clip_denoised, quantize_denoised=quantize_denoised,
+                                            return_x0=True, temperature=temperature[i], noise_dropout=noise_dropout,
+                                            score_corrector=score_corrector, corrector_kwargs=corrector_kwargs)
+            if mask is not None:
+                assert x0 is not None
+                img = self._inpaint(x0, ts, mask, img)
+            if i % log_every_t == 0 or i == timesteps - 1:
+                intermediates.append(x0_partial)
+            if callback:
+                callback(i)
+            if img_callback:
+                img_callback(img, i)
+        return img, intermediates
