@@ -58,6 +58,15 @@ int sdb_nchw_to_nhwc(const float* src, void* dst, int dst_dtype, int N, int C, i
  * the tensor cores without rounding x_t itself to bf16. */
 int sdb_nchw_to_nhwc_split(const float* src, void* dst /* bf16 */, int N, int C, int dst_C, int HW, void* stream);
 int sdb_nhwc_to_nchw(const float* src, float* dst, int N, int C, int HW, void* stream);
+/* The same layout change from TWO channel-concatenated sources, in one pass: the channel order of dst is src0's C0 channels,
+ * then src1's C1 channels (C = C0 + C1), then zeros up to dst_C (0 = C, or 2*C with split).  Replaces
+ * torch.cat([x] + c_concat, dim=1) of DiffusionWrapper.forward (ldm/diffusion/ddpm.py:1992-2034, conditioning_key "concat" /
+ * "hybrid": the inpainting UNet's latent | mask | masked-image latent) together with the boundary transpose feeding conv_in.
+ * src0 [N,C0,HW], src1 [N,C1,HW] fp32 (src1 = NULL exactly when C1 = 0); dst [N,HW,dst_C] of dst_dtype.  split != 0 (bf16 dst,
+ * dst_C >= 2*C): channels C..2C-1 hold the rounding residual of channels 0..C-1, as sdb_nchw_to_nhwc_split.  sdb_nchw_to_nhwc
+ * and sdb_nchw_to_nhwc_split are its C1 = 0 case. */
+int sdb_nchw_concat_to_nhwc(const float* src0, int C0, const float* src1, int C1, void* dst, int dst_dtype, int dst_C, int split,
+                            int N, int HW, void* stream);
 
 /* ---- GroupNorm(32) [+ SiLU] over NHWC, optional two-source channel concat -------------------
  * Replaces GroupNorm32.forward + nn.SiLU (openai_model/utils.py:15-22, model.py:178-181,202-205,

@@ -85,6 +85,7 @@ SIGNATURES = {
     "sdb_pdl_skip_next": (_I, [_I]),
     "sdb_nchw_to_nhwc": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
     "sdb_nchw_to_nhwc_split": (_I, [_P, _P, _I, _I, _I, _I, _P]),
+    "sdb_nchw_concat_to_nhwc": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _I, _P]),
     "sdb_nhwc_to_nchw": (_I, [_P, _P, _I, _I, _I, _P]),
     "sdb_groupnorm_ws_bytes": (_L, [_I, _I, _I, _I]),
     "sdb_groupnorm_nhwc": (_I, [_P, _I, _P, _I, _I, _I, _I, _F, _P, _P, _L, _I, _I, _P, _I, _P, _P, _P, _P]),

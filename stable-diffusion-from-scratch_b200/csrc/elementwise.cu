@@ -5,21 +5,32 @@
 namespace sdb {
 
 // ---- NCHW <-> NHWC (32x32 smem tile transpose, padded against bank conflicts) -------------------
+// Two sources: channels 0..C0-1 come from src0 [N, C0, HW], channels C0..C0+C1-1 from src1 [N, C1, HW] (C1 = 0: src0 only), so the
+// channel concat in front of a conditioned UNet's conv_in (ldm/diffusion/ddpm.py:1992-2034, torch.cat([x] + c_concat, dim=1)) is
+// done by the same pass that changes the layout.  C = C0 + C1.
 // SPLIT (bf16 output only): channels C..2C-1 carry the rounding residual x - float(bf16(x)) of channels 0..C-1, so a bf16
 // contraction whose weights are repeated for both halves sees x to ~2^-17 instead of 2^-9 (the UNet's conv_in on the tensor
 // cores without rounding the latent x_t itself).
 template <bool OUT_BF16, bool SPLIT>
-__global__ void nchw_to_nhwc_kernel(const float* __restrict__ src, void* __restrict__ dst, int C, int Cd, int HW) {
+__global__ void nchw_to_nhwc_kernel(const float* __restrict__ src0, int C0, const float* __restrict__ src1, int C1,
+                                    void* __restrict__ dst, int Cd, int HW) {
     pdl_trigger();
     pdl_wait();
     __shared__ float tile[32][33];
+    const int C = C0 + C1;
     const int n = blockIdx.z;
     const int hw0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
-    const float* s = src + (long long)n * C * HW;
+    const float* s0 = src0 + (long long)n * C0 * HW;
+    const float* s1 = src1 + (long long)n * C1 * HW;
     for (int i = threadIdx.y; i < 32; i += blockDim.y) {
         int c = c0 + i, hw = hw0 + threadIdx.x;
         if (SPLIT && c >= C && c < 2 * C) c -= C;
-        tile[i][threadIdx.x] = (c < C && hw < HW) ? s[(long long)c * HW + hw] : 0.f;     // the remaining channels up to Cd are zero padding
+        float v = 0.f;                                                                  // the remaining channels up to Cd are zero padding
+        if (hw < HW) {
+            if (c < C0) v = s0[(long long)c * HW + hw];
+            else if (c < C) v = s1[(long long)(c - C0) * HW + hw];
+        }
+        tile[i][threadIdx.x] = v;
     }
     __syncthreads();
     for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -582,22 +593,38 @@ static int launch_skinny(const float* x, int M, int K, const void* W, const floa
 
 extern "C" {
 
+int sdb_nchw_concat_to_nhwc(const float* src0, int C0, const float* src1, int C1, void* dst, int dst_dtype, int dst_C, int split,
+                            int N, int HW, void* stream) {
+    SDB_REQUIRE(src0 && dst && N > 0 && C0 > 0 && C1 >= 0 && HW > 0, "nchw_concat_to_nhwc: bad args");
+    SDB_REQUIRE((C1 == 0) == (src1 == nullptr), "nchw_concat_to_nhwc: src1 must be given exactly when C1 > 0 (C1=%d)", C1);
+    SDB_REQUIRE(dst_dtype == SDB_F32 || dst_dtype == SDB_BF16, "nchw_concat_to_nhwc: bad dst_dtype %d", dst_dtype);
+    const int C = C0 + C1;
+    const int Cd = dst_C > 0 ? dst_C : C;
+    if (split) {
+        SDB_REQUIRE(dst_dtype == SDB_BF16, "nchw_concat_to_nhwc: split needs a bf16 destination");
+        SDB_REQUIRE(Cd >= 2 * C, "nchw_concat_to_nhwc: dst_C=%d < 2*C=%d", Cd, 2 * C);
+    } else {
+        SDB_REQUIRE(Cd >= C, "nchw_concat_to_nhwc: dst_C=%d < C=%d", Cd, C);
+    }
+    dim3 grid(ceil_div(HW, 32), ceil_div(Cd, 32), N), block(32, 8);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (split) launch_pdl(nchw_to_nhwc_kernel<true, true>, grid, block, 0, st, src0, C0, src1, C1, dst, Cd, HW);
+    else if (dst_dtype == SDB_BF16) launch_pdl(nchw_to_nhwc_kernel<true, false>, grid, block, 0, st, src0, C0, src1, C1, dst, Cd, HW);
+    else launch_pdl(nchw_to_nhwc_kernel<false, false>, grid, block, 0, st, src0, C0, src1, C1, dst, Cd, HW);
+    return check_launch(split ? "nchw_to_nhwc_kernel(split)" : "nchw_to_nhwc_kernel");
+}
+
 int sdb_nchw_to_nhwc(const float* src, void* dst, int dst_dtype, int N, int C, int dst_C, int HW, void* stream) {
     SDB_REQUIRE(src && dst && N > 0 && C > 0 && HW > 0, "nchw_to_nhwc: bad args");
     const int Cd = dst_C > 0 ? dst_C : C;
     SDB_REQUIRE(Cd >= C, "nchw_to_nhwc: dst_C=%d < C=%d", Cd, C);
-    dim3 grid(ceil_div(HW, 32), ceil_div(Cd, 32), N), block(32, 8);
-    if (dst_dtype == SDB_BF16) launch_pdl(nchw_to_nhwc_kernel<true, false>, dim3(grid), dim3(block), 0, (cudaStream_t)stream, src, dst, C, Cd, HW);
-    else launch_pdl(nchw_to_nhwc_kernel<false, false>, dim3(grid), dim3(block), 0, (cudaStream_t)stream, src, dst, C, Cd, HW);
-    return check_launch("nchw_to_nhwc_kernel");
+    return sdb_nchw_concat_to_nhwc(src, C, nullptr, 0, dst, dst_dtype == SDB_BF16 ? SDB_BF16 : SDB_F32, Cd, 0, N, HW, stream);
 }
 
 int sdb_nchw_to_nhwc_split(const float* src, void* dst, int N, int C, int dst_C, int HW, void* stream) {
     SDB_REQUIRE(src && dst && N > 0 && C > 0 && HW > 0, "nchw_to_nhwc_split: bad args");
     SDB_REQUIRE(dst_C >= 2 * C, "nchw_to_nhwc_split: dst_C=%d < 2*C=%d", dst_C, 2 * C);
-    dim3 grid(ceil_div(HW, 32), ceil_div(dst_C, 32), N), block(32, 8);
-    launch_pdl(nchw_to_nhwc_kernel<true, true>, dim3(grid), dim3(block), 0, (cudaStream_t)stream, src, dst, C, dst_C, HW);
-    return check_launch("nchw_to_nhwc_kernel(split)");
+    return sdb_nchw_concat_to_nhwc(src, C, nullptr, 0, dst, SDB_BF16, dst_C, 1, N, HW, stream);
 }
 
 int sdb_nhwc_to_nchw(const float* src, float* dst, int N, int C, int HW, void* stream) {

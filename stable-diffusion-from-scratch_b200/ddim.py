@@ -103,7 +103,10 @@ class DDIMSampler(object):
                unconditional_conditioning=None, **kwargs):
         if conditioning is not None:
             if isinstance(conditioning, dict):
-                cbs = conditioning[list(conditioning.keys())[0]].shape[0]
+                ctmp = conditioning[list(conditioning.keys())[0]]
+                while isinstance(ctmp, list):         # {"c_concat": [..], "c_crossattn": [..]} of a hybrid model
+                    ctmp = ctmp[0]
+                cbs = ctmp.shape[0]
                 if cbs != batch_size:
                     print(f"Warning: Got {cbs} conditionings but batch-size is {batch_size}")
             else:
@@ -223,6 +226,14 @@ class DDIMSampler(object):
                 self._cfg_ctx = hit
             e_uncond, e_t = self.model.apply_model(torch.cat([x] * 2), torch.cat([t] * 2), hit[3]).chunk(2)
             e_uncond, e_t = e_uncond.contiguous(), e_t.contiguous()
+        elif self._cfg_dict_pairable(c, unconditional_conditioning):
+            # image-conditioned ("concat" / "hybrid") models: one 2B call as well, every entry of the two dicts joined along the
+            # batch as the reference's dict branch does.  Per-sample results are batch-invariant, so this gives the bits of the
+            # two separate calls below; it also keeps ONE context tensor for all steps (the two calls alternate uc and c, which
+            # makes a CUDA-graph UNet re-project the context K/V on every call).
+            c_in = self._cfg_dict_in(c, unconditional_conditioning)
+            e_uncond, e_t = self.model.apply_model(torch.cat([x] * 2), torch.cat([t] * 2), c_in).chunk(2)
+            e_uncond, e_t = e_uncond.contiguous(), e_t.contiguous()
         else:
             e_uncond = self.model.apply_model(x, t, unconditional_conditioning)
             e_t = self.model.apply_model(x, t, c)
@@ -259,6 +270,37 @@ class DDIMSampler(object):
             x_prev = ops.ddim_xprev(pred_x0, ef, sqrt_aprev, dir_coef, k_sigma, e_uncond=uf, cfg_scale=unconditional_guidance_scale,
                                     noise=nf, temperature=k_temp)
         return x_prev, pred_x0
+
+    @staticmethod
+    def _cfg_dict_pairable(c, uc):
+        """Dict conditionings with a c_concat entry whose uc / c entries pair up one to one (same keys, same list lengths)."""
+        if not (isinstance(c, dict) and isinstance(uc, dict)) or "c_concat" not in c or set(c) != set(uc):
+            return False
+        for k in c:
+            a, b = c[k], uc[k]
+            if isinstance(a, list) != isinstance(b, list):
+                return False
+            if isinstance(a, list):
+                if len(a) != len(b) or not all(torch.is_tensor(v) for v in a + b):
+                    return False
+            elif not (torch.is_tensor(a) and torch.is_tensor(b)):
+                return False
+        return True
+
+    def _cfg_dict_in(self, c, uc):
+        """{k: [cat([uc[k][i], c[k][i]]) ...]} (tensor entries: cat([uc[k], c[k]])), built once per (uc, c) pair: the key holds
+        every tensor's data_ptr and _version, and a hit also needs each cached weakref to still be the same live object."""
+        leaves = [(k, i, uc[k][i] if isinstance(uc[k], list) else uc[k], v)
+                  for k in sorted(c) for i, v in (enumerate(c[k]) if isinstance(c[k], list) else [(None, c[k])])]
+        key = ("dict",) + tuple((k, i, u.data_ptr(), u._version, v.data_ptr(), v._version) for k, i, u, v in leaves)
+        hit = self._cfg_ctx
+        if (hit is None or hit[0] != key
+                or any(ru() is not u or rv() is not v for (ru, rv), (_, _, u, v) in zip(hit[1], leaves))):
+            c_in = {k: ([torch.cat([uc[k][i], c[k][i]]) for i in range(len(c[k]))] if isinstance(c[k], list)
+                        else torch.cat([uc[k], c[k]])) for k in c}
+            hit = (key, [(weakref.ref(u), weakref.ref(v)) for _, _, u, v in leaves], c_in)
+            self._cfg_ctx = hit
+        return hit[2]
 
     @torch.no_grad()
     def stochastic_encode(self, x0, t, use_original_steps=False, noise=None):

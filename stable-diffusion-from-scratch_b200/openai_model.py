@@ -714,7 +714,8 @@ class UNetModel(nn.Module):
             emb = ops.add(emb, ops.gather_rows(P["label_emb"], y))
         return ops.skinny_linear(emb, P["emb_w"], P["emb_b"], act_in=1)
 
-    def _forward_nhwc(self, x_nchw, t_f32, context, mode, y=None):
+    def _forward_nhwc(self, x_nchw, t_f32, context, mode, y=None, x1_nchw=None):
+        """x1_nchw: channels appended to x's for conv_in (forward_concat); the concat happens inside the layout kernel."""
         P = self._pack(mode)
         if self.emb_side_stream:
             # The time-embedding chain (4 launches that stream the 20160 x 1280 emb_layers matrix, ~0.1 ms) depends on t only and
@@ -730,7 +731,7 @@ class UNetModel(nn.Module):
                 emb_all = _SideResult(self._time_embedding(P, t_f32, y), side, main)
         else:
             emb_all = self._time_embedding(P, t_f32, y)
-        h = ops.nchw_to_nhwc(x_nchw, out_dtype=P["conv_in"].in_dtype, pad_to=P["conv_in"].cin, split=P["conv_in_split"])
+        h = ops.nchw_to_nhwc(x_nchw, out_dtype=P["conv_in"].in_dtype, pad_to=P["conv_in"].cin, split=P["conv_in_split"], x1=x1_nchw)
         hs = []
         for module in self.input_blocks:
             h = self._run_block(module, P, mode, h, None, emb_all, context)
@@ -748,25 +749,58 @@ class UNetModel(nn.Module):
     def forward(self, x, timesteps=None, context=None, y=None, **kwargs):
         """Apply the model to an input batch (openai_model/model.py:550-595).
         x [N,C,H,W], timesteps [N] (int or float), context [N,S,context_dim] -> [N,out_channels,H,W] in x.dtype."""
+        return self._forward_impl(x, None, timesteps, context, y)
+
+    @torch.no_grad()
+    def forward_concat(self, x, c_concat, timesteps=None, context=None, y=None):
+        """forward(torch.cat([x, *c_concat], 1), timesteps, context, y), bit for bit, without the concatenated tensor: the
+        channel concat of a "concat" / "hybrid" conditioned model (ldm/diffusion/ddpm.py:1992-2034, e.g. an inpainting UNet's
+        4 latent + 1 mask + 4 masked-image channels) is done by the layout kernel that feeds conv_in.
+        c_concat: a tensor [N,Cc,H,W] or a list of them (a list of several is joined once, here).  Shapes must agree with x
+        and the channels add up to in_channels; a mismatch raises ValueError before any kernel runs."""
+        if torch.is_tensor(c_concat):
+            c_concat = [c_concat]
+        if not isinstance(c_concat, (list, tuple)) or len(c_concat) == 0 or not all(torch.is_tensor(c) for c in c_concat):
+            raise ValueError("c_concat must be a tensor or a non-empty list of tensors")
+        if x.dim() != 4 or any(c.dim() != 4 for c in c_concat):
+            raise ValueError("forward_concat needs 4-D [N,C,H,W] tensors, got x %s and c_concat %s" % (
+                tuple(x.shape), [tuple(c.shape) for c in c_concat]))
+        for c in c_concat:
+            if c.shape[0] != x.shape[0] or c.shape[2:] != x.shape[2:]:
+                raise ValueError("c_concat %s does not match x %s in N, H, W" % (tuple(c.shape), tuple(x.shape)))
+            if c.device != x.device:
+                raise ValueError("c_concat is on %s, x on %s: all inputs must be on one device" % (c.device, x.device))
+        for name, v in (("timesteps", timesteps), ("context", context), ("y", y)):
+            if v is not None and v.device != x.device:
+                raise ValueError("%s is on %s, x on %s: all inputs must be on one device" % (name, v.device, x.device))
+        total = x.shape[1] + sum(c.shape[1] for c in c_concat)
+        if total != self.in_channels:
+            raise ValueError("x has %d channels and c_concat %s: %d in all, the model takes in_channels=%d" % (
+                x.shape[1], [c.shape[1] for c in c_concat], total, self.in_channels))
+        cc = c_concat[0] if len(c_concat) == 1 else torch.cat(list(c_concat), 1)
+        return self._forward_impl(x, cc, timesteps, context, y)
+
+    def _forward_impl(self, x, x1, timesteps, context, y):
         assert (y is not None) == (self.num_classes is not None), "must specify y if and only if the model is class-conditional"
         from ._lib import require_cuda
         with torch.cuda.device(x.device):
-            require_cuda(x, timesteps, context, y)
+            require_cuda(x, x1, timesteps, context, y)
             self._check_weights()
             mode = self.compute_mode
             xin = x.float().contiguous()
+            x1in = x1.float().contiguous() if x1 is not None else None
             tin = timesteps.float().contiguous()
             cin = context.float().contiguous() if context is not None else None
             if y is not None:
                 assert y.shape == (x.shape[0],)
                 y = y.to(torch.int64).contiguous()
             if self.use_cuda_graph and y is None and cin is not None:
-                out = self._graph_forward(xin, tin, cin, mode, ctx_src=context)
+                out = self._graph_forward(xin, tin, cin, mode, ctx_src=context, x1=x1in)
             else:
                 # K/V projections of the conditioning are cached against the CALLER's tensor object (cin may be a temporary)
                 self.__dict__["_ctx_src"] = context if cin is not context else None
                 try:
-                    out = self._forward_nhwc(xin, tin, cin, mode, y=y)
+                    out = self._forward_nhwc(xin, tin, cin, mode, y=y, x1_nchw=x1in)
                 finally:
                     self.__dict__["_ctx_src"] = None
         return out if x.dtype == torch.float32 else out.to(x.dtype)
@@ -778,20 +812,23 @@ class UNetModel(nn.Module):
         self._ctx_cache.clear()
         return {id(m): self._kv_context(m, P, mode, context) for m in self.modules() if isinstance(m, BasicTransformerBlock)}
 
-    def _graph_forward(self, x, t, ctx, mode, ctx_src=None):
+    def _graph_forward(self, x, t, ctx, mode, ctx_src=None, x1=None):
         """Two graphs per (mode, shapes): the context projections (to_k / to_v of every cross-attention; they depend on the
         context only, which a sampler passes unchanged for all its steps — ldm/diffusion/ddim.py:174 calls apply_model with
-        the same `c` 50 times) are replayed only when the caller's context tensor changed; the UNet body every call."""
-        key = (mode, tuple(x.shape), tuple(ctx.shape))
+        the same `c` 50 times) are replayed only when the caller's context tensor changed; the UNet body every call.
+        x1 (forward_concat): the concatenated channels, a static input copied in on every replay like x.  Its shape is part of
+        the key (None for forward), so a graph captured for one entry is never replayed for the other."""
+        key = (mode, tuple(x.shape), tuple(ctx.shape), None if x1 is None else tuple(x1.shape))
         g = self._graphs.get(key)
         if g is None:
             sx, st_, sc = x.clone(), t.clone(), ctx.clone()
+            sx1 = x1.clone() if x1 is not None else None
             P = self._pack(mode)
             s = torch.cuda.Stream()
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
                 for _ in range(2):            # warm-up: pack weights, set kernel attributes
-                    self._forward_nhwc(sx, st_, sc, mode)
+                    self._forward_nhwc(sx, st_, sc, mode, x1_nchw=sx1)
             torch.cuda.current_stream().wait_stream(s)
             kv_graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(kv_graph):
@@ -800,14 +837,16 @@ class UNetModel(nn.Module):
             graph = torch.cuda.CUDAGraph()
             try:
                 with torch.cuda.graph(graph, pool=kv_graph.pool()):
-                    out = self._forward_nhwc(sx, st_, sc, mode)
+                    out = self._forward_nhwc(sx, st_, sc, mode, x1_nchw=sx1)
             finally:
                 self._kv_pinned = None
                 self._ctx_cache.clear()
-            g = [graph, kv_graph, sx, st_, sc, out, None, pinned]      # `pinned` keeps the projections' memory alive
+            g = [graph, kv_graph, sx, st_, sc, out, None, pinned, sx1]      # `pinned` keeps the projections' memory alive
             self._graphs[key] = g
         graph, kv_graph, sx, st_, sc, out, seen = g[:7]
         sx.copy_(x)
+        if x1 is not None:
+            g[8].copy_(x1)
         st_.copy_(t)
         # same live tensor object, not modified in place since the last call => same conditioning
         src = ctx_src if ctx_src is not None else ctx

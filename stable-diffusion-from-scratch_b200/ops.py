@@ -18,16 +18,29 @@ def _L():
 
 
 # ---- layout ---------------------------------------------------------------------------------------
-def nchw_to_nhwc(x, out_dtype=torch.float32, pad_to=0, split=False):
+def nchw_to_nhwc(x, out_dtype=torch.float32, pad_to=0, split=False, x1=None):
     """[N,C,H,W] fp32 -> [N,H,W,C] (or [N,H,W,pad_to] with zero channels appended).
-    split=True (bf16 output, pad_to >= 2C): channels C..2C-1 hold the bf16 rounding residual x - bf16(x) of channels 0..C-1."""
-    require_cuda(x)
+    split=True (bf16 output, pad_to >= 2C): channels C..2C-1 hold the bf16 rounding residual x - bf16(x) of channels 0..C-1.
+    x1 [N,C1,H,W] fp32: a second source whose channels follow x's (C = C + C1), i.e. the layout change of torch.cat([x, x1], 1)
+    in the same pass."""
+    require_cuda(x, x1)
     assert x.dtype == torch.float32 and x.is_contiguous()
     N, Cc, H, W = x.shape
-    Cd = max(Cc, pad_to)
+    C1 = 0
+    if x1 is not None:
+        assert x1.dtype == torch.float32 and x1.is_contiguous() and x1.dim() == 4
+        assert x1.shape[0] == N and tuple(x1.shape[2:]) == (H, W), "nchw_to_nhwc: x1 %s does not match x %s" % (
+            tuple(x1.shape), tuple(x.shape))
+        C1 = x1.shape[1]
+    Ct = Cc + C1
+    Cd = max(Ct, pad_to)
     out = torch.empty((N, H, W, Cd), dtype=out_dtype, device=x.device)
     if split:
-        assert out_dtype == torch.bfloat16 and Cd >= 2 * Cc
+        assert out_dtype == torch.bfloat16 and Cd >= 2 * Ct
+    if x1 is not None:
+        check(_L().sdb_nchw_concat_to_nhwc(ptr(x), Cc, ptr(x1), C1, ptr(out), dtype_code(out_dtype), Cd, int(split), N, H * W,
+                                           stream_ptr()), "nchw_concat_to_nhwc")
+    elif split:
         check(_L().sdb_nchw_to_nhwc_split(ptr(x), ptr(out), N, Cc, Cd, H * W, stream_ptr()), "nchw_to_nhwc_split")
     else:
         check(_L().sdb_nchw_to_nhwc(ptr(x), ptr(out), dtype_code(out_dtype), N, Cc, Cd, H * W, stream_ptr()), "nchw_to_nhwc")

@@ -3,7 +3,8 @@
 `LatentDiffusion` exposes exactly what `DDIMSampler` and the reference's `sample_log` /
 `decode_first_stage` call sites need (ldm/diffusion/ddpm.py:1326-1448, 1083-1156, 1814-1826):
 schedule buffers, `apply_model(x, t, cond)`, `decode_first_stage(z)`.  It owns a `UNetModel`
-(as `model.diffusion_model`, like DiffusionWrapper, ddpm.py:1992-2034) and an `AutoencoderKL`.
+(as `model.diffusion_model`, like DiffusionWrapper, ddpm.py:1992-2034, with all five conditioning keys) and an
+`AutoencoderKL`.
 It also carries the reference's ancestral sampler (`sample` / `p_sample_loop` / `progressive_denoising`,
 ddpm.py:1528-1793), whose per-step update runs as one fused kernel (sdb_ddpm_step).
 """
@@ -41,19 +42,46 @@ def make_beta_schedule(schedule, n_timestep, linear_start=1e-4, linear_end=2e-2)
 
 
 class DiffusionWrapper(nn.Module):
-    """ldm/diffusion/ddpm.py:1992-2034, crossattn conditioning only."""
+    """ldm/diffusion/ddpm.py:1992-2034: routes the conditioning to the UNet by `conditioning_key`.
+      None        diffusion_model(x, t)
+      "concat"    diffusion_model(cat([x] + c_concat, 1), t)
+      "crossattn" diffusion_model(x, t, context=cat(c_crossattn, 1))
+      "hybrid"    diffusion_model(cat([x] + c_concat, 1), t, context=cat(c_crossattn, 1))
+      "adm"       diffusion_model(x, t, y=c_crossattn[0])
+    The channel concat goes to the model's `forward_concat` when it has one (UNetModel: the concat is done by the layout
+    kernel feeding conv_in); any other eps-model gets the torch.cat and its plain forward."""
+
+    KEYS = (None, "concat", "crossattn", "hybrid", "adm")
 
     def __init__(self, diffusion_model, conditioning_key="crossattn"):
         super().__init__()
         self.diffusion_model = diffusion_model
         self.conditioning_key = conditioning_key
-        assert conditioning_key in (None, "crossattn")
+        assert conditioning_key in self.KEYS, "unknown conditioning_key %r (one of %s)" % (conditioning_key, self.KEYS)
+
+    @staticmethod
+    def _context(c_crossattn):
+        # one tensor is passed as is (no copy), so a UNet that caches its K/V projections per context tensor keeps hitting
+        return c_crossattn[0] if len(c_crossattn) == 1 else torch.cat(c_crossattn, 1)
+
+    def _concat(self, x, t, c_concat, **kw):
+        c_concat = [c_concat] if torch.is_tensor(c_concat) else list(c_concat)
+        fc = getattr(self.diffusion_model, "forward_concat", None)
+        if fc is not None:
+            return fc(x, c_concat, t, **kw)
+        return self.diffusion_model(torch.cat([x] + c_concat, dim=1), t, **kw)
 
     def forward(self, x, t, c_concat=None, c_crossattn=None):
-        if self.conditioning_key is None:
+        key = self.conditioning_key
+        if key is None:
             return self.diffusion_model(x, t)
-        cc = c_crossattn[0] if len(c_crossattn) == 1 else torch.cat(c_crossattn, 1)
-        return self.diffusion_model(x, t, context=cc)
+        if key == "concat":
+            return self._concat(x, t, c_concat)
+        if key == "crossattn":
+            return self.diffusion_model(x, t, context=self._context(c_crossattn))
+        if key == "hybrid":
+            return self._concat(x, t, c_concat, context=self._context(c_crossattn))
+        return self.diffusion_model(x, t, y=c_crossattn[0])          # "adm"
 
 
 class LatentDiffusion(nn.Module):
@@ -109,7 +137,8 @@ class LatentDiffusion(nn.Module):
         else:
             if not isinstance(cond, list):
                 cond = [cond]
-            cond = {"c_crossattn": cond}
+            key = "c_concat" if self.model.conditioning_key == "concat" else "c_crossattn"
+            cond = {key: cond}
         return self.model(x_noisy, t, **cond)
 
     @torch.no_grad()
