@@ -352,6 +352,31 @@ int sdb_attention_wide_fwd(const void* q, const void* k, const void* v, void* ou
                            long long k_bs, long long k_ss, long long v_bs, long long v_ss, long long o_bs, long long o_ss,
                            int B, int Sq, int Sk, int d, float scale, void* stream);
 
+/* ---- vector quantisation: the VQ first stage's codebook lookup ------------------------------------------------------
+ * sdb_vq_quantize replaces taming's VectorQuantizer2.forward in eval with legacy=True (ldm/tamming/quantize.py:213-311,
+ * the `quantize` of VQModel / VQModelInterface, ldm/models/autoencoder.py):
+ *   zf   = z as [M = N*HW, D] rows in (n, h, w) order
+ *   d    = (sum(zf**2, 1) + sum(W**2, 1)) - 2 * zf @ W.T          fp32, never materialised
+ *   idx  = argmin(d, 1)                                           first index of the minimum; NaN counts as the minimum
+ *   z_q  = z + (W[idx] - z)                                       straight-through, fp32, each operation rounded
+ *   loss = mean((W[idx] - z)**2) + beta * mean((W[idx] - z)**2)   one fp32 scalar, fp64 partials in a fixed order
+ * z fp32 in z_layout (SDB_NCHW: [N, D, HW]; SDB_NHWC: [N, HW, D]); z_q fp32 in zq_layout; idx int64 [M]; codebook W fp32
+ * [n_e, D], 1 <= D <= 16, any n_e >= 1.  z_q, idx and loss are each optional (NULL), not all three.  ws: device scratch of
+ * sdb_vq_ws_bytes(M, n_e) bytes; counters: >= 1 int, zero on entry and left zero (ticket of the CTA that folds the loss
+ * partials; only used when loss != NULL), the same buffer kind sdb_groupnorm_nhwc takes.  When M rows alone cannot fill the
+ * GPU the codebook is split into slices scanned by separate CTAs whose minima are merged by (NaN first, d, index): the
+ * split depends on M and n_e only, and the result does not depend on it. */
+#define SDB_NCHW  0
+#define SDB_NHWC  1
+long long sdb_vq_ws_bytes(long long M, int n_e);                    /* -1 on bad arguments */
+int sdb_vq_quantize(const float* z, int z_layout, int N, int HW, int D, const float* codebook, int n_e, float beta,
+                    float* z_q, int zq_layout, long long* idx, float* loss, void* ws, int* counters, void* stream);
+/* VectorQuantizer2.get_codebook_entry (ldm/tamming/quantize.py:313-329): out = W[idx] for M = N*HW indices in (n, h, w)
+ * order, written as out_layout ([N, D, HW] or [N, HW, D]) fp32.  An index outside [0, n_e) writes a NaN row and is never
+ * dereferenced. */
+int sdb_vq_codebook_gather(const long long* idx, long long M, const float* codebook, int n_e, int D, float* out, int out_layout,
+                           int HW, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -122,6 +122,9 @@ SIGNATURES = {
     "sdb_attention_fwd": (_I, [C.POINTER(AttnArgs), _P]),
     "sdb_attention_set_short_key_kernel": (_I, [_I]),
     "sdb_attention_wide_fwd": (_I, [_P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _L, _L, _I, _I, _I, _I, _F, _P]),
+    "sdb_vq_ws_bytes": (_L, [_L, _I]),
+    "sdb_vq_quantize": (_I, [_P, _I, _I, _I, _I, _P, _I, _F, _P, _I, _P, _P, _P, _P, _P]),
+    "sdb_vq_codebook_gather": (_I, [_P, _L, _P, _I, _I, _P, _I, _I, _P]),
 }
 
 

@@ -9,6 +9,10 @@ Same constructor kwargs and state-dict keys (`decoder.conv_in`, `decoder.mid.blo
 `VAE.autoencoder.AutoEncoderKL.decode` (VAE/autoencoder.py:126-132) is served by the same class
 through the `AutoEncoderKL` alias; its fp16-only 8-head mid attention (Unet/attention.py:221-264)
 is NOT replicated — the numerical oracle is the canonical `ldm` decoder (SURVEY.md §8a V2).
+
+The VQ-regularised first stage of the reference's VQ latent-diffusion models (`VQModel`, `VQModelInterface`,
+ldm/models/autoencoder.py; `IdentityFirstStage` for pixel-space models) is built from the same Encoder / Decoder
+with `double_z=False`, and taming's `VectorQuantizer2` (sdb200.quantize) on the sdb_vq_quantize kernels.
 """
 import torch
 from torch import nn
@@ -274,7 +278,7 @@ class Encoder(_VaeNet):
         for i_level in range(self.num_resolutions):
             for i_block in range(self.num_res_blocks):
                 h = self._resnet(self.down[i_level].block[i_block], P, mode, h)
-                if len(self.down[i_level].attn) > 0:
+                if len(self.down[i_level].attn) > 0 and isinstance(self.down[i_level].attn[i_block], AttnBlock):
                     h = self._attn(self.down[i_level].attn[i_block], P, mode, h)
             if i_level != self.num_resolutions - 1:
                 pc = P[("down", id(self.down[i_level].downsample))]
@@ -395,7 +399,7 @@ class Decoder(_VaeNet):
         for i_level in reversed(range(self.num_resolutions)):
             for i_block in range(self.num_res_blocks + 1):
                 h = self._resnet(self.up[i_level].block[i_block], P, mode, h)
-                if len(self.up[i_level].attn) > 0:
+                if len(self.up[i_level].attn) > 0 and isinstance(self.up[i_level].attn[i_block], AttnBlock):
                     h = self._attn(self.up[i_level].attn[i_block], P, mode, h)
             if i_level != 0:
                 pc = P[("up", id(self.up[i_level].upsample))]
@@ -419,25 +423,9 @@ class Decoder(_VaeNet):
         return out if z.dtype == torch.float32 else out.to(z.dtype)
 
 
-class AutoencoderKL(nn.Module):
-    """ldm/models/autoencoder.py:292-350: decode (hot path), encode and forward ('next' row f3).  The loss / Lightning
-    training hooks are out of scope (SURVEY.md §2.1); their state-dict keys are tolerated with strict=False."""
-
-    def __init__(self, ddconfig, lossconfig=None, embed_dim=4, ckpt_path=None, ignore_keys=[], image_key="image",
-                 colorize_nlabels=None, monitor=None, compute_mode=None, micro_batch=8):
-        super().__init__()
-        self.image_key = image_key
-        self.encoder = Encoder(**ddconfig, compute_mode=compute_mode)
-        self.decoder = Decoder(**ddconfig, compute_mode=compute_mode)
-        assert ddconfig["double_z"]
-        self.quant_conv = nn.Conv2d(2 * ddconfig["z_channels"], 2 * embed_dim, 1)
-        self.post_quant_conv = nn.Conv2d(embed_dim, ddconfig["z_channels"], 1)
-        self.embed_dim = embed_dim
-        self.micro_batch = micro_batch
-        if monitor is not None:
-            self.monitor = monitor
-        if ckpt_path is not None:
-            self.init_from_ckpt(ckpt_path, ignore_keys=ignore_keys)
+class _FirstStage(nn.Module):
+    """What AutoencoderKL and VQModel share: Encoder / Decoder compute mode, checkpoint loading, the fp32 SIMT packing
+    of the 1x1 quant_conv / post_quant_conv, and the micro-batched encode / decode loops."""
 
     @property
     def compute_mode(self):
@@ -476,7 +464,7 @@ class AutoencoderKL(nn.Module):
     _q = None
 
     def _packed_1x1(self, slot, conv):
-        """quant_conv / post_quant_conv packed for the fp32 SIMT kernel (C_in = 4 or 8), re-packed whenever the layer's
+        """quant_conv / post_quant_conv packed for the fp32 SIMT kernel (C_in = 3 ... 8), re-packed whenever the layer's
         parameters were replaced or written in place."""
         fp = (conv.weight.data_ptr(), conv.weight._version, conv.bias.data_ptr(), conv.bias._version)
         cur = getattr(self, slot)
@@ -485,48 +473,182 @@ class AutoencoderKL(nn.Module):
             setattr(self, slot, cur)
         return cur[1]
 
-    @torch.no_grad()
-    def encode(self, x):
-        """AutoencoderKL.encode (autoencoder.py:331-335): Encoder, quant_conv (1x1, 8->8), posterior.
-        x [N,3,H,W] in [-1,1] -> DiagonalGaussianDistribution over [N,embed_dim,H/8,W/8]."""
+    def _encode_quant_conv(self, x):
+        """Encoder then quant_conv, in micro-batches of `micro_batch` images: x [N,C,H,W] -> [N,C',h,w] fp32 NCHW."""
         from ._lib import require_cuda
         with torch.cuda.device(x.device):
             require_cuda(x)
             mode = self.encoder.compute_mode
-            qc = self._packed_1x1("_q", self.quant_conv)                                   # C_in = 8: SIMT fp32 kernel in both modes
+            qc = self._packed_1x1("_q", self.quant_conv)                                   # tiny C_in: SIMT fp32 kernel in both modes
             xf = x.float().contiguous()
             outs = []
             for i in range(0, xf.shape[0], self.micro_batch):
                 h = self.encoder._forward_nhwc(ops.nchw_to_nhwc(xf[i:i + self.micro_batch].contiguous()), mode)
                 outs.append(ops.nhwc_to_nchw(engine.conv(h, qc)))
-            moments = outs[0] if len(outs) == 1 else torch.cat(outs, 0)
-            return DiagonalGaussianDistribution(moments)
+            return outs[0] if len(outs) == 1 else torch.cat(outs, 0)
 
-    @torch.no_grad()
-    def decode(self, z):
-        """AutoencoderKL.decode (autoencoder.py:337-340): post_quant_conv (1x1, 4->4) then Decoder.
-        Large batches are decoded in micro-batches of `micro_batch` images (activations at 512^2 are
-        ~0.5 GB/image); results are identical because nothing on the path reduces over the batch."""
+    def _decode_post_quant(self, z, to_nhwc):
+        """post_quant_conv then Decoder on z [N,C,h,w], in micro-batches of `micro_batch` images (activations at 512^2
+        are ~0.5 GB/image); results are identical because nothing on the path reduces over the batch.  `to_nhwc` turns
+        one NCHW fp32 micro-batch into the NHWC fp32 operand of post_quant_conv."""
         from ._lib import require_cuda
         with torch.cuda.device(z.device):
             require_cuda(z)
             mode = self.decoder.compute_mode
-            pq = self._packed_1x1("_pq", self.post_quant_conv)                             # C_in = 4: SIMT fp32 kernel in both modes
+            pq = self._packed_1x1("_pq", self.post_quant_conv)                             # tiny C_in: SIMT fp32 kernel in both modes
             zf = z.float().contiguous()
             N = zf.shape[0]
             outs = []
             for i in range(0, N, self.micro_batch):
-                h = ops.nchw_to_nhwc(zf[i:i + self.micro_batch].contiguous())
-                h = engine.conv(h, pq)
+                h = engine.conv(to_nhwc(zf[i:i + self.micro_batch].contiguous()), pq)
                 outs.append(ops.nhwc_to_nchw(self.decoder._forward_nhwc(h, mode)))
             out = outs[0] if len(outs) == 1 else torch.cat(outs, 0)
         return out if z.dtype == torch.float32 else out.to(z.dtype)
+
+
+class AutoencoderKL(_FirstStage):
+    """ldm/models/autoencoder.py:292-350: decode (hot path), encode and forward ('next' row f3).  The loss / Lightning
+    training hooks are out of scope (SURVEY.md §2.1); their state-dict keys are tolerated with strict=False."""
+
+    def __init__(self, ddconfig, lossconfig=None, embed_dim=4, ckpt_path=None, ignore_keys=[], image_key="image",
+                 colorize_nlabels=None, monitor=None, compute_mode=None, micro_batch=8):
+        super().__init__()
+        self.image_key = image_key
+        self.encoder = Encoder(**ddconfig, compute_mode=compute_mode)
+        self.decoder = Decoder(**ddconfig, compute_mode=compute_mode)
+        assert ddconfig["double_z"]
+        self.quant_conv = nn.Conv2d(2 * ddconfig["z_channels"], 2 * embed_dim, 1)
+        self.post_quant_conv = nn.Conv2d(embed_dim, ddconfig["z_channels"], 1)
+        self.embed_dim = embed_dim
+        self.micro_batch = micro_batch
+        if monitor is not None:
+            self.monitor = monitor
+        if ckpt_path is not None:
+            self.init_from_ckpt(ckpt_path, ignore_keys=ignore_keys)
+
+    @torch.no_grad()
+    def encode(self, x):
+        """AutoencoderKL.encode (autoencoder.py:331-335): Encoder, quant_conv (1x1, 8->8), posterior.
+        x [N,3,H,W] in [-1,1] -> DiagonalGaussianDistribution over [N,embed_dim,H/8,W/8]."""
+        moments = self._encode_quant_conv(x)
+        with torch.cuda.device(moments.device):
+            return DiagonalGaussianDistribution(moments)
+
+    @torch.no_grad()
+    def decode(self, z):
+        """AutoencoderKL.decode (autoencoder.py:337-340): post_quant_conv (1x1, 4->4) then Decoder."""
+        return self._decode_post_quant(z, ops.nchw_to_nhwc)
 
     def forward(self, input, sample_posterior=True):
         """autoencoder.py:342-349: (reconstruction, posterior)."""
         posterior = self.encode(input)
         z = posterior.sample() if sample_posterior else posterior.mode()
         return self.decode(z), posterior
+
+
+class VQModel(_FirstStage):
+    """ldm/models/autoencoder.py VQModel (inference): Encoder, quant_conv (z_channels -> embed_dim), VectorQuantizer2
+    (`quantize`, n_embed codes of embed_dim), post_quant_conv (embed_dim -> z_channels), Decoder; the reference's
+    constructor kwargs and state-dict keys (`quantize.embedding.weight`, ...).  The loss, Lightning training hooks,
+    batch resizing and the LR schedule are out of scope: their kwargs are accepted and ignored and `loss.*` keys are
+    tolerated with strict=False."""
+
+    def __init__(self, ddconfig, lossconfig, n_embed, embed_dim, ckpt_path=None, ignore_keys=[], image_key="image",
+                 colorize_nlabels=None, monitor=None, batch_resize_range=None, scheduler_config=None, lr_g_factor=1.0,
+                 remap=None, sane_index_shape=False, use_ema=False, compute_mode=None, micro_batch=8):
+        super().__init__()
+        if use_ema:
+            raise NotImplementedError("sdb200 VQModel: use_ema (LitEma training copy) is not built")
+        from .quantize import VectorQuantizer2
+        self.embed_dim = embed_dim
+        self.n_embed = n_embed
+        self.image_key = image_key
+        self.encoder = Encoder(**ddconfig, compute_mode=compute_mode)
+        self.decoder = Decoder(**ddconfig, compute_mode=compute_mode)
+        self.quantize = VectorQuantizer2(n_embed, embed_dim, beta=0.25, remap=remap, sane_index_shape=sane_index_shape)
+        self.quant_conv = nn.Conv2d(ddconfig["z_channels"], embed_dim, 1)
+        self.post_quant_conv = nn.Conv2d(embed_dim, ddconfig["z_channels"], 1)
+        self.micro_batch = micro_batch
+        self.batch_resize_range = batch_resize_range
+        self.scheduler_config = scheduler_config
+        self.lr_g_factor = lr_g_factor
+        self.use_ema = use_ema
+        if monitor is not None:
+            self.monitor = monitor
+        if ckpt_path is not None:
+            self.init_from_ckpt(ckpt_path, ignore_keys=ignore_keys)
+
+    @torch.no_grad()
+    def encode(self, x):
+        """(quant, emb_loss, (None, None, indices)): Encoder, quant_conv, quantize."""
+        return self.quantize(self.encode_to_prequant(x))
+
+    @torch.no_grad()
+    def encode_to_prequant(self, x):
+        """Encoder then quant_conv: x [N,3,H,W] -> [N,embed_dim,h,w] fp32."""
+        return self._encode_quant_conv(x)
+
+    @torch.no_grad()
+    def decode(self, quant):
+        """post_quant_conv then Decoder."""
+        return self._decode_post_quant(quant, ops.nchw_to_nhwc)
+
+    def decode_code(self, code_b):
+        # the reference calls quantize.embed_code, which VectorQuantizer2 does not define
+        raise NotImplementedError("VQModel.decode_code: VectorQuantizer2 has no embed_code; use "
+                                  "decode(quantize.get_codebook_entry(indices, shape))")
+
+    def forward(self, input, return_pred_indices=False):
+        quant, diff, (_, _, ind) = self.encode(input)
+        dec = self.decode(quant)
+        if return_pred_indices:
+            return dec, diff, ind
+        return dec, diff
+
+
+class VQModelInterface(VQModel):
+    """ldm/models/autoencoder.py VQModelInterface, the first stage of the VQ latent-diffusion models: encode stops
+    before the quantizer; decode quantizes (unless force_not_quantize) and decodes.  On the decode path the quantizer
+    writes z_q channels-last straight into post_quant_conv's operand."""
+
+    def __init__(self, embed_dim, *args, **kwargs):
+        super().__init__(*args, embed_dim=embed_dim, **kwargs)
+        self.embed_dim = embed_dim
+
+    @torch.no_grad()
+    def encode(self, x):
+        return self.encode_to_prequant(x)
+
+    @torch.no_grad()
+    def decode(self, h, force_not_quantize=False):
+        from ._lib import require_cuda
+        require_cuda(h)
+        if force_not_quantize:
+            return self._decode_post_quant(h, ops.nchw_to_nhwc)
+        to_nhwc = lambda z: self.quantize._quantize(z, zq_layout="nhwc", want_idx=False, want_loss=False)[0]
+        return self._decode_post_quant(h, to_nhwc)
+
+
+class IdentityFirstStage(nn.Module):
+    """ldm/models/autoencoder.py IdentityFirstStage: the first stage of pixel-space models."""
+
+    def __init__(self, *args, vq_interface=False, **kwargs):
+        self.vq_interface = vq_interface
+        super().__init__()
+
+    def encode(self, x, *args, **kwargs):
+        return x
+
+    def decode(self, x, *args, **kwargs):
+        return x
+
+    def quantize(self, x, *args, **kwargs):
+        if self.vq_interface:
+            return x, None, [None, None, None]
+        return x
+
+    def forward(self, x, *args, **kwargs):
+        return x
 
 
 AutoEncoderKL = AutoencoderKL   # VAE/autoencoder.py spells it with a capital E

@@ -350,6 +350,65 @@ def inpaint_blend(x0, noise, a, c, mask, img):
     return out
 
 
+# ---- vector quantisation ------------------------------------------------------------------------------
+_LAYOUTS = {"nchw": 0, "nhwc": 1}
+
+
+def vq_quantize(z, codebook, beta=0.25, z_layout="nchw", zq_layout="nchw", want_zq=True, want_idx=True, want_loss=True):
+    """VectorQuantizer2.forward arithmetic (see include/sdb200.h sdb_vq_quantize) on contiguous fp32 tensors.
+    z [N,D,H,W] ("nchw") or [N,H,W,D] ("nhwc"); codebook [n_e, D].  Returns (z_q in zq_layout, idx int64 [N*H*W] in
+    (n, h, w) order, loss fp32 0-d tensor), each None when not wanted."""
+    require_cuda(z, codebook)
+    _f32c("z", z)
+    _f32c("codebook", codebook)
+    if z_layout not in _LAYOUTS or zq_layout not in _LAYOUTS:
+        raise _lib.SdbError("vq_quantize: layouts are 'nchw' or 'nhwc' (got %r, %r)" % (z_layout, zq_layout))
+    if z.dim() != 4 or codebook.dim() != 2:
+        raise _lib.SdbError("vq_quantize: z must be 4-d and the codebook [n_e, D] (got %s, %s)"
+                            % (tuple(z.shape), tuple(codebook.shape)))
+    if z_layout == "nchw":
+        N, D, H, W_ = z.shape
+    else:
+        N, H, W_, D = z.shape
+    n_e = codebook.shape[0]
+    if codebook.shape[1] != D:
+        raise _lib.SdbError("vq_quantize: codebook %s does not match D=%d of z" % (tuple(codebook.shape), D))
+    M = N * H * W_
+    lib = _L()
+    ws_bytes = lib.sdb_vq_ws_bytes(M, n_e)
+    if ws_bytes < 0:
+        raise _lib.SdbError("vq_quantize: unsupported shape M=%d n_e=%d" % (M, n_e))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=z.device)
+    zq = None
+    if want_zq:
+        zq = torch.empty((N, D, H, W_) if zq_layout == "nchw" else (N, H, W_, D), dtype=torch.float32, device=z.device)
+    idx = torch.empty(M, dtype=torch.int64, device=z.device) if want_idx else None
+    loss = torch.empty((), dtype=torch.float32, device=z.device) if want_loss else None
+    # the GroupNorm kernels' ticket counters: zero between launches, so one buffer per stream serves both
+    counters = _gn_ticket_buffer(z.device, 1) if want_loss else None
+    check(lib.sdb_vq_quantize(ptr(z), _LAYOUTS[z_layout], N, H * W_, D, ptr(codebook), n_e, float(beta), ptr(zq),
+                              _LAYOUTS[zq_layout], ptr(idx), ptr(loss), ptr(ws), ptr(counters), stream_ptr()), "vq_quantize")
+    return zq, idx, loss
+
+
+def vq_codebook_gather(idx, codebook, shape, out_layout="nchw"):
+    """codebook[idx] as an fp32 image: idx int64 with N*H*W entries in (n, h, w) order, shape = (N, H, W) ->
+    [N,D,H,W] ("nchw") or [N,H,W,D] ("nhwc").  Out-of-range indices give NaN rows."""
+    require_cuda(idx, codebook)
+    _f32c("codebook", codebook)
+    N, H, W_ = (int(s) for s in shape)
+    if idx.dtype != torch.int64 or not idx.is_contiguous() or idx.numel() != N * H * W_:
+        raise _lib.SdbError("vq_codebook_gather: idx must be a contiguous int64 tensor of %d indices (got %s %s)"
+                            % (N * H * W_, idx.dtype, tuple(idx.shape)))
+    if out_layout not in _LAYOUTS:
+        raise _lib.SdbError("vq_codebook_gather: layouts are 'nchw' or 'nhwc' (got %r)" % (out_layout,))
+    n_e, D = codebook.shape
+    out = torch.empty((N, D, H, W_) if out_layout == "nchw" else (N, H, W_, D), dtype=torch.float32, device=codebook.device)
+    check(_L().sdb_vq_codebook_gather(ptr(idx), idx.numel(), ptr(codebook), n_e, D, ptr(out), _LAYOUTS[out_layout], H * W_,
+                                      stream_ptr()), "vq_codebook_gather")
+    return out
+
+
 def diag_gaussian(moments, noise=None):
     """moments [N,2C,H,W] fp32 -> (mean, logvar, std, var, sample or None), each [N,C,H,W]
     (DiagonalGaussianDistribution, ldm/modules/distributions/distributions.py:24-37)."""

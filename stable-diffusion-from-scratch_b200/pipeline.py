@@ -4,7 +4,8 @@
 `decode_first_stage` call sites need (ldm/diffusion/ddpm.py:1326-1448, 1083-1156, 1814-1826):
 schedule buffers, `apply_model(x, t, cond)`, `decode_first_stage(z)`.  It owns a `UNetModel`
 (as `model.diffusion_model`, like DiffusionWrapper, ddpm.py:1992-2034, with all five conditioning keys) and an
-`AutoencoderKL`.
+`AutoencoderKL` (or any first stage given as `first_stage_model`: a `VQModelInterface` for the VQ models, built with
+`scale_factor=1.0` and `channels=3`).
 It also carries the reference's ancestral sampler (`sample` / `p_sample_loop` / `progressive_denoising`,
 ddpm.py:1528-1793), whose per-step update runs as one fused kernel (sdb_ddpm_step).
 """
@@ -15,7 +16,7 @@ import torch
 from torch import nn
 
 from . import ops
-from .autoencoder import AutoencoderKL
+from .autoencoder import AutoencoderKL, VQModelInterface
 from .ddim import DDIMSampler
 from .openai_model import UNetModel
 
@@ -167,9 +168,15 @@ class LatentDiffusion(nn.Module):
         return out if x_start.dtype == torch.float32 else out.to(x_start.dtype)
 
     @torch.no_grad()
-    def decode_first_stage(self, z):
-        """ldm/diffusion/ddpm.py:1083-1156: z / scale_factor then first_stage_model.decode."""
+    def decode_first_stage(self, z, predict_cids=False, force_not_quantize=False):
+        """ldm/diffusion/ddpm.py:1083-1156: z / scale_factor then first_stage_model.decode; a VQModelInterface first
+        stage is told whether to quantize (decode(z, force_not_quantize=predict_cids or force_not_quantize)).
+        predict_cids needs the UNet's codebook-id head, which is not built."""
+        if predict_cids:
+            raise NotImplementedError("decode_first_stage(predict_cids=True) needs the UNet n_embed codebook head, which is not built")
         z = 1. / self.scale_factor * z
+        if isinstance(self.first_stage_model, VQModelInterface):
+            return self.first_stage_model.decode(z, force_not_quantize=predict_cids or force_not_quantize)
         return self.first_stage_model.decode(z)
 
     @torch.no_grad()
