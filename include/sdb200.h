@@ -377,6 +377,25 @@ int sdb_vq_quantize(const float* z, int z_layout, int N, int HW, int D, const fl
 int sdb_vq_codebook_gather(const long long* idx, long long M, const float* codebook, int n_e, int D, float* out, int out_layout,
                            int HW, void* stream);
 
+/* ---- patch-distributed fold / unfold: LatentDiffusion's split_input_params branch -----------------------------------
+ * (ldm/diffusion/ddpm.py:1344-1437 apply_model, 1097-1139 decode_first_stage.)  The crop grid of an image of H x W with
+ * crops kh x kw at stride (sh, sw) is Ly = (H - kh) / sh + 1 by Lx = (W - kw) / sw + 1, crop l = ly * Lx + lx with its
+ * origin at (ly * sh, lx * sw).  Crops are stored crop-major, [L*B, C, kh, kw] with row l*B + b, so that the L crops of a
+ * batch of B images are one batch of L*B samples.  Both use 64-bit element indices, never allocate and never sync.
+ *
+ * sdb_patch_unfold: out = unfold(x).view(B, C, kh, kw, L)[..., l] for every l (torch.nn.Unfold, dilation 1, no padding),
+ * x fp32 NCHW [B, C, H, W]; a pure copy. */
+int sdb_patch_unfold(const float* x, int B, int C, int H, int W, int kh, int kw, int sh, int sw, float* out, void* stream);
+/* sdb_patch_fold: out = fold(o * weighting) / fold(weighting) on an fp32 NCHW [B, C, OH, OW] output, o fp32 [L*B, C, KH, KW]
+ * crop-major, with the per-crop weight w_l(p) = wpix[p] (wcrop == NULL) or fl(wpix[p] * wcrop[l]) (the tie breaker), wpix
+ * fp32 [KH*KW], wcrop fp32 [L]:
+ *   out[b, c, y, x] = (sum_l fl(o_l * w_l)) / (sum_l w_l)     over the crops l covering (y, x)
+ * Both sums start at 0.0f and run in fp32 in increasing l, the order of torch's CUDA col2im, so the result is the bits of
+ * the reference's torch.nn.Fold expression.  A pixel no crop covers is 0 / 0 = NaN, as in the reference.  L must equal
+ * Ly * Lx and the grid must lie inside (OH, OW). */
+int sdb_patch_fold(const float* o, int B, int C, int KH, int KW, int Ly, int Lx, int SH, int SW, int OH, int OW,
+                   const float* wpix, const float* wcrop, int L, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

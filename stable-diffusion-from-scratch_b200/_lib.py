@@ -125,6 +125,8 @@ SIGNATURES = {
     "sdb_vq_ws_bytes": (_L, [_L, _I]),
     "sdb_vq_quantize": (_I, [_P, _I, _I, _I, _I, _P, _I, _F, _P, _I, _P, _P, _P, _P, _P]),
     "sdb_vq_codebook_gather": (_I, [_P, _L, _P, _I, _I, _P, _I, _I, _P]),
+    "sdb_patch_unfold": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
+    "sdb_patch_fold": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P]),
 }
 
 

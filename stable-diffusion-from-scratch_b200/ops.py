@@ -409,6 +409,47 @@ def vq_codebook_gather(idx, codebook, shape, out_layout="nchw"):
     return out
 
 
+# ---- patch-distributed fold / unfold (LatentDiffusion.split_input_params) -----------------------------------------------
+def patch_grid(h, w, ks, stride):
+    """(Ly, Lx): the crops of ks at `stride` that fit in h x w, as torch.nn.Unfold counts them."""
+    return (h - ks[0]) // stride[0] + 1, (w - ks[1]) // stride[1] + 1
+
+
+def patch_unfold(x, ks, stride):
+    """x [B,C,H,W] -> its Ly*Lx crops of ks at `stride` as one batch [L*B, C, ks[0], ks[1]] fp32, crop-major (row l*B + b):
+    unfold(x).view(B, C, *ks, L)[..., l] for every l, a pure copy (see include/sdb200.h sdb_patch_unfold)."""
+    require_cuda(x)
+    xf = x.float().contiguous()
+    if xf.dim() != 4:
+        raise _lib.SdbError("patch_unfold: x must be 4-d (got %s)" % (tuple(x.shape),))
+    B, C, H, W_ = xf.shape
+    Ly, Lx = patch_grid(H, W_, ks, stride)
+    out = torch.empty((max(Ly * Lx, 0) * B, C, ks[0], ks[1]), dtype=torch.float32, device=x.device)
+    check(_L().sdb_patch_unfold(ptr(xf), B, C, H, W_, int(ks[0]), int(ks[1]), int(stride[0]), int(stride[1]), ptr(out),
+                                stream_ptr()), "patch_unfold")
+    return out
+
+
+def patch_fold(o, B, grid, stride, out_hw, wpix, wcrop=None):
+    """Crops o [L*B, C, KH, KW] (crop-major) of a Ly x Lx `grid` at `stride` -> fold(o * w) / fold(w) as [B, C, *out_hw] fp32,
+    w = wpix [KH*KW] per pixel, times wcrop [L] per crop when given (see include/sdb200.h sdb_patch_fold)."""
+    require_cuda(o, wpix, wcrop)
+    _f32c("o", o)
+    _f32c("wpix", wpix)
+    _f32c("wcrop", wcrop)
+    if o.dim() != 4 or o.shape[0] % B or wpix.numel() != o.shape[2] * o.shape[3]:
+        raise _lib.SdbError("patch_fold: crops %s do not match B=%d and a weight table of %d" % (tuple(o.shape), B, wpix.numel()))
+    _, C, KH, KW = o.shape
+    Ly, Lx = grid
+    L = o.shape[0] // B
+    if wcrop is not None and wcrop.numel() != L:
+        raise _lib.SdbError("patch_fold: %d crop weights for %d crops" % (wcrop.numel(), L))
+    out = torch.empty((B, C, out_hw[0], out_hw[1]), dtype=torch.float32, device=o.device)
+    check(_L().sdb_patch_fold(ptr(o), B, C, KH, KW, int(Ly), int(Lx), int(stride[0]), int(stride[1]), int(out_hw[0]),
+                              int(out_hw[1]), ptr(wpix), ptr(wcrop), L, ptr(out), stream_ptr()), "patch_fold")
+    return out
+
+
 def diag_gaussian(moments, noise=None):
     """moments [N,2C,H,W] fp32 -> (mean, logvar, std, var, sample or None), each [N,C,H,W]
     (DiagonalGaussianDistribution, ldm/modules/distributions/distributions.py:24-37)."""

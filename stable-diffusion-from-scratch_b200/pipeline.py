@@ -89,7 +89,7 @@ class LatentDiffusion(nn.Module):
     def __init__(self, unet_config=None, first_stage_config=None, timesteps=1000, linear_start=0.00085, linear_end=0.0120,
                  beta_schedule="linear", scale_factor=0.18215, conditioning_key="crossattn", compute_mode=None,
                  unet=None, first_stage_model=None, cond_stage_model=None, v_posterior=0., clip_denoised=True,
-                 log_every_t=100, channels=4, image_size=64):
+                 log_every_t=100, channels=4, image_size=64, cond_stage_key="image"):
         super().__init__()
         # optional text conditioner (Diffusion/config.yaml:69-70: FrozenCLIPEmbedder); None = the caller supplies `context` tensors
         self.cond_stage_model = cond_stage_model
@@ -106,6 +106,10 @@ class LatentDiffusion(nn.Module):
         self.log_every_t = log_every_t
         self.channels = channels
         self.image_size = image_size
+        # read only by the split_input_params branch of apply_model: which conditionings are cut into crops with the latent
+        self.cond_stage_key = cond_stage_key
+        # split_input_params branch: at most this many crops per model call (None = all L crops of a call in one batch)
+        self.patch_batch = None
         self.num_timesteps = int(timesteps)
         betas = make_beta_schedule(beta_schedule, timesteps, linear_start=linear_start, linear_end=linear_end)
         alphas_cumprod = np.cumprod(1. - betas, axis=0)
@@ -132,7 +136,15 @@ class LatentDiffusion(nn.Module):
         return self.betas.device
 
     def apply_model(self, x_noisy, t, cond, return_ids=False):
-        """ldm/diffusion/ddpm.py:1326-1448 without the fold/unfold patch branch."""
+        """ldm/diffusion/ddpm.py:1326-1448.  A non-dict `cond` goes under c_concat ("concat") or c_crossattn (other keys).
+
+        With a `split_input_params` attribute (the reference's patch-distributed branch, ddpm.py:1344-1437) x_noisy is cut
+        into its crops of split_input_params["ks"] at ["stride"], the model is run on every crop, and the outputs are
+        stitched with the border-weighted fold divided by the folded weights.  The reference loops over the L crops; here
+        they run as one batch of L*B samples (at most `patch_batch` crops per call), which gives the same bits because
+        per-sample results do not depend on the batch.  Conditioning: with cond_stage_key in "image", "LR_image",
+        "segmentation", "bbox_img" and a conditioning_key, the single conditioning tensor is cut into the same crops;
+        otherwise every crop gets the whole conditioning."""
         if isinstance(cond, dict):
             pass
         else:
@@ -140,7 +152,147 @@ class LatentDiffusion(nn.Module):
                 cond = [cond]
             key = "c_concat" if self.model.conditioning_key == "concat" else "c_crossattn"
             cond = {key: cond}
+        if hasattr(self, "split_input_params"):
+            assert len(cond) == 1  # the reference's branch takes one conditioning entry
+            assert not return_ids
+            return self._apply_model_split(x_noisy, t, cond)
         return self.model(x_noisy, t, **cond)
+
+    # ---- split_input_params: patch-distributed fold / unfold (ldm/diffusion/ddpm.py:1030-1139, 1344-1437) ----------------
+    SPLIT_IMAGE_KEYS = ("image", "LR_image", "segmentation", "bbox_img")
+
+    def meshgrid(self, h, w):
+        y = torch.arange(0, h).view(h, 1, 1).repeat(1, w, 1)
+        x = torch.arange(0, w).view(1, w, 1).repeat(h, 1, 1)
+        arr = torch.cat([y, x], dim=-1)
+        return arr
+
+    def delta_border(self, h, w):
+        """Normalised distance of each pixel of an h x w crop to the crop's border: 0 at the border, 0.5 at the centre."""
+        lower_right_corner = torch.tensor([h - 1, w - 1]).view(1, 1, 2)
+        arr = self.meshgrid(h, w) / lower_right_corner
+        dist_left_up = torch.min(arr, dim=-1, keepdims=True)[0]
+        dist_right_down = torch.min(1 - arr, dim=-1, keepdims=True)[0]
+        edge_dist = torch.min(torch.cat([dist_left_up, dist_right_down], dim=-1), dim=-1)[0]
+        return edge_dist
+
+    def get_weighting(self, h, w, Ly, Lx, device):
+        """[1, h*w, Ly*Lx] per-pixel crop weights, evaluated on the host; times the clipped per-crop border weight of the
+        Ly x Lx grid with split_input_params["tie_braker"]."""
+        weighting = self.delta_border(h, w)
+        weighting = torch.clip(weighting, self.split_input_params["clip_min_weight"], self.split_input_params["clip_max_weight"], )
+        weighting = weighting.view(1, h * w, 1).repeat(1, 1, Ly * Lx)
+        if self.split_input_params["tie_braker"]:
+            L_weighting = self.delta_border(Ly, Lx)
+            L_weighting = torch.clip(L_weighting, self.split_input_params["clip_min_tie_weight"],
+                                     self.split_input_params["clip_max_tie_weight"])
+            L_weighting = L_weighting.view(1, 1, Ly * Lx)
+            weighting = weighting * L_weighting
+        return weighting.to(device)
+
+    def _patch_weights(self, h, w, Ly, Lx, device):
+        """The device tables of sdb_patch_fold for crops of h x w on a Ly x Lx grid: (wpix [h*w], wcrop [Ly*Lx] or None).
+        fl(wpix[p] * wcrop[l]) is get_weighting's element (p, l).  Cached per geometry, clip values and device, so a
+        sampling step makes no host-to-device copy."""
+        sp = self.split_input_params
+        tie = bool(sp["tie_braker"])
+        clips = (sp["clip_min_weight"], sp["clip_max_weight"]) + ((sp["clip_min_tie_weight"], sp["clip_max_tie_weight"]) if tie else ())
+        key = (h, w, Ly, Lx, clips, tie, torch.device(device))
+        cache = self.__dict__.setdefault("_patch_weight_cache", {})
+        if key not in cache:
+            wpix = torch.clip(self.delta_border(h, w), sp["clip_min_weight"], sp["clip_max_weight"]).reshape(-1)
+            wcrop = None
+            if tie:
+                wcrop = torch.clip(self.delta_border(Ly, Lx), sp["clip_min_tie_weight"], sp["clip_max_tie_weight"]).reshape(-1)
+                wcrop = wcrop.float().contiguous().to(device)
+            cache[key] = (wpix.float().contiguous().to(device), wcrop)
+        return cache[key]
+
+    def _split_geometry(self, h, w, ks, stride, uf=1, df=1):
+        """get_fold_unfold's fold side for an h x w input cut into crops of ks at `stride`: (Ly, Lx), the fold's crop size,
+        its stride and its output size.  uf > 1 (decode) scales the crops up, df > 1 (encode) down."""
+        Ly, Lx = ops.patch_grid(h, w, ks, stride)
+        if uf == 1 and df == 1:
+            return (Ly, Lx), tuple(ks), tuple(stride), (h, w)
+        if ks[0] != ks[1]:
+            # the reference folds with a square (ks[0] * f, ks[0] * f) kernel but weights (ks[0] * f, ks[1] * f) crops
+            raise NotImplementedError("split_input_params: a non-square ks %s with vqf > 1 is not supported" % (tuple(ks),))
+        if uf > 1:
+            return (Ly, Lx), (ks[0] * uf, ks[0] * uf), (stride[0] * uf, stride[1] * uf), (h * uf, w * uf)
+        return (Ly, Lx), (ks[0] // df, ks[0] // df), (stride[0] // df, stride[1] // df), (h // df, w // df)
+
+    def _fold_crops(self, o, B, grid, fks, fstride, out_hw, device):
+        if tuple(o.shape[2:]) != tuple(fks) or o.shape[0] != grid[0] * grid[1] * B:
+            raise ValueError("split_input_params: the crops came back as %s, the fold expects %d x [%d, C, %d, %d]"
+                             % (tuple(o.shape), grid[0] * grid[1], B, fks[0], fks[1]))
+        wpix, wcrop = self._patch_weights(fks[0], fks[1], grid[0], grid[1], device)
+        return ops.patch_fold(o.float().contiguous(), B, grid, fstride, out_hw, wpix, wcrop)
+
+    def _repeat_cond(self, v, n):
+        """v repeated n times along the batch (the same conditioning for n crops), cached per (caller's tensor, data_ptr,
+        _version, n): a UNet that caches its context K/V projections per context tensor keeps hitting across steps."""
+        if not torch.is_tensor(v) or n == 1:
+            return v
+        cache = self.__dict__.setdefault("_split_cond_cache", {})
+        key = (id(v), v.data_ptr(), v._version, n)
+        hit = cache.get(key)
+        if hit is None or hit[0]() is not v:
+            for k in [k for k, (r, _) in cache.items() if r() is None]:
+                del cache[k]
+            if len(cache) >= 8:
+                cache.clear()
+            hit = (weakref.ref(v), v.repeat(n, *((1,) * (v.dim() - 1))))
+            cache[key] = hit
+        return hit[1]
+
+    def _apply_model_split(self, x_noisy, t, cond):
+        sp = self.split_input_params
+        ks, stride = tuple(sp["ks"]), tuple(sp["stride"])
+        B, _, h, w = x_noisy.shape
+        grid, fks, fstride, out_hw = self._split_geometry(h, w, ks, stride)
+        L = grid[0] * grid[1]
+        c_key, c_val = next(iter(cond.items()))
+        if self.cond_stage_key in self.SPLIT_IMAGE_KEYS and self.model.conditioning_key:
+            assert len(c_val) == 1  # one conditioning tensor, cut like the latent
+            c = c_val[0]
+            if not torch.is_tensor(c) or c.dim() != 4 or tuple(c.shape[-2:]) != (h, w):
+                raise ValueError("split_input_params with cond_stage_key %r: the conditioning must be a 4-d tensor of the "
+                                 "latent's size %s (got %s)" % (self.cond_stage_key, (h, w),
+                                                                tuple(c.shape) if torch.is_tensor(c) else type(c).__name__))
+            cc = ops.patch_unfold(c, ks, stride)
+            cond_for = lambda l0, l1: {c_key: [cc[l0 * B:l1 * B]]}
+        elif self.cond_stage_key == "coordinates_bbox":
+            raise NotImplementedError("split_input_params with cond_stage_key 'coordinates_bbox' is not supported")
+        else:
+            def cond_for(l0, l1):
+                rep = lambda v: [self._repeat_cond(e, l1 - l0) for e in v] if isinstance(v, list) else self._repeat_cond(v, l1 - l0)
+                return {k: rep(v) for k, v in cond.items()}
+        z = ops.patch_unfold(x_noisy, ks, stride)
+        n = L if not self.patch_batch else max(1, min(int(self.patch_batch), L))
+        outs = [self.model(z[l0 * B:min(L, l0 + n) * B], t.repeat(min(L, l0 + n) - l0), **cond_for(l0, min(L, l0 + n)))
+                for l0 in range(0, L, n)]
+        assert not isinstance(outs[0], tuple)
+        o = outs[0] if len(outs) == 1 else torch.cat(outs)
+        out = self._fold_crops(o, B, grid, fks, fstride, out_hw, x_noisy.device)
+        return out if x_noisy.dtype == torch.float32 else out.to(x_noisy.dtype)
+
+    def _split_first_stage(self, x, fn, uf=1, df=1):
+        """decode_first_stage / encode_first_stage with split_input_params["patch_distributed_vq"]: ks and stride are
+        reduced to the input size, the crops go through `fn` as one batch, and the results are folded."""
+        sp = self.split_input_params
+        ks, stride = tuple(sp["ks"]), tuple(sp["stride"])
+        B, _, h, w = x.shape
+        if ks[0] > h or ks[1] > w:
+            ks = (min(ks[0], h), min(ks[1], w))
+            print("reducing Kernel")
+        if stride[0] > h or stride[1] > w:
+            stride = (min(stride[0], h), min(stride[1], w))
+            print("reducing stride")
+        grid, fks, fstride, out_hw = self._split_geometry(h, w, ks, stride, uf=uf, df=df)
+        o = fn(ops.patch_unfold(x, ks, stride))
+        if not torch.is_tensor(o):
+            raise NotImplementedError("split_input_params: the first stage returned %s, not a tensor" % type(o).__name__)
+        return self._fold_crops(o, B, grid, fks, fstride, out_hw, x.device)
 
     @torch.no_grad()
     def get_learned_conditioning(self, c):
@@ -171,17 +323,30 @@ class LatentDiffusion(nn.Module):
     def decode_first_stage(self, z, predict_cids=False, force_not_quantize=False):
         """ldm/diffusion/ddpm.py:1083-1156: z / scale_factor then first_stage_model.decode; a VQModelInterface first
         stage is told whether to quantize (decode(z, force_not_quantize=predict_cids or force_not_quantize)).
-        predict_cids needs the UNet's codebook-id head, which is not built."""
+        predict_cids needs the UNet's codebook-id head, which is not built.
+        With split_input_params["patch_distributed_vq"] the latent is cut into crops (ks and stride reduced to its size),
+        all crops are decoded as one batch and the images are stitched by the border-weighted fold at vqf times the size."""
         if predict_cids:
             raise NotImplementedError("decode_first_stage(predict_cids=True) needs the UNet n_embed codebook head, which is not built")
         z = 1. / self.scale_factor * z
         if isinstance(self.first_stage_model, VQModelInterface):
-            return self.first_stage_model.decode(z, force_not_quantize=predict_cids or force_not_quantize)
-        return self.first_stage_model.decode(z)
+            decode = lambda v: self.first_stage_model.decode(v, force_not_quantize=predict_cids or force_not_quantize)
+        else:
+            decode = self.first_stage_model.decode
+        if hasattr(self, "split_input_params") and self.split_input_params["patch_distributed_vq"]:
+            return self._split_first_stage(z, decode, uf=self.split_input_params["vqf"])
+        return decode(z)
 
     @torch.no_grad()
     def encode_first_stage(self, x):
-        """ldm/diffusion/ddpm.py `encode_first_stage`: first_stage_model.encode(x) -> posterior (SURVEY.md §8 f3)."""
+        """ldm/diffusion/ddpm.py `encode_first_stage`: first_stage_model.encode(x) -> posterior (SURVEY.md §8 f3).
+        With split_input_params["patch_distributed_vq"] the image is cut into crops, encoded as one batch and folded at
+        1/vqf of the size; that needs a first stage whose encode returns a tensor (VQModelInterface, IdentityFirstStage)."""
+        if hasattr(self, "split_input_params") and self.split_input_params["patch_distributed_vq"]:
+            if isinstance(self.first_stage_model, AutoencoderKL):
+                raise NotImplementedError("split_input_params: AutoencoderKL.encode returns a distribution, which cannot be folded")
+            self.split_input_params["original_image_size"] = x.shape[-2:]
+            return self._split_first_stage(x, self.first_stage_model.encode, df=self.split_input_params["vqf"])
         return self.first_stage_model.encode(x)
 
     @torch.no_grad()
