@@ -200,7 +200,8 @@ class _VaeNet(nn.Module):
             W3 = 3 * Cc
             o = ops.attention_wide(qkv, qkv[:, Cc:], qkv[:, 2 * Cc:], B, S, S, Cc, float(int(Cc) ** (-0.5)),
                                    (S * W3, W3), (S * W3, W3), (S * W3, W3))
-            out = engine.linear(o.reshape(B * S, Cc), P[("proj_out", id(ab))], residual=x.reshape(B * S, Cc))
+            # rows_per_item: the measured launch plan of this shape (tc_plans, keyed per image) applies
+            out = engine.linear(o.reshape(B * S, Cc), P[("proj_out", id(ab))], residual=x.reshape(B * S, Cc), rows_per_item=S)
             return out.reshape(B, Hh, Ww, Cc)
         q = engine.linear(hn, P[("q", id(ab))], out_dtype=odt)
         k = engine.linear(hn, P[("k", id(ab))], out_dtype=odt)
@@ -219,7 +220,7 @@ class _VaeNet(nn.Module):
                 sc = ops.gemm_simt(qb, kb)
                 pm = ops.softmax_rows(sc, scale)
                 ops.gemm_simt(pm, v, b_kn=True, out=o[b * S:(b + 1) * S])
-        out = engine.linear(o, P[("proj_out", id(ab))], residual=x.reshape(B * S, Cc))
+        out = engine.linear(o, P[("proj_out", id(ab))], residual=x.reshape(B * S, Cc), rows_per_item=S)
         return out.reshape(B, Hh, Ww, Cc)
 
 
