@@ -396,6 +396,33 @@ int sdb_patch_unfold(const float* x, int B, int C, int H, int W, int kh, int kw,
 int sdb_patch_fold(const float* o, int B, int C, int KH, int KW, int Ly, int Lx, int SH, int SW, int OH, int OW,
                    const float* wpix, const float* wcrop, int L, float* out, void* stream);
 
+/* ---- conditioning stages: the embedders and the spatial rescaler of ldm/modules/encoders/modules.py ------------------
+ * sdb_embed_rows replaces TransformerWrapper's `token_emb(x) + pos_emb(x)` (ldm/modules/x_transformer.py, a gather and an
+ * add) and ClassEmbedder's `embedding(c)` (pos_table == NULL):
+ *   out[i] = table[ids[i]] + pos_table[i % seq_len]          fp32 [n_ids, dim], one rounding
+ * table fp32 [vocab, dim], ids int64 [n_ids], pos_table fp32 [>= seq_len, dim] or NULL (seq_len is then ignored).  An id
+ * outside [0, vocab) writes a NaN row and is never dereferenced. */
+int sdb_embed_rows(const float* table, const long long* ids, long long n_ids, int dim, int vocab, const float* pos_table,
+                   int seq_len, float* out, void* stream);
+/* sdb_interpolate_nchw replaces one stage of SpatialRescaler.forward, F.interpolate(x, scale_factor=s, mode=...) or
+ * F.interpolate(x, size=(OH, OW), mode=...) with align_corners=None and recompute_scale_factor=None, and, with `weight`, the
+ * 1x1 nn.Conv2d channel_mapper that follows the last stage.  x fp32 NCHW [N, C, H, W]; out fp32 [N, C, OH, OW], or
+ * [N, Cout, OH, OW] when weight fp32 [Cout, C] (and optional bias fp32 [Cout]) is given: the map is an fp32 dot over the
+ * interpolated channels in increasing order, formed in registers, so the C-channel map at output resolution is never
+ * written.  scale_h / scale_w: the scale factor F.interpolate was given (the coordinate scale is then float(1 / s)), or 0
+ * when the size was given (in / out).  Coordinates and evaluation order are those of torch's CUDA kernels:
+ *   NEAREST   src = min(floor(dst * scale), in - 1)                     (legacy 'nearest', not 'nearest-exact')
+ *   BILINEAR  src = max(scale * (dst + 0.5) - 0.5, 0), i1 = min(i0 + 1, in - 1)
+ *   BICUBIC   A = -0.75, source not clamped, taps clamped to [0, in - 1]
+ *   AREA      adaptive_avg_pool2d windows [floor(o * in / out), ceil((o + 1) * in / out)), summed row-major, / kh / kw
+ * (torch computes a 1 x 1 area output as a mean reduction, whose summation order differs.) */
+#define SDB_INTERP_NEAREST   0
+#define SDB_INTERP_BILINEAR  1
+#define SDB_INTERP_BICUBIC   2
+#define SDB_INTERP_AREA      3
+int sdb_interpolate_nchw(const float* x, int N, int C, int H, int W, int OH, int OW, int mode, double scale_h, double scale_w,
+                         const float* weight, const float* bias, int Cout, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

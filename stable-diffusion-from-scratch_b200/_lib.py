@@ -76,7 +76,7 @@ class AttnArgs(C.Structure):
 
 
 # name -> (restype, argtypes); kept in one table so tests can check it against include/sdb200.h
-_P, _I, _L, _F = C.c_void_p, C.c_int, C.c_longlong, C.c_float
+_P, _I, _L, _F, _D = C.c_void_p, C.c_int, C.c_longlong, C.c_float, C.c_double
 SIGNATURES = {
     "sdb_version": (_I, []),
     "sdb_last_error_string": (C.c_char_p, []),
@@ -127,6 +127,8 @@ SIGNATURES = {
     "sdb_vq_codebook_gather": (_I, [_P, _L, _P, _I, _I, _P, _I, _I, _P]),
     "sdb_patch_unfold": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
     "sdb_patch_fold": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P]),
+    "sdb_embed_rows": (_I, [_P, _P, _L, _I, _I, _P, _I, _P, _P]),
+    "sdb_interpolate_nchw": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _D, _D, _P, _P, _I, _P, _P]),
 }
 
 

@@ -74,7 +74,7 @@ class TextModelOutput(object):
         return (self.last_hidden_state,)[i]
 
 
-class CLIPTextModel(nn.Module):
+class CLIPTextModel(engine.PackedWeights, nn.Module):
     """HF `CLIPTextModel` (text tower only, `last_hidden_state` only), same state-dict keys.  `config`: a dict with the keys of
     CLIP_VIT_L14_TEXT, or an HF CLIPTextConfig.  Extra keyword: compute_mode "bf16" (tensor cores) / "fp32" (SIMT parity mode)."""
 
@@ -92,28 +92,7 @@ class CLIPTextModel(nn.Module):
         self.config = cfg
         self.compute_mode = compute_mode or engine.default_mode()
         self.text_model = CLIPTextTransformer(cfg)
-        self._packed = {}
-        self.register_load_state_dict_post_hook(lambda module, incompatible_keys: module._invalidate())
-
-    def _invalidate(self):
-        self._packed = {}
-        self.__dict__.pop("_param_list", None)
-        self.__dict__.pop("_fp_seen", None)
-
-    def _apply(self, fn, *a, **k):
-        r = super()._apply(fn, *a, **k)
-        self._invalidate()
-        return r
-
-    def _check_weights(self):
-        ps = self.__dict__.get("_param_list")
-        if ps is None:
-            ps = self.__dict__["_param_list"] = list(self.parameters())
-        fp = (ps[0].data_ptr(), ps[0].device, sum(p._version for p in ps))
-        if fp != self.__dict__.get("_fp_seen"):
-            if self.__dict__.get("_fp_seen") is not None:
-                self._invalidate()
-            self.__dict__["_fp_seen"] = fp
+        self._init_packing()
 
     def _pack(self, mode):
         if mode in self._packed:

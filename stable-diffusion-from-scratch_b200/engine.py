@@ -50,6 +50,37 @@ class PackedConv:
         return torch.bfloat16 if self.use_tc else torch.float32
 
 
+class PackedWeights:
+    """Mixin for an nn.Module that keeps per-mode packed copies of its parameters in `self._packed`: the copies are dropped
+    when a state dict is loaded, when the module is moved or cast (`_apply`), and when a parameter is changed in place
+    (`_check_weights`, a fingerprint of the first parameter's storage and every parameter's `_version`).  Call
+    `_init_packing()` in `__init__` and `_check_weights()` before every use of the packed copies."""
+
+    def _init_packing(self):
+        self._packed = {}
+        self.register_load_state_dict_post_hook(lambda module, incompatible_keys: module._invalidate())
+
+    def _invalidate(self):
+        self._packed = {}
+        self.__dict__.pop("_param_list", None)
+        self.__dict__.pop("_fp_seen", None)
+
+    def _apply(self, fn, *a, **k):
+        r = super()._apply(fn, *a, **k)
+        self._invalidate()
+        return r
+
+    def _check_weights(self):
+        ps = self.__dict__.get("_param_list")
+        if ps is None:
+            ps = self.__dict__["_param_list"] = list(self.parameters())
+        fp = (ps[0].data_ptr(), ps[0].device, sum(p._version for p in ps))
+        if fp != self.__dict__.get("_fp_seen"):
+            if self.__dict__.get("_fp_seen") is not None:
+                self._invalidate()
+            self.__dict__["_fp_seen"] = fp
+
+
 class PackedLinear:
     def __init__(self, weight, bias, mode, geglu=False):
         self.n, self.k = weight.shape
@@ -104,15 +135,17 @@ def linear(x, pl, residual=None, out_dtype=torch.float32, col_group=0, col_group
     return ops.gemm_simt(x2, pl.w, pl.bias, residual=residual, out_dtype=out_dtype)
 
 
-def attention_fp32(q, k, v, B, H, Sq, Sk, d, scale):
+def attention_fp32(q, k, v, B, H, Sq, Sk, d, scale, ld=None):
     """fp32 unfused attention: scores = q k^T (batched over (b, h)), row softmax, out = P v.
-    q [B*Sq, H*d], k/v [B*Sk, H*d] fp32 -> [B*Sq, H*d] fp32."""
+    q [B*Sq, H*d], k/v [B*Sk, H*d] fp32 -> [B*Sq, H*d] fp32.  ld: the row stride of q, k and v in elements when they are
+    column blocks of one wider tensor (e.g. the q | k | v projection), else H*d."""
     Cc = H * d
+    ld = Cc if ld is None else ld
     scores = torch.empty((B, H, Sq, Sk), dtype=torch.float32, device=q.device)
-    ops.gemm_simt(q, k, out=scores, M=Sq, N=Sk, K=d, lda=Cc, ldb=Cc, ldc=Sk, batch=(B, H),
-                  sa=(Sq * Cc, d), sb=(Sk * Cc, d), sc=(H * Sq * Sk, Sq * Sk))
+    ops.gemm_simt(q, k, out=scores, M=Sq, N=Sk, K=d, lda=ld, ldb=ld, ldc=Sk, batch=(B, H),
+                  sa=(Sq * ld, d), sb=(Sk * ld, d), sc=(H * Sq * Sk, Sq * Sk))
     P = ops.softmax_rows(scores, scale)
     out = torch.empty((B * Sq, Cc), dtype=torch.float32, device=q.device)
-    ops.gemm_simt(P, v, out=out, b_kn=True, M=Sq, N=d, K=Sk, lda=Sk, ldb=Cc, ldc=Cc, batch=(B, H),
-                  sa=(H * Sq * Sk, Sq * Sk), sb=(Sk * Cc, d), sc=(Sq * Cc, d))
+    ops.gemm_simt(P, v, out=out, b_kn=True, M=Sq, N=d, K=Sk, lda=Sk, ldb=ld, ldc=Cc, batch=(B, H),
+                  sa=(H * Sq * Sk, Sq * Sk), sb=(Sk * ld, d), sc=(Sq * Cc, d))
     return out

@@ -5,6 +5,7 @@ torch is used for allocation (`torch.empty`) and pointers only.  Activations are
 images [N, H, W, C], tokens [rows, C].
 """
 import ctypes as C
+import math
 import os
 
 import torch
@@ -447,6 +448,77 @@ def patch_fold(o, B, grid, stride, out_hw, wpix, wcrop=None):
     out = torch.empty((B, C, out_hw[0], out_hw[1]), dtype=torch.float32, device=o.device)
     check(_L().sdb_patch_fold(ptr(o), B, C, KH, KW, int(Ly), int(Lx), int(stride[0]), int(stride[1]), int(out_hw[0]),
                               int(out_hw[1]), ptr(wpix), ptr(wcrop), L, ptr(out), stream_ptr()), "patch_fold")
+    return out
+
+
+# ---- conditioning stages (ldm/modules/encoders/modules.py) ------------------------------------------------------------
+def embed_rows(table, ids, pos=None, seq_len=0):
+    """table[ids] (+ pos[i % seq_len] for flat row i) as fp32 [n, dim] in one launch (see include/sdb200.h sdb_embed_rows):
+    TransformerWrapper's token_emb(x) + pos_emb(x), or nn.Embedding with pos None.  An id outside [0, vocab) gives a NaN
+    row."""
+    require_cuda(table, ids, pos)
+    _f32c("table", table)
+    _f32c("pos", pos)
+    if table.dim() != 2 or table.numel() == 0:
+        raise _lib.SdbError("embed_rows: table must be a non-empty [vocab, dim] tensor (got %s)" % (tuple(table.shape),))
+    if ids.dtype != torch.int64 or not ids.is_contiguous() or ids.numel() == 0:
+        raise _lib.SdbError("embed_rows: ids must be a non-empty contiguous int64 tensor (got %s %s)" % (ids.dtype, tuple(ids.shape)))
+    vocab, dim = table.shape
+    if pos is not None and (pos.dim() != 2 or pos.shape[1] != dim or not 0 < seq_len <= pos.shape[0]):
+        raise _lib.SdbError("embed_rows: position table %s cannot serve seq_len=%d rows of dim %d" % (tuple(pos.shape), seq_len, dim))
+    out = torch.empty((ids.numel(), dim), dtype=torch.float32, device=table.device)
+    check(_L().sdb_embed_rows(ptr(table), ptr(ids), ids.numel(), dim, vocab, ptr(pos), int(seq_len) if pos is not None else 0,
+                              ptr(out), stream_ptr()), "embed_rows")
+    return out
+
+
+INTERP_MODES = {"nearest": 0, "bilinear": 1, "bicubic": 2, "area": 3}
+
+
+def interpolate_size(hw, scale_factor=None, size=None):
+    """F.interpolate's output size of a 4-d input: `size`, or floor(in * scale_factor) per axis (recompute_scale_factor=None)."""
+    if (scale_factor is None) == (size is None):
+        raise ValueError("interpolate: give exactly one of size and scale_factor")
+    if size is not None:
+        return tuple(int(v) for v in ((size, size) if isinstance(size, int) else size))
+    s = (scale_factor, scale_factor) if isinstance(scale_factor, (int, float)) else tuple(scale_factor)
+    return tuple(int(math.floor(float(n) * float(f))) for n, f in zip(hw, s))
+
+
+def interpolate(x, scale_factor=None, size=None, mode="nearest", weight=None, bias=None):
+    """One F.interpolate(x, size=size / scale_factor=scale_factor, mode=mode) of an NCHW fp32 tensor, align_corners=None,
+    recompute_scale_factor=None (see include/sdb200.h sdb_interpolate_nchw).  weight [Cout, C] (or a 1x1 conv weight
+    [Cout, C, 1, 1]) with optional bias [Cout] applies the 1x1 channel map to the result in the same launch."""
+    if mode in ("linear", "trilinear"):
+        raise NotImplementedError("interpolate: got 4D input, but %s mode needs %dD input" % (mode, 3 if mode == "linear" else 5))
+    if mode not in INTERP_MODES:
+        raise ValueError("interpolate: mode %r is not one of %s" % (mode, tuple(INTERP_MODES)))
+    require_cuda(x, weight, bias)
+    _f32c("x", x)
+    if x.dim() != 4:
+        raise _lib.SdbError("interpolate: x must be 4-d NCHW (got %s)" % (tuple(x.shape),))
+    N, Cc, H, W_ = x.shape
+    OH, OW = interpolate_size((H, W_), scale_factor, size)
+    if scale_factor is None:
+        sh = sw = 0.0
+    else:
+        sh, sw = (float(scale_factor),) * 2 if isinstance(scale_factor, (int, float)) else (float(f) for f in scale_factor)
+        if sh <= 0 or sw <= 0:
+            raise _lib.SdbError("interpolate: scale_factor must be positive (got %s)" % (scale_factor,))
+    Cout = 0
+    if weight is not None:
+        weight = weight.reshape(weight.shape[0], -1)
+        _f32c("weight", weight)
+        _f32c("bias", bias)
+        Cout = weight.shape[0]
+        if weight.shape[1] != Cc or (bias is not None and bias.numel() != Cout):
+            raise _lib.SdbError("interpolate: channel map %s / bias %s does not map %d channels" % (
+                tuple(weight.shape), None if bias is None else tuple(bias.shape), Cc))
+    elif bias is not None:
+        raise _lib.SdbError("interpolate: a bias needs the channel-map weight")
+    out = torch.empty((N, Cout or Cc, OH, OW), dtype=torch.float32, device=x.device)
+    check(_L().sdb_interpolate_nchw(ptr(x), N, Cc, H, W_, OH, OW, INTERP_MODES[mode], sh, sw, ptr(weight), ptr(bias), Cout,
+                                    ptr(out), stream_ptr()), "interpolate_nchw")
     return out
 
 

@@ -16,7 +16,7 @@ import torch
 from torch import nn
 
 from . import ops
-from .autoencoder import AutoencoderKL, VQModelInterface
+from .autoencoder import AutoencoderKL, DiagonalGaussianDistribution, VQModelInterface
 from .ddim import DDIMSampler
 from .openai_model import UNetModel
 
@@ -89,15 +89,24 @@ class LatentDiffusion(nn.Module):
     def __init__(self, unet_config=None, first_stage_config=None, timesteps=1000, linear_start=0.00085, linear_end=0.0120,
                  beta_schedule="linear", scale_factor=0.18215, conditioning_key="crossattn", compute_mode=None,
                  unet=None, first_stage_model=None, cond_stage_model=None, v_posterior=0., clip_denoised=True,
-                 log_every_t=100, channels=4, image_size=64, cond_stage_key="image"):
+                 log_every_t=100, channels=4, image_size=64, cond_stage_key="image", cond_stage_config=None,
+                 cond_stage_forward=None, cond_stage_trainable=False):
         super().__init__()
-        # optional text conditioner (Diffusion/config.yaml:69-70: FrozenCLIPEmbedder); None = the caller supplies `context` tensors
+        # optional conditioner (Diffusion/config.yaml:69-70: FrozenCLIPEmbedder; sdb200.encoders for the other stages);
+        # None = the caller supplies the conditioning tensors.  cond_stage_config picks one by the reference's special values.
         self.cond_stage_model = cond_stage_model
+        if cond_stage_config == "__is_unconditional__":
+            conditioning_key = None                      # ldm/diffusion/ddpm.py LatentDiffusion.__init__
+        # sampling only: accepted for the reference's configs, no gradient path is built
+        self.cond_stage_trainable = cond_stage_trainable
+        self.cond_stage_forward = cond_stage_forward
         unet = unet if unet is not None else UNetModel(**(unet_config or SD_UNET_CONFIG), compute_mode=compute_mode)
         self.model = DiffusionWrapper(unet, conditioning_key)
         if first_stage_model is None and first_stage_config is not False:
             first_stage_model = AutoencoderKL(ddconfig=(first_stage_config or SD_VAE_DDCONFIG), embed_dim=4, compute_mode=compute_mode)
         self.first_stage_model = first_stage_model
+        if cond_stage_config is not None:
+            self.instantiate_cond_stage(cond_stage_config)
         self.scale_factor = scale_factor
         self.parameterization = "eps"
         self.shorten_cond_schedule = False
@@ -294,12 +303,32 @@ class LatentDiffusion(nn.Module):
             raise NotImplementedError("split_input_params: the first stage returned %s, not a tensor" % type(o).__name__)
         return self._fold_crops(o, B, grid, fks, fstride, out_hw, x.device)
 
+    def instantiate_cond_stage(self, config):
+        """ldm/diffusion/ddpm.py `instantiate_cond_stage` for its two special values: "__is_first_stage__" conditions on the
+        first stage's encoding (the inpainting LDM), "__is_unconditional__" has no conditioner.  A `target:` config is not
+        instantiated here: build the stage (sdb200.encoders) and pass it as `cond_stage_model`."""
+        if config not in ("__is_first_stage__", "__is_unconditional__"):
+            raise NotImplementedError("cond_stage_config %r: only '__is_first_stage__' and '__is_unconditional__' are "
+                                      "resolved here; pass the conditioning stage as cond_stage_model" % (config,))
+        assert not self.cond_stage_trainable, "a trainable cond stage cannot be %s" % config
+        if self.cond_stage_model is not None:
+            raise ValueError("cond_stage_config %r and a cond_stage_model were both given" % (config,))
+        self.cond_stage_model = self.first_stage_model if config == "__is_first_stage__" else None
+
     @torch.no_grad()
     def get_learned_conditioning(self, c):
-        """ldm/diffusion/ddpm.py `get_learned_conditioning`: cond_stage_model.encode(c) (text or token ids -> [B, 77, 768])."""
+        """ldm/diffusion/ddpm.py `get_learned_conditioning`: getattr(cond_stage_model, cond_stage_forward)(c) when
+        cond_stage_forward is set, else cond_stage_model.encode(c) (the distribution's mode when encode returns a
+        DiagonalGaussianDistribution) or, without an encode method, cond_stage_model(c)."""
         assert self.cond_stage_model is not None, "no cond_stage_model was given"
+        if self.cond_stage_forward is not None:
+            assert hasattr(self.cond_stage_model, self.cond_stage_forward)
+            return getattr(self.cond_stage_model, self.cond_stage_forward)(c)
         if hasattr(self.cond_stage_model, "encode") and callable(self.cond_stage_model.encode):
-            return self.cond_stage_model.encode(c)
+            c = self.cond_stage_model.encode(c)
+            if isinstance(c, DiagonalGaussianDistribution):
+                c = c.mode()
+            return c
         return self.cond_stage_model(c)
 
     def q_sample_coefficients(self, t):
