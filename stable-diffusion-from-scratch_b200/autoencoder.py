@@ -86,53 +86,18 @@ def make_attn(in_channels, attn_type="vanilla"):
     raise NotImplementedError("sdb200 VAE: linear attention is outside the hot path")
 
 
-def _fingerprint(module):
-    """(first parameter's address, device, sum of parameter versions): changes when parameters are replaced, moved or
-    written in place (load through a parent module, EMA copy_to, ...)."""
-    ps = module.__dict__.get("_param_list")
-    if ps is None:
-        ps = module.__dict__["_param_list"] = list(module.parameters())
-    return (ps[0].data_ptr(), ps[0].device, sum(p._version for p in ps))
-
-
 FUSED_ATTN_CHANNELS = (256, 512)     # head widths of tc_attention_wide_kernel
 
 
-class _VaeNet(nn.Module):
+class _VaeNet(engine.PackedWeights, nn.Module):
     """Packing and block execution shared by Encoder and Decoder."""
     fused_attention = True           # False: AttnBlock as three GEMMs + row softmax per image (the round-1 path, kept for A/B)
 
     def __init__(self):
         super().__init__()
-        # a parent's load_state_dict recurses through _load_from_state_dict and never reaches the override below
-        self.register_load_state_dict_post_hook(lambda module, incompatible_keys: module._invalidate())
+        self._init_packing()
 
-    def _invalidate(self):
-        self._packed = {}
-        self.__dict__.pop("_param_list", None)
-        self.__dict__.pop("_fp_seen", None)
-
-    def _check_weights(self):
-        fp = _fingerprint(self)
-        if fp != self.__dict__.get("_fp_seen"):
-            if self.__dict__.get("_fp_seen") is not None:
-                self._invalidate()
-            self.__dict__["_fp_seen"] = fp
-
-    def load_state_dict(self, *a, **k):
-        r = super().load_state_dict(*a, **k)
-        self._invalidate()
-        return r
-
-    def _apply(self, fn, *a, **k):
-        r = super()._apply(fn, *a, **k)
-        self._invalidate()
-        return r
-
-    def _pack(self, mode):
-        self._check_weights()
-        if mode in self._packed:
-            return self._packed[mode]
+    def _build_pack(self, mode):
         P = {}
         for m in self.modules():
             if isinstance(m, ResnetBlock):
@@ -161,7 +126,6 @@ class _VaeNet(nn.Module):
                 P[("down", id(m))] = PackedConv(m.conv.weight, m.conv.bias, mode, stride=2, pad=0, pad_hi=1)
         P["conv_in"] = PackedConv(self.conv_in.weight, self.conv_in.bias, mode)
         P["conv_out"] = PackedConv(self.conv_out.weight, self.conv_out.bias, mode)
-        self._packed[mode] = P
         return P
 
     @staticmethod
@@ -269,11 +233,10 @@ class Encoder(_VaeNet):
         self.mid.block_2 = ResnetBlock(in_channels=block_in, out_channels=block_in, temb_channels=self.temb_ch, dropout=dropout)
         self.norm_out = Normalize(block_in)
         self.conv_out = nn.Conv2d(block_in, 2 * z_channels if double_z else z_channels, kernel_size=3, stride=1, padding=1)
-        self._packed = {}
 
     def _forward_nhwc(self, x, mode):
         """x [N,H,W,in_channels] fp32 -> [N,H/2^(L-1),W/2^(L-1),2*z_channels] fp32 (Encoder.forward, model.py:434-465)."""
-        P = self._pack(mode)
+        P = self.packed(mode)
         ci = P["conv_in"]
         h = engine.conv(x if ci.in_dtype == torch.float32 else ops.cast_concat(x, None, out_dtype=torch.bfloat16), ci, want_stats=True)
         for i_level in range(self.num_resolutions):
@@ -299,6 +262,7 @@ class Encoder(_VaeNet):
         from ._lib import require_cuda
         with torch.cuda.device(x.device):
             require_cuda(x)
+            self._check_weights()
             h = ops.nchw_to_nhwc(x.float().contiguous())
             out = ops.nhwc_to_nchw(self._forward_nhwc(h, self.compute_mode))
         return out if x.dtype == torch.float32 else out.to(x.dtype)
@@ -388,10 +352,9 @@ class Decoder(_VaeNet):
             self.up.insert(0, up)
         self.norm_out = Normalize(block_in)
         self.conv_out = nn.Conv2d(block_in, out_ch, kernel_size=3, stride=1, padding=1)
-        self._packed = {}
 
     def _forward_nhwc(self, z, mode):
-        P = self._pack(mode)
+        P = self.packed(mode)
         h = engine.conv(z, P["conv_in"], want_stats=True)
         h = self._resnet(self.mid.block_1, P, mode, h)
         if isinstance(self.mid.attn_1, AttnBlock):
@@ -418,6 +381,7 @@ class Decoder(_VaeNet):
         from ._lib import require_cuda
         with torch.cuda.device(z.device):
             require_cuda(z)
+            self._check_weights()
             self.last_z_shape = z.shape
             h = ops.nchw_to_nhwc(z.float().contiguous())
             out = ops.nhwc_to_nchw(self._forward_nhwc(h, self.compute_mode))
@@ -425,8 +389,9 @@ class Decoder(_VaeNet):
 
 
 class _FirstStage(nn.Module):
-    """What AutoencoderKL and VQModel share: Encoder / Decoder compute mode, checkpoint loading, the fp32 SIMT packing
-    of the 1x1 quant_conv / post_quant_conv, and the micro-batched encode / decode loops."""
+    """What AutoencoderKL and VQModel share: Encoder / Decoder compute mode, checkpoint loading, and the micro-batched
+    encode / decode loops with the 1x1 quant_conv / post_quant_conv on the fp32 SIMT kernel (tiny C_in, both modes).  A
+    1x1 fp32 PackedConv is a view of the layer's parameters, so it is built per call and never stale."""
 
     @property
     def compute_mode(self):
@@ -445,42 +410,14 @@ class _FirstStage(nn.Module):
                     del sd[k]
         self.load_state_dict(sd, strict=False)
 
-    def _invalidate(self):
-        self.decoder._invalidate()
-        self.encoder._invalidate()
-        self._pq = None
-        self._q = None
-
-    def load_state_dict(self, *a, **k):
-        r = super().load_state_dict(*a, **k)
-        self._invalidate()
-        return r
-
-    def _apply(self, fn, *a, **k):
-        r = super()._apply(fn, *a, **k)
-        self._invalidate()
-        return r
-
-    _pq = None
-    _q = None
-
-    def _packed_1x1(self, slot, conv):
-        """quant_conv / post_quant_conv packed for the fp32 SIMT kernel (C_in = 3 ... 8), re-packed whenever the layer's
-        parameters were replaced or written in place."""
-        fp = (conv.weight.data_ptr(), conv.weight._version, conv.bias.data_ptr(), conv.bias._version)
-        cur = getattr(self, slot)
-        if cur is None or cur[0] != fp:
-            cur = (fp, PackedConv(conv.weight, conv.bias, "fp32"))
-            setattr(self, slot, cur)
-        return cur[1]
-
     def _encode_quant_conv(self, x):
         """Encoder then quant_conv, in micro-batches of `micro_batch` images: x [N,C,H,W] -> [N,C',h,w] fp32 NCHW."""
         from ._lib import require_cuda
         with torch.cuda.device(x.device):
             require_cuda(x)
+            self.encoder._check_weights()
             mode = self.encoder.compute_mode
-            qc = self._packed_1x1("_q", self.quant_conv)                                   # tiny C_in: SIMT fp32 kernel in both modes
+            qc = PackedConv(self.quant_conv.weight, self.quant_conv.bias, "fp32")
             xf = x.float().contiguous()
             outs = []
             for i in range(0, xf.shape[0], self.micro_batch):
@@ -495,8 +432,9 @@ class _FirstStage(nn.Module):
         from ._lib import require_cuda
         with torch.cuda.device(z.device):
             require_cuda(z)
+            self.decoder._check_weights()
             mode = self.decoder.compute_mode
-            pq = self._packed_1x1("_pq", self.post_quant_conv)                             # tiny C_in: SIMT fp32 kernel in both modes
+            pq = PackedConv(self.post_quant_conv.weight, self.post_quant_conv.bias, "fp32")
             zf = z.float().contiguous()
             N = zf.shape[0]
             outs = []

@@ -94,11 +94,7 @@ class CLIPTextModel(engine.PackedWeights, nn.Module):
         self.text_model = CLIPTextTransformer(cfg)
         self._init_packing()
 
-    def _pack(self, mode):
-        if mode in self._packed:
-            return self._packed[mode]
-        if mode not in engine.MODES:
-            raise ValueError("compute_mode must be one of %s" % (engine.MODES,))
+    def _build_pack(self, mode):
         tm = self.text_model
         P = {"tok": tm.embeddings.token_embedding.weight.detach().float().contiguous(),
              "pos": tm.embeddings.position_embedding.weight.detach().float().contiguous(), "pos_rep": {}}
@@ -109,12 +105,11 @@ class CLIPTextModel(engine.PackedWeights, nn.Module):
             P[("out", i)] = PackedLinear(a.out_proj.weight, a.out_proj.bias, mode)
             P[("fc1", i)] = PackedLinear(L.mlp.fc1.weight, L.mlp.fc1.bias, mode)
             P[("fc2", i)] = PackedLinear(L.mlp.fc2.weight, L.mlp.fc2.bias, mode)
-        self._packed[mode] = P
         return P
 
     def _forward_tokens(self, ids, mode):
         cfg = self.config
-        P = self._pack(mode)
+        P = self.packed(mode)
         B, S = ids.shape
         D, H = cfg["hidden_size"], cfg["num_attention_heads"]
         d = D // H
@@ -136,7 +131,7 @@ class CLIPTextModel(engine.PackedWeights, nn.Module):
                                      (S * W3, W3, d), (S * W3, W3, d), (S * W3, W3, d), dense=True, causal=True)
                 o = o.reshape(B * S, D)
             else:
-                o = self._attn_fp32_causal(qkv, B, H, S, d, scale)
+                o = engine.attention_fp32(qkv, qkv[:, D:], qkv[:, 2 * D:], B, H, S, S, d, scale, causal=True)
             x = engine.linear(o, P[("out", i)], residual=x, rows_per_item=S)
             a = ops.layernorm(x, L.layer_norm2.weight, L.layer_norm2.bias, L.layer_norm2.eps, out_dtype=odt)
             h = engine.linear(a, P[("fc1", i)], rows_per_item=S)                                # fp32 [B*S, 4D]
@@ -144,22 +139,6 @@ class CLIPTextModel(engine.PackedWeights, nn.Module):
             x = engine.linear(h, P[("fc2", i)], residual=x, rows_per_item=S)
         fl = self.text_model.final_layer_norm
         return ops.layernorm(x, fl.weight, fl.bias, fl.eps, out_dtype=torch.float32).reshape(B, S, D)
-
-    @staticmethod
-    def _attn_fp32_causal(qkv, B, H, S, d, scale):
-        """fp32 parity mode: batched SIMT GEMMs + the causal row softmax."""
-        D = H * d
-        W3 = 3 * D
-        dev = qkv.device
-        scores = torch.empty((B, H, S, S), dtype=torch.float32, device=dev)
-        flat = qkv.reshape(-1)
-        ops.gemm_simt(flat, flat[D:], out=scores, M=S, N=S, K=d, lda=W3, ldb=W3, ldc=S, batch=(B, H),
-                      sa=(S * W3, d), sb=(S * W3, d), sc=(H * S * S, S * S))
-        Pm = ops.softmax_rows_causal(scores, scale, S)
-        out = torch.empty((B * S, D), dtype=torch.float32, device=dev)
-        ops.gemm_simt(Pm, flat[2 * D:], out=out, b_kn=True, M=S, N=d, K=S, lda=S, ldb=W3, ldc=D, batch=(B, H),
-                      sa=(H * S * S, S * S), sb=(S * W3, d), sc=(S * D, d))
-        return out
 
     @torch.no_grad()
     def forward(self, input_ids=None, **kwargs):

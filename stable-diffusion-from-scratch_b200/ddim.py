@@ -6,12 +6,10 @@ Same constructor / method signatures and the same duck-typed `model` interface a
 Schedule tables are built on the host with the reference's own mixed torch/numpy arithmetic so the
 four per-step coefficients are bit-identical fp32 values.
 """
-import weakref
-
 import numpy as np
 import torch
 
-from . import ops
+from . import engine, ops
 
 
 def make_ddim_timesteps(ddim_discr_method, num_ddim_timesteps, num_ddpm_timesteps, verbose=True):
@@ -47,11 +45,10 @@ def _f32(v):
 
 
 class DDIMSampler(object):
-    _cfg_ctx = None
-
     def __init__(self, model, schedule="linear", **kwargs):
         super().__init__()
         self.model = model
+        self._cfg_ctx = engine.TensorMemo(1)      # the CFG conditioning of one 2B call, built once per (uc, c) pair
         self.ddpm_num_timesteps = model.num_timesteps
         self.schedule = schedule
         # The reference always draws torch.randn in p_sample_ddim, even when sigma == 0 (util.py:264-267).  The draw cannot
@@ -219,12 +216,9 @@ class DDIMSampler(object):
         elif isinstance(c, torch.Tensor) and isinstance(unconditional_conditioning, torch.Tensor):
             # one 2B call like the reference (ddim.py:176-179).  The concatenated conditioning is built once per (uc, c)
             # pair and reused for every step, so a UNet that caches the context K/V projections keeps hitting its cache.
-            hit = self._cfg_ctx
-            key = (c.data_ptr(), c._version, unconditional_conditioning.data_ptr(), unconditional_conditioning._version)
-            if hit is None or hit[0] != key or hit[1]() is not c or hit[2]() is not unconditional_conditioning:
-                hit = (key, weakref.ref(c), weakref.ref(unconditional_conditioning), torch.cat([unconditional_conditioning, c]))
-                self._cfg_ctx = hit
-            e_uncond, e_t = self.model.apply_model(torch.cat([x] * 2), torch.cat([t] * 2), hit[3]).chunk(2)
+            uc = unconditional_conditioning
+            c_in = self._cfg_ctx.get((c, uc), "tensor", lambda: torch.cat([uc, c]))
+            e_uncond, e_t = self.model.apply_model(torch.cat([x] * 2), torch.cat([t] * 2), c_in).chunk(2)
             e_uncond, e_t = e_uncond.contiguous(), e_t.contiguous()
         elif self._cfg_dict_pairable(c, unconditional_conditioning):
             # image-conditioned ("concat" / "hybrid") models: one 2B call as well, every entry of the two dicts joined along the
@@ -288,19 +282,14 @@ class DDIMSampler(object):
         return True
 
     def _cfg_dict_in(self, c, uc):
-        """{k: [cat([uc[k][i], c[k][i]]) ...]} (tensor entries: cat([uc[k], c[k]])), built once per (uc, c) pair: the key holds
-        every tensor's data_ptr and _version, and a hit also needs each cached weakref to still be the same live object."""
+        """{k: [cat([uc[k][i], c[k][i]]) ...]} (tensor entries: cat([uc[k], c[k]])), built once per (uc, c) pair of live,
+        unwritten tensors."""
         leaves = [(k, i, uc[k][i] if isinstance(uc[k], list) else uc[k], v)
                   for k in sorted(c) for i, v in (enumerate(c[k]) if isinstance(c[k], list) else [(None, c[k])])]
-        key = ("dict",) + tuple((k, i, u.data_ptr(), u._version, v.data_ptr(), v._version) for k, i, u, v in leaves)
-        hit = self._cfg_ctx
-        if (hit is None or hit[0] != key
-                or any(ru() is not u or rv() is not v for (ru, rv), (_, _, u, v) in zip(hit[1], leaves))):
-            c_in = {k: ([torch.cat([uc[k][i], c[k][i]]) for i in range(len(c[k]))] if isinstance(c[k], list)
-                        else torch.cat([uc[k], c[k]])) for k in c}
-            hit = (key, [(weakref.ref(u), weakref.ref(v)) for _, _, u, v in leaves], c_in)
-            self._cfg_ctx = hit
-        return hit[2]
+        build = lambda: {k: ([torch.cat([uc[k][i], c[k][i]]) for i in range(len(c[k]))] if isinstance(c[k], list)
+                             else torch.cat([uc[k], c[k]])) for k in c}
+        tensors = [t for _, _, u, v in leaves for t in (u, v)]
+        return self._cfg_ctx.get(tensors, ("dict",) + tuple((k, i) for k, i, _, _ in leaves), build)
 
     @torch.no_grad()
     def stochastic_encode(self, x0, t, use_original_steps=False, noise=None):

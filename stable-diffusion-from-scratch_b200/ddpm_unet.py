@@ -111,7 +111,7 @@ class AttentionUpBlock(_Block):
         super().__init__(in_channels, out_channels, num_layers, time_emb_channels, num_groups, num_att_heads, upsample=upsample)
 
 
-class UNet(nn.Module):
+class UNet(engine.PackedWeights, nn.Module):
     """DDPM/models/unet.py:11-81."""
 
     def __init__(self, image_size=256, input_channels=3, compute_mode=None):
@@ -129,21 +129,9 @@ class UNet(nn.Module):
             ConvUpBlock(512 + 512, 512, 2, T, 32), AttentionUpBlock(512 + 256, 256, 2, T, 32, 4),
             ConvUpBlock(256 + 256, 256, 2, T, 32), ConvUpBlock(256 + 128, 128, 2, T, 32), ConvUpBlock(128 + 128, 128, 2, T, 32)])
         self.output_conv = nn.Sequential(nn.GroupNorm(num_channels=256, num_groups=32), nn.SiLU(), nn.Conv2d(256, 3, 3, padding=1))
-        self._packed = {}
+        self._init_packing()
 
-    def load_state_dict(self, *a, **k):
-        r = super().load_state_dict(*a, **k)
-        self._packed = {}
-        return r
-
-    def _apply(self, fn, *a, **k):
-        r = super()._apply(fn, *a, **k)
-        self._packed = {}
-        return r
-
-    def _pack(self, mode):
-        if mode in self._packed:
-            return self._packed[mode]
+    def _build_pack(self, mode):
         P = {}
         dev = self.initial_conv.weight.device
         P["pe"] = self.positional_encoding[0].pe_matrix.to(dev).float().contiguous()
@@ -173,7 +161,6 @@ class UNet(nn.Module):
         P["tw"], P["tb"] = torch.cat(ws, 0).contiguous(), torch.cat(bs, 0).contiguous()
         P["ic"] = PackedConv(self.initial_conv.weight, self.initial_conv.bias, mode)
         P["oc"] = PackedConv(self.output_conv[2].weight, self.output_conv[2].bias, mode)
-        self._packed[mode] = P
         return P
 
     @staticmethod
@@ -217,9 +204,8 @@ class UNet(nn.Module):
             o = ops.attention_tc(qkv, qkv[:, H * dp:], qkv[:, 2 * H * dp:], B, H, S, S, d, dp, scale,
                                  (S * W3, W3, dp), (S * W3, W3, dp), (S * W3, W3, dp)).reshape(B * S, Cc)
         else:
-            from .openai_model import UNetModel
             qkv = engine.linear(t, P[("qkv", id(ab))])
-            o = UNetModel._attn_fp32(qkv, 3 * Cc, 0, qkv, 3 * Cc, Cc, qkv, 3 * Cc, 2 * Cc, B, H, S, S, d, scale)
+            o = engine.attention_fp32(qkv, qkv[:, Cc:], qkv[:, 2 * Cc:], B, H, S, S, d, scale)
         y = engine.linear(o, P[("fp", id(ab))], residual=t).reshape(B, Hh, Ww, Cc)      # final_projection + input
         return ops.groupnorm(y, ab.norm.weight, ab.norm.bias, ab.norm.eps, act=0, out_dtype=torch.float32,
                              groups=ab.norm.num_groups, exact=(mode == "fp32"))
@@ -242,8 +228,9 @@ class UNet(nn.Module):
     def forward(self, input_tensor, time):
         from ._lib import require_cuda
         require_cuda(input_tensor, time)
+        self._check_weights()
         mode = self.compute_mode
-        P = self._pack(mode)
+        P = self.packed(mode)
         te = ops.gather_rows(P["pe"], time.long().contiguous())                      # pe_matrix[timestep]
         te = ops.skinny_linear(te, P["pl1"][0], P["pl1"][1], act_out=2)             # Linear -> GELU
         te = ops.skinny_linear(te, P["pl3"][0], P["pl3"][1])

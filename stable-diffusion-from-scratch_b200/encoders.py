@@ -96,11 +96,7 @@ class TransformerWrapper(engine.PackedWeights, nn.Module):
         self.compute_mode = compute_mode or engine.default_mode()
         self._init_packing()
 
-    def _pack(self, mode):
-        if mode in self._packed:
-            return self._packed[mode]
-        if mode not in engine.MODES:
-            raise ValueError("compute_mode must be one of %s" % (engine.MODES,))
+    def _build_pack(self, mode):
         P = {"tok": self.token_emb.weight.detach().float().contiguous(),
              "pos": self.pos_emb.emb.weight.detach().float().contiguous()}
         layers = self.attn_layers.layers
@@ -110,11 +106,10 @@ class TransformerWrapper(engine.PackedWeights, nn.Module):
             P[("out", i)] = PackedLinear(a.to_out.weight, a.to_out.bias, mode)
             P[("ff1", i)] = PackedLinear(f.net[0][0].weight, f.net[0][0].bias, mode)
             P[("ff2", i)] = PackedLinear(f.net[2].weight, f.net[2].bias, mode)
-        self._packed[mode] = P
         return P
 
     def _forward_tokens(self, ids, mode):
-        P = self._pack(mode)
+        P = self.packed(mode)
         B, S = ids.shape
         D = self.attn_layers.dim
         inner, W3 = HEADS * DIM_HEAD, 3 * HEADS * DIM_HEAD
@@ -132,7 +127,7 @@ class TransformerWrapper(engine.PackedWeights, nn.Module):
                                      engine.head_pad(DIM_HEAD), a.scale, st, st, st, dense=True, causal=False)
                 o = o.reshape(B * S, inner)
             else:
-                o = engine.attention_fp32(qkv, qkv[:, inner:], qkv[:, 2 * inner:], B, HEADS, S, S, DIM_HEAD, a.scale, ld=W3)
+                o = engine.attention_fp32(qkv, qkv[:, inner:], qkv[:, 2 * inner:], B, HEADS, S, S, DIM_HEAD, a.scale)
             x = engine.linear(o, P[("out", i)], residual=x, rows_per_item=S)
             h = ops.layernorm(x, nf.weight, nf.bias, nf.eps, out_dtype=odt)
             h = engine.linear(h, P[("ff1", i)], rows_per_item=S)                                 # fp32 [B*S, 4D]

@@ -7,6 +7,7 @@ Two compute modes (the constructor/env switch SURVEY.md §8b asks for, not a sig
 There is no other path: both modes run hand-written kernels from libsdb200.so.
 """
 import os
+import weakref
 
 import torch
 
@@ -52,9 +53,10 @@ class PackedConv:
 
 class PackedWeights:
     """Mixin for an nn.Module that keeps per-mode packed copies of its parameters in `self._packed`: the copies are dropped
-    when a state dict is loaded, when the module is moved or cast (`_apply`), and when a parameter is changed in place
-    (`_check_weights`, a fingerprint of the first parameter's storage and every parameter's `_version`).  Call
-    `_init_packing()` in `__init__` and `_check_weights()` before every use of the packed copies."""
+    when a state dict is loaded (also through a parent module), when the module is moved or cast (`_apply`), and when a
+    parameter is changed in place (`_check_weights`, a fingerprint of the first parameter's storage and every parameter's
+    `_version`).  Call `_init_packing()` in `__init__`, `_check_weights()` once per public call and `packed(mode)` for the
+    copies; a subclass implements `_build_pack(mode)`."""
 
     def _init_packing(self):
         self._packed = {}
@@ -79,6 +81,43 @@ class PackedWeights:
             if self.__dict__.get("_fp_seen") is not None:
                 self._invalidate()
             self.__dict__["_fp_seen"] = fp
+
+    def packed(self, mode):
+        P = self._packed.get(mode)
+        if P is None:
+            if mode not in MODES:
+                raise ValueError("compute_mode must be one of %s" % (MODES,))
+            P = self._packed[mode] = self._build_pack(mode)
+        return P
+
+
+class TensorMemo:
+    """Values derived from tensors the owner does not own (a projection of the caller's conditioning, a table built from
+    schedule buffers).  An entry stays valid only while each source tensor is the same live object (weakref), unwritten
+    since (`_version`) and in the same place (`data_ptr`: `Module.to()` moves a Parameter without changing either of the
+    others).  At `capacity` entries, a new one first drops entries whose sources died, then clears the memo."""
+
+    def __init__(self, capacity):
+        self.capacity = capacity
+        self._entries = {}           # key -> (((weakref, _version, data_ptr) per source tensor), value)
+
+    def get(self, tensors, key, build):
+        """The value stored under `key` for these live `tensors`, else `build()`, stored."""
+        hit = self._entries.get(key)
+        if hit is not None and len(hit[0]) == len(tensors) and all(
+                r() is t and v == t._version and p == t.data_ptr() for (r, v, p), t in zip(hit[0], tensors)):
+            return hit[1]
+        stamp = tuple((weakref.ref(t), t._version, t.data_ptr()) for t in tensors)
+        value = build()
+        if key not in self._entries and len(self._entries) >= self.capacity:
+            self._entries = {k: e for k, e in self._entries.items() if all(r() is not None for r, _, _ in e[0])}
+            if len(self._entries) >= self.capacity:
+                self._entries.clear()
+        self._entries[key] = (stamp, value)
+        return value
+
+    def clear(self):
+        self._entries.clear()
 
 
 class PackedLinear:
@@ -135,17 +174,19 @@ def linear(x, pl, residual=None, out_dtype=torch.float32, col_group=0, col_group
     return ops.gemm_simt(x2, pl.w, pl.bias, residual=residual, out_dtype=out_dtype)
 
 
-def attention_fp32(q, k, v, B, H, Sq, Sk, d, scale, ld=None):
-    """fp32 unfused attention: scores = q k^T (batched over (b, h)), row softmax, out = P v.
-    q [B*Sq, H*d], k/v [B*Sk, H*d] fp32 -> [B*Sq, H*d] fp32.  ld: the row stride of q, k and v in elements when they are
-    column blocks of one wider tensor (e.g. the q | k | v projection), else H*d."""
+def attention_fp32(q, k, v, B, H, Sq, Sk, d, scale, o_strides=None, causal=False):
+    """fp32 unfused attention: scores = q k^T (batched over (b, h)), row softmax (causal: query i sees keys 0 .. i),
+    out = P v.  q [B*Sq, >= H*d], k / v [B*Sk, >= H*d] fp32 row views (e.g. column blocks of the q | k | v projection,
+    each read at its own row stride) -> [B*Sq, H*d] fp32.  o_strides = (batch, seq, head) element strides of another
+    output layout."""
     Cc = H * d
-    ld = Cc if ld is None else ld
+    ldq, ldk, ldv = q.stride(0), k.stride(0), v.stride(0)
     scores = torch.empty((B, H, Sq, Sk), dtype=torch.float32, device=q.device)
-    ops.gemm_simt(q, k, out=scores, M=Sq, N=Sk, K=d, lda=ld, ldb=ld, ldc=Sk, batch=(B, H),
-                  sa=(Sq * ld, d), sb=(Sk * ld, d), sc=(H * Sq * Sk, Sq * Sk))
-    P = ops.softmax_rows(scores, scale)
+    ops.gemm_simt(q, k, out=scores, M=Sq, N=Sk, K=d, lda=ldq, ldb=ldk, ldc=Sk, batch=(B, H),
+                  sa=(Sq * ldq, d), sb=(Sk * ldk, d), sc=(H * Sq * Sk, Sq * Sk))
+    P = ops.softmax_rows_causal(scores, scale, Sq) if causal else ops.softmax_rows(scores, scale)
     out = torch.empty((B * Sq, Cc), dtype=torch.float32, device=q.device)
-    ops.gemm_simt(P, v, out=out, b_kn=True, M=Sq, N=d, K=Sk, lda=Sk, ldb=ld, ldc=Cc, batch=(B, H),
-                  sa=(H * Sq * Sk, Sq * Sk), sb=(Sk * ld, d), sc=(Sq * Cc, d))
+    o_bs, o_ss, o_hs = o_strides if o_strides is not None else (Sq * Cc, Cc, d)
+    ops.gemm_simt(P, v, out=out, b_kn=True, M=Sq, N=d, K=Sk, lda=Sk, ldb=ldv, ldc=o_ss, batch=(B, H),
+                  sa=(H * Sq * Sk, Sq * Sk), sb=(Sk * ldv, d), sc=(o_bs, o_hs))
     return out

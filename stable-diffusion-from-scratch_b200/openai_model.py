@@ -14,7 +14,6 @@ silently computing something else.
 """
 import math
 import os
-import weakref
 
 import torch
 from torch import nn
@@ -216,7 +215,7 @@ class _SideResult:
         return self.tensor
 
 
-class UNetModel(nn.Module):
+class UNetModel(engine.PackedWeights, nn.Module):
     """The full UNet with attention and timestep embedding (openai_model/model.py:259-595).
 
     Extra keyword (not in the reference): `compute_mode` = "bf16" (tcgen05 tensor cores, default) or
@@ -324,22 +323,18 @@ class UNetModel(nn.Module):
                 self.output_blocks.append(TimestepEmbedSequential(*layers))
         self.out = nn.Sequential(normalization(ch), nn.SiLU(), zero_module(nn.Conv2d(model_channels, out_channels, 3, padding=1)))
 
-        self._packed = {}        # mode -> packed weights
-        self._ctx_cache = {}     # (mode, block, id(context)) -> (weakref(context), version, projected K/V)
-        # a parent's load_state_dict (e.g. LatentDiffusion's) never calls the override below: drop the packed copies from a hook
-        self.register_load_state_dict_post_hook(lambda module, incompatible_keys: module._invalidate())
+        self._init_packing()
+        self._ctx_cache = engine.TensorMemo(256)     # projected K/V (and the bf16 copy) of the caller's context tensors
         self._kv_pinned = None   # graph mode: {id(block): projected K/V of the static context buffer}
         self._graphs = {}
         self._padbufs = {}       # (rows, width, d, dp) -> zero-initialised padded-head projection buffer
 
     # ---- weight packing ---------------------------------------------------------------------------
     def _invalidate(self):
-        self._packed = {}
-        self._ctx_cache = {}
+        self._ctx_cache.clear()
         self._graphs = {}
         self._padbufs = {}
-        self.__dict__.pop("_param_list", None)
-        self.__dict__.pop("_fp_seen", None)
+        super()._invalidate()
 
     def _padbuf(self, rows, width, d, dp, dev):
         """Persistent [rows, width] bf16 buffer for q/k/v heads stored padded from d to dp channels.  The GEMM
@@ -352,41 +347,12 @@ class UNetModel(nn.Module):
             self._padbufs[key] = buf
         return buf
 
-    def load_state_dict(self, *a, **k):
-        r = super().load_state_dict(*a, **k)
-        self._invalidate()
-        return r
-
-    def _apply(self, fn, *a, **k):
-        r = super()._apply(fn, *a, **k)
-        self._invalidate()
-        return r
-
-    def _weights_fingerprint(self):
-        """Changes whenever a parameter is replaced or written in place (EMA `copy_to`, optimizer step, a parent module's
-        load_state_dict — which recurses through `_load_from_state_dict` and never reaches the override above)."""
-        ps = self.__dict__.get("_param_list")
-        if ps is None:
-            ps = self.__dict__["_param_list"] = list(self.parameters())
-        return (ps[0].data_ptr(), ps[0].device, sum(p._version for p in ps))
-
-    def _check_weights(self):
-        fp = self._weights_fingerprint()
-        if fp != self.__dict__.get("_fp_seen"):
-            if self.__dict__.get("_fp_seen") is not None:
-                self._invalidate()
-            self.__dict__["_fp_seen"] = fp
-
     def _res_blocks(self):
         for m in self.modules():
             if isinstance(m, ResBlock):
                 yield m
 
-    def _pack(self, mode):
-        if mode in self._packed:
-            return self._packed[mode]
-        if mode not in engine.MODES:
-            raise ValueError("compute_mode must be one of %s" % (engine.MODES,))
+    def _build_pack(self, mode):
         P = {}
         dev = self.time_embed[0].weight.device
         half = self.model_channels // 2
@@ -448,7 +414,6 @@ class UNetModel(nn.Module):
             P["conv_in_split"] = True
         P["conv_in"] = PackedConv(cin_w, self.input_blocks[0][0].bias, mode)
         P["conv_out"] = PackedConv(self.out[2].weight, self.out[2].bias, mode)
-        self._packed[mode] = P
         return P
 
     # ---- building blocks (all tensors NHWC / [rows, C]) ---------------------------------------------
@@ -539,53 +504,32 @@ class UNetModel(nn.Module):
                                  (T * W3, W3, d), (T * W3, W3, d), (T * W3, W3, d), o_strides=o_strides, dense=True)
         else:
             qkv = engine.linear(xn, P[("qkv", id(ab))], rows_per_item=T)                                       # [B*T, 3C]
-            o = self._attn_fp32(qkv, 3 * Cc, 0, qkv, 3 * Cc, Cc, qkv, 3 * Cc, 2 * Cc, B, H, T, T, d, scale, o_strides=o_strides)
+            o = engine.attention_fp32(qkv, qkv[:, Cc:], qkv[:, 2 * Cc:], B, H, T, T, d, scale, o_strides=o_strides)
         out = engine.linear(o.reshape(B * T, Cc), P[("aout", id(ab))], residual=x.reshape(B * T, Cc), rows_per_item=T)
         return out.reshape(B, Hh, Ww, Cc)
 
-    def _ctx_lookup(self, key, src):
-        """Cache entries are valid only for the SAME live tensor object, unmodified since: a data_ptr()/shape key alone
-        collides when the allocator hands a freed conditioning's address to the next prompt's."""
-        hit = self._ctx_cache.get(key)
-        if hit is not None and hit[0]() is src and hit[1] == src._version:
-            return hit[2]
-        return None
-
-    def _ctx_store(self, key, src, val):
-        if len(self._ctx_cache) > 256:
-            self._ctx_cache = {k: v for k, v in self._ctx_cache.items() if v[0]() is not None}
-            if len(self._ctx_cache) > 256:
-                self._ctx_cache.clear()
-        self._ctx_cache[key] = (weakref.ref(src), src._version, val)
-
     def _kv_context(self, blk, P, mode, context, src=None):
         """to_k / to_v of the (step-invariant) context, cached per LIVE context tensor (`src` = the caller's own tensor
-        object when `context` is a converted temporary of it)."""
+        object when `context` is a converted temporary of it): an address / shape key alone collides when the allocator
+        hands a freed conditioning's memory to the next prompt's."""
         pinned = self._kv_pinned
         if pinned is not None:                       # CUDA-graph mode: projections live in their own graph (see _graph_forward)
             return pinned[id(blk)]
         src = context if src is None else src
-        key = (mode, id(blk), id(src))
-        hit = self._ctx_lookup(key, src)
-        if hit is not None:
-            return hit
+        return self._ctx_cache.get((src,), (mode, id(blk), id(src)), lambda: self._project_kv(blk, P, mode, context, src))
+
+    def _project_kv(self, blk, P, mode, context, src):
         a2 = blk.attn2
         H, d = a2.heads, a2.dim_head
         B, Sk, Cc = context.shape
         if mode == "bf16":
-            cb = self._ctx_lookup(("ctx_bf16", id(src)), src)
-            if cb is None:
-                cb = ops.cast_concat(context.reshape(1, 1, B * Sk, Cc).contiguous(), None, out_dtype=torch.bfloat16).reshape(B * Sk, Cc)
-                self._ctx_store(("ctx_bf16", id(src)), src, cb)
+            cb = self._ctx_cache.get((src,), ("ctx_bf16", id(src)), lambda: ops.cast_concat(
+                context.reshape(1, 1, B * Sk, Cc).contiguous(), None, out_dtype=torch.bfloat16).reshape(B * Sk, Cc))
             if self.dense_heads:
-                kv = engine.linear(cb, P[("kv2", id(blk))], out_dtype=torch.bfloat16, rows_per_item=Sk)                                   # [B*Sk, 2*H*d]
-            else:
-                dp = head_pad(d)
-                kv = engine.linear(cb, P[("kv2", id(blk))], out_dtype=torch.bfloat16, col_group=d, col_group_stride=dp, rows_per_item=Sk)   # [B*Sk, 2*H*dp]
-        else:
-            kv = engine.linear(context.reshape(B * Sk, Cc), P[("kv2", id(blk))], rows_per_item=Sk)                                      # [B*Sk, 2*H*d]
-        self._ctx_store(key, src, kv)
-        return kv
+                return engine.linear(cb, P[("kv2", id(blk))], out_dtype=torch.bfloat16, rows_per_item=Sk)                                 # [B*Sk, 2*H*d]
+            dp = head_pad(d)
+            return engine.linear(cb, P[("kv2", id(blk))], out_dtype=torch.bfloat16, col_group=d, col_group_stride=dp, rows_per_item=Sk)   # [B*Sk, 2*H*dp]
+        return engine.linear(context.reshape(B * Sk, Cc), P[("kv2", id(blk))], rows_per_item=Sk)                                      # [B*Sk, 2*H*d]
 
     def _tblock(self, blk, P, mode, t, B, S, context, final_dtype=torch.float32):
         """BasicTransformerBlock._forward (openai_model/attention.py:233-257) on tokens t [B*S, C] fp32."""
@@ -631,36 +575,17 @@ class UNetModel(nn.Module):
         else:
             a = ops.layernorm(t, blk.norm1.weight, blk.norm1.bias, blk.norm1.eps, out_dtype=odt)
             qkv = engine.linear(a, P[("qkv1", id(blk))], rows_per_item=S)                                                     # [B*S, 3C]
-            o = self._attn_fp32(qkv, 3 * Cc, 0, qkv, 3 * Cc, Cc, qkv, 3 * Cc, 2 * Cc, B, H, S, S, d, a1.scale)
+            o = engine.attention_fp32(qkv, qkv[:, Cc:], qkv[:, 2 * Cc:], B, H, S, S, d, a1.scale)
             t = engine.linear(o, P[("o1", id(blk))], residual=t, rows_per_item=S)
             a = ops.layernorm(t, blk.norm2.weight, blk.norm2.bias, blk.norm2.eps, out_dtype=odt)
             q = engine.linear(a, P[("q2", id(blk))], rows_per_item=S)
-            o = self._attn_fp32(q, Cc, 0, kv, 2 * Cc, 0, kv, 2 * Cc, Cc, B, H, S, Sk, d, a2.scale)
+            o = engine.attention_fp32(q, kv, kv[:, Cc:], B, H, S, Sk, d, a2.scale)
             t = engine.linear(o, P[("o2", id(blk))], residual=t, rows_per_item=S)
         a = ops.layernorm(t, blk.norm3.weight, blk.norm3.bias, blk.norm3.eps, out_dtype=odt)
         g = engine.linear(a, P[("ff1", id(blk))], out_dtype=odt, rows_per_item=S)          # GEGLU fused (bf16) or gemm + geglu kernel (fp32)
         # `final_dtype` bf16: the block's result only feeds proj_out's tensor-core operand, so it is rounded here
         t = engine.linear(g, P[("ff2", id(blk))], residual=t, rows_per_item=S, out_dtype=final_dtype)
         return t
-
-    @staticmethod
-    def _attn_fp32(q, ldq, qoff, k, ldk, koff, v, ldv, voff, B, H, Sq, Sk, d, scale, o_strides=None):
-        """softmax(q k^T * scale) v per (batch, head) with strided fp32 SIMT GEMMs; returns [B*Sq, H*d]
-        (o_strides = (batch, seq, head) element strides of another output layout)."""
-        Cc = H * d
-        dev = q.device
-        scores = torch.empty((B, H, Sq, Sk), dtype=torch.float32, device=dev)
-        qv = q.reshape(-1)[qoff:]
-        kv_ = k.reshape(-1)[koff:]
-        vv = v.reshape(-1)[voff:]
-        ops.gemm_simt(qv, kv_, out=scores, M=Sq, N=Sk, K=d, lda=ldq, ldb=ldk, ldc=Sk, batch=(B, H),
-                      sa=(Sq * ldq, d), sb=(Sk * ldk, d), sc=(H * Sq * Sk, Sq * Sk))
-        Pm = ops.softmax_rows(scores, scale)
-        out = torch.empty((B * Sq, Cc), dtype=torch.float32, device=dev)
-        o_bs, o_ss, o_hs = o_strides if o_strides is not None else (Sq * Cc, Cc, d)
-        ops.gemm_simt(Pm, vv, out=out, b_kn=True, M=Sq, N=d, K=Sk, lda=Sk, ldb=ldv, ldc=o_ss, batch=(B, H),
-                      sa=(H * Sq * Sk, Sq * Sk), sb=(Sk * ldv, d), sc=(o_bs, o_hs))
-        return out
 
     def _st(self, st, P, mode, x, context):
         """SpatialTransformer.forward (openai_model/attention.py:336-363); NHWC makes both rearranges free."""
@@ -716,7 +641,7 @@ class UNetModel(nn.Module):
 
     def _forward_nhwc(self, x_nchw, t_f32, context, mode, y=None, x1_nchw=None):
         """x1_nchw: channels appended to x's for conv_in (forward_concat); the concat happens inside the layout kernel."""
-        P = self._pack(mode)
+        P = self.packed(mode)
         if self.emb_side_stream:
             # The time-embedding chain (4 launches that stream the 20160 x 1280 emb_layers matrix, ~0.1 ms) depends on t only and
             # is first needed by the first ResBlock's conv epilogue: it runs on a side stream beside the layout change, conv_in
@@ -823,7 +748,7 @@ class UNetModel(nn.Module):
         if g is None:
             sx, st_, sc = x.clone(), t.clone(), ctx.clone()
             sx1 = x1.clone() if x1 is not None else None
-            P = self._pack(mode)
+            P = self.packed(mode)
             s = torch.cuda.Stream()
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
@@ -841,19 +766,15 @@ class UNetModel(nn.Module):
             finally:
                 self._kv_pinned = None
                 self._ctx_cache.clear()
-            g = [graph, kv_graph, sx, st_, sc, out, None, pinned, sx1]      # `pinned` keeps the projections' memory alive
+            # g[6]: the conditioning the projections were last replayed for (`pinned` keeps their memory alive)
+            g = [graph, kv_graph, sx, st_, sc, out, engine.TensorMemo(1), pinned, sx1]
             self._graphs[key] = g
         graph, kv_graph, sx, st_, sc, out, seen = g[:7]
         sx.copy_(x)
         if x1 is not None:
             g[8].copy_(x1)
         st_.copy_(t)
-        # same live tensor object, not modified in place since the last call => same conditioning
-        src = ctx_src if ctx_src is not None else ctx
-        same = seen is not None and seen[0]() is src and seen[1] == src._version
-        if not same:                          # new conditioning: copy it in and re-project K / V
-            sc.copy_(ctx)
-            kv_graph.replay()
-            g[6] = (weakref.ref(src), src._version)
+        # a new conditioning (another tensor object, or this one written or moved since): copy it in and re-project K / V
+        seen.get((ctx_src if ctx_src is not None else ctx,), None, lambda: (sc.copy_(ctx), kv_graph.replay()))
         graph.replay()
         return out.clone()

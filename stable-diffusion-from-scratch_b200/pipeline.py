@@ -9,13 +9,11 @@ schedule buffers, `apply_model(x, t, cond)`, `decode_first_stage(z)`.  It owns a
 It also carries the reference's ancestral sampler (`sample` / `p_sample_loop` / `progressive_denoising`,
 ddpm.py:1528-1793), whose per-step update runs as one fused kernel (sdb_ddpm_step).
 """
-import weakref
-
 import numpy as np
 import torch
 from torch import nn
 
-from . import ops
+from . import engine, ops
 from .autoencoder import AutoencoderKL, DiagonalGaussianDistribution, VQModelInterface
 from .ddim import DDIMSampler
 from .openai_model import UNetModel
@@ -139,6 +137,8 @@ class LatentDiffusion(nn.Module):
         self.register_buffer("posterior_log_variance_clipped", to_t(np.log(np.maximum(posterior_variance, 1e-20))))
         self.register_buffer("posterior_mean_coef1", to_t(betas * np.sqrt(alphas_cumprod_prev) / (1. - alphas_cumprod)))
         self.register_buffer("posterior_mean_coef2", to_t((1. - alphas_cumprod_prev) * np.sqrt(alphas) / (1. - alphas_cumprod)))
+        self._split_cond_cache = engine.TensorMemo(8)     # _repeat_cond
+        self._ddpm_tables = engine.TensorMemo(1)          # _ddpm_cache
 
     @property
     def device(self):
@@ -238,21 +238,11 @@ class LatentDiffusion(nn.Module):
         return ops.patch_fold(o.float().contiguous(), B, grid, fstride, out_hw, wpix, wcrop)
 
     def _repeat_cond(self, v, n):
-        """v repeated n times along the batch (the same conditioning for n crops), cached per (caller's tensor, data_ptr,
-        _version, n): a UNet that caches its context K/V projections per context tensor keeps hitting across steps."""
+        """v repeated n times along the batch (the same conditioning for n crops), cached per (live caller's tensor, n): a
+        UNet that caches its context K/V projections per context tensor keeps hitting across steps."""
         if not torch.is_tensor(v) or n == 1:
             return v
-        cache = self.__dict__.setdefault("_split_cond_cache", {})
-        key = (id(v), v.data_ptr(), v._version, n)
-        hit = cache.get(key)
-        if hit is None or hit[0]() is not v:
-            for k in [k for k, (r, _) in cache.items() if r() is None]:
-                del cache[k]
-            if len(cache) >= 8:
-                cache.clear()
-            hit = (weakref.ref(v), v.repeat(n, *((1,) * (v.dim() - 1))))
-            cache[key] = hit
-        return hit[1]
+        return self._split_cond_cache.get((v,), (id(v), n), lambda: v.repeat(n, *((1,) * (v.dim() - 1))))
 
     def _apply_model_split(self, x_noisy, t, cond):
         sp = self.split_input_params
@@ -432,21 +422,18 @@ class LatentDiffusion(nn.Module):
     def _ddpm_cache(self):
         """(posterior_std [T] on the host, [5, T] device table of sdb_ddpm_step) for the current schedule buffers.  Built once
         per schedule and rebuilt when any buffer it derives from is replaced (.to(), reassignment) or written in place
-        (load_state_dict): the key holds each buffer's identity, data_ptr and _version."""
+        (load_state_dict)."""
         src = (self.betas, self.sqrt_recip_alphas_cumprod, self.sqrt_recipm1_alphas_cumprod, self.posterior_mean_coef1,
                self.posterior_mean_coef2, self.posterior_log_variance_clipped)
-        key = tuple((b.data_ptr(), b._version) for b in src)
-        hit = self.__dict__.get("_ddpm_tables")
-        if hit is None or hit[0] != key or any(r() is not b for r, b in zip(hit[1], src)):
+
+        def build():
             # (0.5 * model_log_variance).exp() of p_sample, evaluated per element on a [1,1,1,1] fp32 host tensor: torch's CPU
             # exp is not correctly rounded, and the reference applies it to a [b,1,1,1] tensor, i.e. element by element
             lv = self.posterior_log_variance_clipped.detach().float().cpu()
             std = torch.tensor([float((0.5 * torch.full((1, 1, 1, 1), float(v))).exp()) for v in lv], dtype=torch.float32)
             dev = self.betas.device
-            table = torch.stack([b.detach().float().to(dev) for b in src[1:5]] + [std.to(dev)]).contiguous()
-            hit = (key, tuple(weakref.ref(b) for b in src), std, table)
-            self.__dict__["_ddpm_tables"] = hit
-        return hit[2], hit[3]
+            return std, torch.stack([b.detach().float().to(dev) for b in src[1:5]] + [std.to(dev)]).contiguous()
+        return self._ddpm_tables.get(src, None, build)
 
     def posterior_std(self):
         """fp32 [T] host table exp(0.5 * posterior_log_variance_clipped[t]): the std p_sample adds noise with."""

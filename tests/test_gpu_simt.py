@@ -43,21 +43,27 @@ def test_gemm_simt(cuda, M, N, K):
 
 
 @pytest.mark.parametrize("B,H,Sq,Sk,d", [(2, 8, 64, 64, 40), (1, 2, 100, 77, 32), (2, 4, 16, 16, 64)])
-def test_attention_fp32_path(cuda, B, H, Sq, Sk, d):
-    from sdb200.openai_model import UNetModel
+def test_attention_fp32_row_views(cuda, B, H, Sq, Sk, d):
+    from sdb200.engine import attention_fp32
     C = H * d
     q, k, v = randn(B * Sq, C, seed=1), randn(B * Sk, C, seed=2), randn(B * Sk, C, seed=3)
     scale = d ** -0.5
-    o = UNetModel._attn_fp32(q, C, 0, k, C, 0, v, C, 0, B, H, Sq, Sk, d, scale)
+    o = attention_fp32(q, k, v, B, H, Sq, Sk, d, scale)
     qh = q.double().view(B, Sq, H, d).transpose(1, 2)
     kh = k.double().view(B, Sk, H, d).transpose(1, 2)
     vh = v.double().view(B, Sk, H, d).transpose(1, 2)
     ref = (torch.softmax(qh @ kh.transpose(-1, -2) * scale, -1) @ vh).transpose(1, 2).reshape(B * Sq, C)
     assert rel(o, ref) < 2e-6
-    # fused-qkv layout with offsets, as the UNet uses it
+    # fused-qkv layout (column views of one [rows, 3C] tensor), as the UNet uses it
     qkv = torch.cat([q, q * 0.5 + 1, q * 2 - 1], 1).contiguous() if Sq == Sk else None
     if qkv is not None:
-        o2 = UNetModel._attn_fp32(qkv, 3 * C, 0, qkv, 3 * C, C, qkv, 3 * C, 2 * C, B, H, Sq, Sq, d, scale)
+        o2 = attention_fp32(qkv, qkv[:, C:], qkv[:, 2 * C:], B, H, Sq, Sq, d, scale)
         k2, v2 = (q * 0.5 + 1).double().view(B, Sq, H, d).transpose(1, 2), (q * 2 - 1).double().view(B, Sq, H, d).transpose(1, 2)
-        ref2 = (torch.softmax(qh @ k2.transpose(-1, -2) * scale, -1) @ v2).transpose(1, 2).reshape(B * Sq, C)
+        s2 = qh @ k2.transpose(-1, -2) * scale
+        ref2 = (torch.softmax(s2, -1) @ v2).transpose(1, 2).reshape(B * Sq, C)
         assert rel(o2, ref2) < 2e-6
+        # causal (CLIP's text tower): query i sees keys 0 .. i
+        o3 = attention_fp32(qkv, qkv[:, C:], qkv[:, 2 * C:], B, H, Sq, Sq, d, scale, causal=True)
+        mask = torch.ones(Sq, Sq, dtype=torch.bool, device=q.device).triu(1)
+        ref3 = (torch.softmax(s2.masked_fill(mask, float("-inf")), -1) @ v2).transpose(1, 2).reshape(B * Sq, C)
+        assert rel(o3, ref3) < 2e-6

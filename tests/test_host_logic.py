@@ -2,6 +2,7 @@
 import numpy as np
 import pytest
 import torch
+from torch import nn
 
 from oracle import restate as R
 from oracle import weights as W
@@ -226,58 +227,74 @@ def _tiny_unet():
                      num_heads=2, use_spatial_transformer=True, context_dim=8, channel_mult=(1,))
 
 
-def test_context_cache_is_keyed_on_the_live_tensor():
-    """The cross-attention K/V cache must not confuse a new conditioning tensor with a freed one that had the same address,
-    shape and version (ADVICE r1: data_ptr()-keyed entries collided after the allocator recycled the block)."""
-    net = _tiny_unet()
+def test_tensor_memo_is_keyed_on_the_live_tensor():
+    """The cross-attention K/V cache (an engine.TensorMemo) must not confuse a new conditioning tensor with a freed one that
+    had the same address, shape and version (ADVICE r1: data_ptr()-keyed entries collided after the allocator recycled the
+    block), nor keep a projection of a tensor written in place or moved."""
+    memo = _tiny_unet()._ctx_cache
+    built = []
+
+    def get(t, key):
+        return memo.get((t,), key, lambda: built.append(key) or "kv-%d" % len(built))
+
     a = torch.zeros(2, 7, 8)
     key = ("bf16", 1234, id(a))
-    net._ctx_store(key, a, "kv-of-a")
-    assert net._ctx_lookup(key, a) == "kv-of-a"
+    assert get(a, key) == "kv-1" and get(a, key) == "kv-1"     # built once, then a hit
     b = torch.zeros(2, 7, 8)
-    assert net._ctx_lookup(key, b) is None                    # same shape / version, different object
+    assert get(b, key) == "kv-2"                               # same shape / version, different object
     a.add_(1)
-    assert net._ctx_lookup(key, a) is None                    # modified in place since it was projected
-    net._ctx_store(key, a, "kv-of-a2")
+    assert get(a, key) == "kv-3"                               # modified in place since it was projected
     del a
     import gc
     gc.collect()
     c = torch.zeros(2, 7, 8)
-    assert net._ctx_lookup(("bf16", 1234, id(c)), c) is None  # even if id() / the address is recycled, the weakref is dead
-    for i in range(400):                                      # bounded: dead entries are dropped
-        t = torch.zeros(1)
-        net._ctx_store(("k", i), t, i)
-    assert len(net._ctx_cache) <= 257
+    assert get(c, key) == "kv-4"                               # even if id() / the address is recycled, the weakref is dead
+    lin = nn.Linear(8, 8)
+    w = lin.weight
+    assert get(w, "w") == "kv-5"
+    v0, p0 = w._version, w.data_ptr()
+    lin.to(torch.float64)                                      # same Parameter object, same _version, new storage
+    assert lin.weight is w and w._version == v0 and w.data_ptr() != p0
+    assert get(w, "w") == "kv-6"
+    for i in range(400):                                       # bounded: dead entries are dropped, then the memo is cleared
+        get(torch.zeros(1), ("k", i))
+        assert len(memo._entries) <= 256
 
 
-def test_packed_weights_are_invalidated_through_a_parent_module():
+def test_weight_packs_are_invalidated_through_a_parent_module():
     """Packed copies / graphs must be dropped when a checkpoint is loaded through a PARENT (nn.Module.load_state_dict recurses
     via _load_from_state_dict and never calls the child's override), when .to() is applied to the parent, and when a
     parameter is written in place (EMA copy_to)."""
     from sdb200.autoencoder import AutoencoderKL
+    from sdb200.ddpm_unet import UNet
+    from sdb200.engine import PackedConv
     from sdb200.pipeline import LatentDiffusion
     vae_cfg = dict(double_z=True, z_channels=4, resolution=16, in_channels=3, out_ch=3, ch=32, ch_mult=(1,), num_res_blocks=1,
                    attn_resolutions=[], dropout=0.0)
     ld = LatentDiffusion(unet=_tiny_unet(), first_stage_model=AutoencoderKL(ddconfig=vae_cfg, embed_dim=4))
     unet, vae = ld.model.diffusion_model, ld.first_stage_model
+    ddpm = UNet(image_size=32)
+    ddpm_parent = nn.Sequential(ddpm)
 
     def poison():
         unet._packed = {"bf16": "stale"}
         unet._graphs = {"k": "stale"}
         vae.decoder._packed = {"bf16": "stale"}
         vae.encoder._packed = {"bf16": "stale"}
-        vae._pq = ("stale", None)
-        vae._q = ("stale", None)
+        ddpm._packed = {"bf16": "stale"}
 
     def clean():
-        return unet._packed == {} and unet._graphs == {} and vae.decoder._packed == {} and vae.encoder._packed == {}
+        return (unet._packed == {} and unet._graphs == {} and vae.decoder._packed == {} and vae.encoder._packed == {}
+                and ddpm._packed == {})
 
     poison()
     ld.load_state_dict(ld.state_dict())
+    ddpm_parent.load_state_dict(ddpm_parent.state_dict())
     assert clean()
     poison()
     ld.to(torch.float32)                                       # _apply on the parent
-    assert clean() and vae._pq is None and vae._q is None
+    ddpm_parent.to(torch.float32)
+    assert clean()
     # in-place parameter update: the fingerprint changes, the next forward re-packs
     unet._check_weights()
     unet._packed = {"bf16": "stale"}
@@ -293,10 +310,20 @@ def test_packed_weights_are_invalidated_through_a_parent_module():
         vae.decoder.conv_in.weight.add_(1.0)
     vae.decoder._check_weights()
     assert vae.decoder._packed == {}
-    fp0 = (vae.post_quant_conv.weight.data_ptr(), vae.post_quant_conv.weight._version)
+    ddpm._check_weights()
+    ddpm._packed = {"bf16": "stale"}
     with torch.no_grad():
-        vae.post_quant_conv.weight.add_(1.0)
-    assert (vae.post_quant_conv.weight.data_ptr(), vae.post_quant_conv.weight._version) != fp0     # what _packed_1x1 keys on
+        ddpm.initial_conv.weight.mul_(0.5)
+    ddpm._check_weights()
+    assert ddpm._packed == {}
+    # quant_conv / post_quant_conv are packed per call as views of their parameters: an in-place write reaches the next call
+    conv = vae.post_quant_conv
+    with torch.no_grad():
+        conv.weight.add_(1.0)
+    pc = PackedConv(conv.weight, conv.bias, "fp32")
+    assert pc.w.untyped_storage().data_ptr() == conv.weight.untyped_storage().data_ptr()
+    assert pc.bias.untyped_storage().data_ptr() == conv.bias.untyped_storage().data_ptr()
+    assert torch.equal(pc.w.reshape(conv.weight.shape[:2]), conv.weight.detach().reshape(conv.weight.shape[:2]))
 
 
 def test_sampler_defaults_and_coefficient_cache():
