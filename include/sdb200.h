@@ -181,6 +181,26 @@ int sdb_ddim_step(const float* x, const float* e_cond, const float* e_uncond, fl
  * (the caller replaced it by first_stage_model.quantize(pred_x0)), x_prev = sqrt_aprev*pred_x0 + dir_coef*e + sigma_t*noise*temperature. */
 int sdb_ddim_xprev(const float* pred_x0, const float* e_cond, const float* e_uncond, float cfg_scale, const float* noise,
                    float sqrt_aprev, float dir_coef, float sigma_t, float temperature, float* x_prev, long long n, void* stream);
+/* ---- PLMS update ---------------------------------------------------------------------------
+ * Replaces p_sample_plms's arithmetic (ldm/models/diffusion/plms.py: get_model_output's guidance combine, the
+ * multistep combine and get_x_prev_and_pred_x0):
+ *   e       = e_uncond + cfg_scale*(e - e_uncond)                   (if e_uncond != NULL)
+ *   e'      = order 0: (e_old1 + e) / 2       second half of the first step (pseudo improved Euler), e_old1 = first eval
+ *             order 1: e
+ *             order 2: (3*e - e_old1) / 2
+ *             order 3: (23*e - 16*e_old1 + 5*e_old2) / 12
+ *             order 4: (55*e - 59*e_old1 + 37*e_old2 - 9*e_old3) / 24     (e_old1 = old_eps[-1], e_old2 = [-2], e_old3 = [-3])
+ *   pred_x0 = (x - sqrt_one_minus_at*e') / sqrt_at
+ *   x_prev  = sqrt_aprev*pred_x0 + dir_coef*e' + sigma_t*noise*temperature
+ * all fp32, every operation individually rounded (no FMA contraction) in the reference's left-to-right order; the
+ * divisions are divisions.  The five scalars are sdb_ddim_step's.  Outputs, each optional but at least one: e_out = the
+ * combined e (what the sampler's eps history keeps), e_prime_out = e', pred_x0, x_prev.  History pointers the order does
+ * not read are ignored.  noise may be NULL when sigma_t == 0.  No output may overlap an input or another output.
+ * n = number of elements of every operand. */
+int sdb_plms_step(const float* x, const float* e, const float* e_uncond, float cfg_scale, const float* e_old1, const float* e_old2,
+                  const float* e_old3, int order, const float* noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
+                  float sqrt_one_minus_at, float temperature, float* e_out, float* e_prime_out, float* pred_x0, float* x_prev,
+                  long long n, void* stream);
 /* ---- ancestral (DDPM) update ---------------------------------------------------------------
  * Replaces LatentDiffusion.p_sample's arithmetic (ldm/diffusion/ddpm.py:1528-1793: predict_start_from_noise,
  * x_recon.clamp_, q_posterior, `model_mean + nonzero_mask * (0.5 * model_log_variance).exp() * noise`):

@@ -313,11 +313,16 @@ __global__ void skinny_linear_kernel(const float* __restrict__ x, int M, int K, 
 // ---- DDIM update (reference ldm/diffusion/ddim.py:175-205) --------------------------------------
 // Every operation is a separately rounded fp32 op (__f*_rn blocks FMA contraction) so that, given
 // the same eps, x_prev / pred_x0 are bit-identical to the eager reference arithmetic.
+// Classifier-free guidance combine e_u + cfg * (e_c - e_u) (ddim.py:176-179).
+__device__ __forceinline__ float cfg_combine_1(float e, float u, float cfg) {
+    return __fadd_rn(u, __fmul_rn(cfg, __fsub_rn(e, u)));
+}
+
 // One element of the update; `p0_in` != NULL: pred_x0 is given (quantize_denoised branch, ddim.py:198-199) and only x_prev is formed.
 __device__ __forceinline__ void ddim_update_1(float xv, float e, bool has_u, float u, float cfg, bool has_nz, float nzv,
                                               float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
                                               float sqrt_one_minus_at, float temperature, bool p0_given, float& p0, float& xp) {
-    if (has_u) e = __fadd_rn(u, __fmul_rn(cfg, __fsub_rn(e, u)));
+    if (has_u) e = cfg_combine_1(e, u, cfg);
     if (!p0_given) p0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(sqrt_one_minus_at, e)), sqrt_at);
     const float dir = __fmul_rn(dir_coef, e);
     float nz = 0.f;
@@ -357,6 +362,86 @@ ddim_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, con
                           sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, p0_in != nullptr, p0, xp);
             x_prev[i] = xp;
             if (pred_x0) pred_x0[i] = p0;
+        }
+    }
+}
+
+// ---- PLMS update (ldm/models/diffusion/plms.py, p_sample_plms) ------------------------------------------------------------
+//   e  = e_u given ? e_u + cfg * (e - e_u) : e                       (written to e_out: what the eps history keeps)
+//   e' = order 0: (o1 + e) / 2                                        (second half of the first step; o1 = the first eval)
+//        order 1: e
+//        order 2: (3 e - o1) / 2
+//        order 3: (23 e - 16 o1 + 5 o2) / 12
+//        order 4: (55 e - 59 o1 + 37 o2 - 9 o3) / 24                  (o1 = old_eps[-1], o2 = old_eps[-2], o3 = old_eps[-3])
+//   then the DDIM update (ddim_update_1) with e'.
+// Separately rounded fp32 operations, left to right as the eager reference evaluates them; / 2, / 12, / 24 are divisions.
+__device__ __forceinline__ float plms_combine_1(int order, float e, float o1, float o2, float o3) {
+    switch (order) {
+    case 0: return __fdiv_rn(__fadd_rn(o1, e), 2.f);
+    case 2: return __fdiv_rn(__fsub_rn(__fmul_rn(3.f, e), o1), 2.f);
+    case 3: return __fdiv_rn(__fadd_rn(__fsub_rn(__fmul_rn(23.f, e), __fmul_rn(16.f, o1)), __fmul_rn(5.f, o2)), 12.f);
+    case 4: return __fdiv_rn(__fsub_rn(__fadd_rn(__fsub_rn(__fmul_rn(55.f, e), __fmul_rn(59.f, o1)), __fmul_rn(37.f, o2)),
+                                       __fmul_rn(9.f, o3)), 24.f);
+    default: return e;
+    }
+}
+
+struct PlmsOut { float e, ep, p0, xp; };
+
+__device__ __forceinline__ PlmsOut plms_update_1(int order, float xv, float e, bool has_u, float u, float cfg, float o1, float o2,
+                                                 float o3, bool has_nz, float nzv, float sqrt_at, float sqrt_aprev, float dir_coef,
+                                                 float sigma_t, float sqrt_one_minus_at, float temperature) {
+    PlmsOut r;
+    r.e = has_u ? cfg_combine_1(e, u, cfg) : e;
+    r.ep = plms_combine_1(order, r.e, o1, o2, o3);
+    ddim_update_1(xv, r.ep, false, 0.f, 1.f, has_nz, nzv, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature,
+                  false, r.p0, r.xp);
+    return r;
+}
+
+// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, n % 4 == 0), VEC = 1: any alignment.  History pointers the
+// order does not read are NULL (the host clears them), and so are the outputs not requested.
+template <int VEC>
+__global__ void __launch_bounds__(256)
+plms_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, const float* __restrict__ e_u, float cfg,
+                 const float* __restrict__ o1, const float* __restrict__ o2, const float* __restrict__ o3, int order,
+                 const float* __restrict__ noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
+                 float sqrt_one_minus_at, float temperature, float* __restrict__ e_out, float* __restrict__ ep_out,
+                 float* __restrict__ pred_x0, float* __restrict__ x_prev, long long n) {
+    pdl_trigger();
+    pdl_wait();
+    const long long nv = n / VEC;
+    const bool hu = e_u != nullptr, hn = noise != nullptr;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+        if (VEC == 4) {
+            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+            const float4 x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
+            const float4 e4 = __ldg(reinterpret_cast<const float4*>(e_c) + i);
+            const float4 u4 = hu ? __ldg(reinterpret_cast<const float4*>(e_u) + i) : zero;
+            const float4 a4 = o1 ? __ldg(reinterpret_cast<const float4*>(o1) + i) : zero;
+            const float4 b4 = o2 ? __ldg(reinterpret_cast<const float4*>(o2) + i) : zero;
+            const float4 c4 = o3 ? __ldg(reinterpret_cast<const float4*>(o3) + i) : zero;
+            const float4 n4 = hn ? __ldg(reinterpret_cast<const float4*>(noise) + i) : zero;
+            const PlmsOut rx = plms_update_1(order, x4.x, e4.x, hu, u4.x, cfg, a4.x, b4.x, c4.x, hn, n4.x, sqrt_at, sqrt_aprev,
+                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
+            const PlmsOut ry = plms_update_1(order, x4.y, e4.y, hu, u4.y, cfg, a4.y, b4.y, c4.y, hn, n4.y, sqrt_at, sqrt_aprev,
+                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
+            const PlmsOut rz = plms_update_1(order, x4.z, e4.z, hu, u4.z, cfg, a4.z, b4.z, c4.z, hn, n4.z, sqrt_at, sqrt_aprev,
+                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
+            const PlmsOut rw = plms_update_1(order, x4.w, e4.w, hu, u4.w, cfg, a4.w, b4.w, c4.w, hn, n4.w, sqrt_at, sqrt_aprev,
+                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
+            if (e_out) reinterpret_cast<float4*>(e_out)[i] = make_float4(rx.e, ry.e, rz.e, rw.e);
+            if (ep_out) reinterpret_cast<float4*>(ep_out)[i] = make_float4(rx.ep, ry.ep, rz.ep, rw.ep);
+            if (pred_x0) reinterpret_cast<float4*>(pred_x0)[i] = make_float4(rx.p0, ry.p0, rz.p0, rw.p0);
+            if (x_prev) reinterpret_cast<float4*>(x_prev)[i] = make_float4(rx.xp, ry.xp, rz.xp, rw.xp);
+        } else {
+            const PlmsOut r = plms_update_1(order, x[i], e_c[i], hu, hu ? e_u[i] : 0.f, cfg, o1 ? o1[i] : 0.f, o2 ? o2[i] : 0.f,
+                                            o3 ? o3[i] : 0.f, hn, hn ? noise[i] : 0.f, sqrt_at, sqrt_aprev, dir_coef, sigma_t,
+                                            sqrt_one_minus_at, temperature);
+            if (e_out) e_out[i] = r.e;
+            if (ep_out) ep_out[i] = r.ep;
+            if (pred_x0) pred_x0[i] = r.p0;
+            if (x_prev) x_prev[i] = r.xp;
         }
     }
 }
@@ -764,6 +849,49 @@ int sdb_ddim_xprev(const float* pred_x0, const float* e_cond, const float* e_unc
     SDB_REQUIRE(noise || sigma_t == 0.0f, "ddim_xprev: sigma_t != 0 needs a noise tensor");
     return launch_ddim(nullptr, e_cond, e_uncond, cfg_scale, noise, pred_x0, 1.0f, sqrt_aprev, dir_coef, sigma_t, 0.0f,
                        temperature, x_prev, nullptr, n, stream);
+}
+
+// [a, a + n) and [b, b + n) (fp32 elements) share an element; NULL never overlaps.
+static bool ranges_overlap(const float* a, const float* b, long long n) {
+    if (!a || !b) return false;
+    const uintptr_t pa = reinterpret_cast<uintptr_t>(a), pb = reinterpret_cast<uintptr_t>(b), len = (uintptr_t)n * sizeof(float);
+    return pa < pb + len && pb < pa + len;
+}
+
+int sdb_plms_step(const float* x, const float* e, const float* e_uncond, float cfg_scale, const float* e_old1, const float* e_old2,
+                  const float* e_old3, int order, const float* noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
+                  float sqrt_one_minus_at, float temperature, float* e_out, float* e_prime_out, float* pred_x0, float* x_prev,
+                  long long n, void* stream) {
+    SDB_REQUIRE(x && e && n > 0, "plms_step: null input or empty problem (n=%lld)", n);
+    SDB_REQUIRE(order >= 0 && order <= 4, "plms_step: order %d outside 0..4", order);
+    SDB_REQUIRE(e_out || e_prime_out || pred_x0 || x_prev, "plms_step: no output requested");
+    SDB_REQUIRE(order < 2 || e_old1, "plms_step: order %d needs e_old1", order);
+    SDB_REQUIRE(order != 0 || e_old1, "plms_step: order 0 needs the first evaluation in e_old1");
+    SDB_REQUIRE(order < 3 || e_old2, "plms_step: order %d needs e_old2", order);
+    SDB_REQUIRE(order < 4 || e_old3, "plms_step: order 4 needs e_old3");
+    SDB_REQUIRE(noise || sigma_t == 0.0f, "plms_step: sigma_t != 0 needs a noise tensor");
+    const float* o1 = (order == 0 || order >= 2) ? e_old1 : nullptr;
+    const float* o2 = order >= 3 ? e_old2 : nullptr;
+    const float* o3 = order >= 4 ? e_old3 : nullptr;
+    const float* ins[] = {x, e, e_uncond, o1, o2, o3, noise};
+    float* outs[] = {e_out, e_prime_out, pred_x0, x_prev};
+    for (int j = 0; j < 4; ++j) {
+        for (const float* in : ins) SDB_REQUIRE(!ranges_overlap(outs[j], in, n), "plms_step: output %d overlaps an input", j);
+        for (int k = 0; k < j; ++k) SDB_REQUIRE(!ranges_overlap(outs[j], outs[k], n), "plms_step: outputs %d and %d overlap", k, j);
+    }
+    uintptr_t al = 0;
+    for (const float* p : ins) al |= reinterpret_cast<uintptr_t>(p);
+    for (const float* p : outs) al |= reinterpret_cast<uintptr_t>(p);
+    if ((al & 15) == 0 && n % 4 == 0) {
+        launch_pdl(plms_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond, cfg_scale,
+                   o1, o2, o3, order, noise, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, e_out,
+                   e_prime_out, pred_x0, x_prev, n);
+    } else {
+        launch_pdl(plms_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond, cfg_scale,
+                   o1, o2, o3, order, noise, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, e_out,
+                   e_prime_out, pred_x0, x_prev, n);
+    }
+    return check_launch("plms_step_kernel");
 }
 
 int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const float* noise, const long long* t,

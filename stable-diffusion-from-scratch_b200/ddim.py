@@ -44,6 +44,11 @@ def _f32(v):
     return float(torch.full((1,), v).float().item()) if not torch.is_tensor(v) else float(v.float().item())
 
 
+def _f32_contiguous(t):
+    """t as the contiguous fp32 tensor the update kernels read (None passes through)."""
+    return t if (t is None or (t.dtype == torch.float32 and t.is_contiguous())) else t.float().contiguous()
+
+
 class DDIMSampler(object):
     def __init__(self, model, schedule="linear", **kwargs):
         super().__init__()
@@ -98,17 +103,7 @@ class DDIMSampler(object):
                quantize_x0=False, eta=0., mask=None, x0=None, temperature=1., noise_dropout=0., score_corrector=None,
                corrector_kwargs=None, verbose=True, x_T=None, log_every_t=100, unconditional_guidance_scale=1.,
                unconditional_conditioning=None, **kwargs):
-        if conditioning is not None:
-            if isinstance(conditioning, dict):
-                ctmp = conditioning[list(conditioning.keys())[0]]
-                while isinstance(ctmp, list):         # {"c_concat": [..], "c_crossattn": [..]} of a hybrid model
-                    ctmp = ctmp[0]
-                cbs = ctmp.shape[0]
-                if cbs != batch_size:
-                    print(f"Warning: Got {cbs} conditionings but batch-size is {batch_size}")
-            else:
-                if conditioning.shape[0] != batch_size:
-                    print(f"Warning: Got {conditioning.shape[0]} conditionings but batch-size is {batch_size}")
+        self._warn_conditioning_batch(conditioning, batch_size)
         self.make_schedule(ddim_num_steps=S, ddim_eta=eta, verbose=verbose)
         C, H, W = shape
         size = (batch_size, C, H, W)
@@ -121,6 +116,32 @@ class DDIMSampler(object):
                                   unconditional_guidance_scale=unconditional_guidance_scale,
                                   unconditional_conditioning=unconditional_conditioning)
 
+    @staticmethod
+    def _warn_conditioning_batch(conditioning, batch_size):
+        """ddim.py:80-87: a warning, not an error, when the conditioning's batch differs from batch_size."""
+        if conditioning is not None:
+            if isinstance(conditioning, dict):
+                ctmp = conditioning[list(conditioning.keys())[0]]
+                while isinstance(ctmp, list):         # {"c_concat": [..], "c_crossattn": [..]} of a hybrid model
+                    ctmp = ctmp[0]
+                cbs = ctmp.shape[0]
+                if cbs != batch_size:
+                    print(f"Warning: Got {cbs} conditionings but batch-size is {batch_size}")
+            else:
+                if conditioning.shape[0] != batch_size:
+                    print(f"Warning: Got {conditioning.shape[0]} conditionings but batch-size is {batch_size}")
+
+    def _time_range(self, timesteps, ddim_use_original_steps):
+        """ddim.py:120-141: (the step values to visit, in order, as a list or array; their count)."""
+        if timesteps is None:
+            timesteps = self.ddpm_num_timesteps if ddim_use_original_steps else self.ddim_timesteps
+        elif timesteps is not None and not ddim_use_original_steps:
+            subset_end = int(min(timesteps / self.ddim_timesteps.shape[0], 1) * self.ddim_timesteps.shape[0]) - 1
+            timesteps = self.ddim_timesteps[:subset_end]
+        time_range = list(reversed(range(0, timesteps))) if ddim_use_original_steps else np.flip(timesteps)
+        total_steps = timesteps if ddim_use_original_steps else timesteps.shape[0]
+        return time_range, total_steps
+
     @torch.no_grad()
     def ddim_sampling(self, cond, shape, x_T=None, ddim_use_original_steps=False, callback=None, timesteps=None,
                       quantize_denoised=False, mask=None, x0=None, img_callback=None, log_every_t=100, temperature=1.,
@@ -130,14 +151,8 @@ class DDIMSampler(object):
         device = self.model.betas.device
         b = shape[0]
         img = torch.randn(shape, device=device) if x_T is None else x_T
-        if timesteps is None:
-            timesteps = self.ddpm_num_timesteps if ddim_use_original_steps else self.ddim_timesteps
-        elif timesteps is not None and not ddim_use_original_steps:
-            subset_end = int(min(timesteps / self.ddim_timesteps.shape[0], 1) * self.ddim_timesteps.shape[0]) - 1
-            timesteps = self.ddim_timesteps[:subset_end]
+        time_range, total_steps = self._time_range(timesteps, ddim_use_original_steps)
         intermediates = {'x_inter': [img], 'pred_x0': [img]}
-        time_range = reversed(range(0, timesteps)) if ddim_use_original_steps else np.flip(timesteps)
-        total_steps = timesteps if ddim_use_original_steps else timesteps.shape[0]
         # one device tensor of timesteps per step value (tiny H2D, outside the kernels' critical path)
         for i, step in enumerate(time_range):
             index = total_steps - i - 1
@@ -210,6 +225,26 @@ class DDIMSampler(object):
         """ddim.py:167-206.  CFG runs the model on the unconditional and conditional halves separately
         (same per-sample arithmetic as the reference's concatenated 2B batch) and the combine
         e_uc + s*(e_c - e_uc) is fused into the update kernel."""
+        e_t, e_uncond = self._model_eps(x, c, t, score_corrector, corrector_kwargs, unconditional_guidance_scale,
+                                        unconditional_conditioning)
+        sqrt_at, sqrt_aprev, dir_coef, sigma_t, s1m = self.derived_coefficients(index, use_original_steps)
+        noise, k_sigma, k_temp = self._step_noise(x, sigma_t, temperature, noise_dropout, repeat_noise)
+        f = _f32_contiguous
+        xf, ef, uf, nf = f(x), f(e_t), f(e_uncond), f(noise)
+        x_prev, pred_x0 = ops.ddim_step(xf, ef, sqrt_at, sqrt_aprev, dir_coef, k_sigma, s1m, e_uncond=uf,
+                                        cfg_scale=unconditional_guidance_scale, noise=nf, temperature=k_temp)
+        if quantize_denoised:
+            # ddim.py:198-199: pred_x0 is replaced by the first stage's codebook projection before x_prev is formed
+            pred_x0, _, *_ = self.model.first_stage_model.quantize(pred_x0)
+            pred_x0 = f(pred_x0)
+            x_prev = ops.ddim_xprev(pred_x0, ef, sqrt_aprev, dir_coef, k_sigma, e_uncond=uf, cfg_scale=unconditional_guidance_scale,
+                                    noise=nf, temperature=k_temp)
+        return x_prev, pred_x0
+
+    def _model_eps(self, x, c, t, score_corrector, corrector_kwargs, unconditional_guidance_scale, unconditional_conditioning):
+        """The model-evaluation half of p_sample_ddim (ddim.py:174-186; PLMS's get_model_output is the same code):
+        (e_t, e_uncond).  With CFG and no score corrector, e_uncond is the unconditional half and the combine is left to the
+        update kernel; otherwise e_uncond is None and e_t is the final eps."""
         e_uncond = None
         if unconditional_conditioning is None or unconditional_guidance_scale == 1.:
             e_t = self.model.apply_model(x, t, c)
@@ -237,8 +272,12 @@ class DDIMSampler(object):
                 e_t = e_uncond + unconditional_guidance_scale * (e_t - e_uncond)
                 e_uncond = None
             e_t = score_corrector.modify_score(self.model, e_t, x, t, c, **corrector_kwargs)
-        sqrt_at, sqrt_aprev, dir_coef, sigma_t, s1m = self.derived_coefficients(index, use_original_steps)
+        return e_t, e_uncond
 
+    def _step_noise(self, x, sigma_t, temperature, noise_dropout, repeat_noise):
+        """The noise term of one update (ddim.py:200-204): (noise or None, sigma and temperature to pass to the kernel).  The
+        draws follow the reference's: randn on every call unless consume_rng_like_reference is off and sigma_t == 0, and the
+        dropout mask when noise_dropout > 0."""
         noise = None
         if sigma_t != 0.0 or self.consume_rng_like_reference or noise_dropout > 0.:
             if repeat_noise:
@@ -253,17 +292,7 @@ class DDIMSampler(object):
             k_sigma, k_temp = 1.0, 1.0
         elif sigma_t == 0.0:
             noise = None
-        f = lambda t_: t_ if (t_ is None or (t_.dtype == torch.float32 and t_.is_contiguous())) else t_.float().contiguous()
-        xf, ef, uf, nf = f(x), f(e_t), f(e_uncond), f(noise)
-        x_prev, pred_x0 = ops.ddim_step(xf, ef, sqrt_at, sqrt_aprev, dir_coef, k_sigma, s1m, e_uncond=uf,
-                                        cfg_scale=unconditional_guidance_scale, noise=nf, temperature=k_temp)
-        if quantize_denoised:
-            # ddim.py:198-199: pred_x0 is replaced by the first stage's codebook projection before x_prev is formed
-            pred_x0, _, *_ = self.model.first_stage_model.quantize(pred_x0)
-            pred_x0 = f(pred_x0)
-            x_prev = ops.ddim_xprev(pred_x0, ef, sqrt_aprev, dir_coef, k_sigma, e_uncond=uf, cfg_scale=unconditional_guidance_scale,
-                                    noise=nf, temperature=k_temp)
-        return x_prev, pred_x0
+        return noise, k_sigma, k_temp
 
     @staticmethod
     def _cfg_dict_pairable(c, uc):

@@ -307,6 +307,26 @@ def ddim_xprev(pred_x0, e_cond, sqrt_aprev, dir_coef, sigma_t, e_uncond=None, cf
     return x_prev
 
 
+def plms_step(x, e, order, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, e_uncond=None, cfg_scale=1.0, e_old=(),
+              noise=None, temperature=1.0, want_e=False, want_e_prime=False, want_pred_x0=True, want_x_prev=True):
+    """One fused PLMS update (p_sample_plms arithmetic, see include/sdb200.h sdb_plms_step): guidance combine, the order-`order`
+    multistep combine and the DDIM update.  e_old = (old_eps[-1], old_eps[-2], old_eps[-3]) as far as the order reads them;
+    order 0 takes the first evaluation of the step as e_old[0].  Every tensor operand must be contiguous fp32 with x's element
+    count.  Returns (e, e', pred_x0, x_prev), each None unless requested."""
+    e_old = tuple(e_old) + (None,) * (3 - len(e_old))
+    require_cuda(x, e, e_uncond, noise, *e_old)
+    _f32c("x", x)
+    for name, t in (("e", e), ("e_uncond", e_uncond), ("e_old1", e_old[0]), ("e_old2", e_old[1]), ("e_old3", e_old[2]),
+                    ("noise", noise)):
+        _f32c(name, t, x)
+    outs = [torch.empty_like(x) if w else None for w in (want_e, want_e_prime, want_pred_x0, want_x_prev)]
+    check(_L().sdb_plms_step(ptr(x), ptr(e), ptr(e_uncond), float(cfg_scale), ptr(e_old[0]), ptr(e_old[1]), ptr(e_old[2]),
+                             int(order), ptr(noise), float(sqrt_at), float(sqrt_aprev), float(dir_coef), float(sigma_t),
+                             float(sqrt_one_minus_at), float(temperature), *[ptr(o) for o in outs], x.numel(), stream_ptr()),
+          "plms_step")
+    return tuple(outs)
+
+
 def ddpm_step(x, t, table, eps=None, x0=None, noise=None, clip=False, temperature=1.0, want_x_prev=True, want_x0=False):
     """One fused ancestral update (LatentDiffusion.p_sample arithmetic, see include/sdb200.h sdb_ddpm_step).
     x / eps / x0 / noise: contiguous fp32 [B, ...] with x's element count; t: int64 [B] on the device; table: fp32 [5, T]

@@ -17,6 +17,7 @@ from . import engine, ops
 from .autoencoder import AutoencoderKL, DiagonalGaussianDistribution, VQModelInterface
 from .ddim import DDIMSampler
 from .openai_model import UNetModel
+from .plms import PLMSSampler
 
 SD_UNET_CONFIG = dict(  # Diffusion/config.yaml:31-44
     image_size=32, in_channels=4, out_channels=4, model_channels=320, attention_resolutions=[4, 2, 1],
@@ -405,11 +406,15 @@ class LatentDiffusion(nn.Module):
 
     @torch.no_grad()
     def txt2img(self, cond, batch_size, ddim_steps=50, shape=(4, 64, 64), x_T=None, eta=0.0,
-                unconditional_guidance_scale=1.0, unconditional_conditioning=None):
-        """DDIM-`ddim_steps` + VAE decode: latents and [-1,1] images."""
-        z, _ = self.sample_log(cond, batch_size, ddim=True, ddim_steps=ddim_steps, shape=shape, x_T=x_T, eta=eta,
-                               unconditional_guidance_scale=unconditional_guidance_scale,
-                               unconditional_conditioning=unconditional_conditioning)
+                unconditional_guidance_scale=1.0, unconditional_conditioning=None, plms=False):
+        """DDIM-`ddim_steps` (plms=True: PLMS-`ddim_steps`, as scripts/txt2img.py --plms; eta must be 0) + VAE decode:
+        latents and [-1,1] images."""
+        kw = dict(x_T=x_T, eta=eta, unconditional_guidance_scale=unconditional_guidance_scale,
+                  unconditional_conditioning=unconditional_conditioning)
+        if plms:
+            z, _ = PLMSSampler(self).sample(ddim_steps, batch_size, shape, cond, verbose=False, **kw)
+        else:
+            z, _ = self.sample_log(cond, batch_size, ddim=True, ddim_steps=ddim_steps, shape=shape, **kw)
         return z, self.decode_first_stage(z)
 
     # ---- ancestral sampler (ldm/diffusion/ddpm.py:1528-1793) -------------------------------------------------------------
