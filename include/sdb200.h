@@ -201,6 +201,26 @@ int sdb_plms_step(const float* x, const float* e, const float* e_uncond, float c
                   const float* e_old3, int order, const float* noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
                   float sqrt_one_minus_at, float temperature, float* e_out, float* e_prime_out, float* pred_x0, float* x_prev,
                   long long n, void* stream);
+/* ---- multistep DPM-Solver++ update ------------------------------------------------------------
+ * Replaces one model evaluation's arithmetic in DPM_Solver.sample(method='multistep') with predict_x0=True and
+ * solver_type='dpm_solver' (CompVis ldm/models/diffusion/dpm_solver/dpm_solver.py: model_wrapper's classifier-free
+ * combine, data_prediction_fn, and dpm_solver_first_update / multistep_dpm_solver_second_update / _third_update):
+ *   e    = e_uncond + cfg_scale*(e - e_uncond)                        (if e_uncond != NULL)
+ *   m0   = (x - sigma_s*e) / alpha_s                                  data prediction at the evaluated time s = t_prev_0
+ *   order 1: x_next = c_x*x - c_0*m0                                  c_x = sigma_t/sigma_s, c_0 = alpha_t*expm1(-h)
+ *   order 2: D1_0 = inv_r0*(m0 - m1)                                  inv_r0 = 1/r0, c_x = sigma_t/sigma_prev_0,
+ *            x_next = c_x*x - c_0*m0 - c_1*D1_0                       c_0 = alpha_t*(exp(-h) - 1), c_1 = 0.5*c_0
+ *   order 3: D1_0 = inv_r0*(m0 - m1), D1_1 = inv_r1*(m1 - m2)         c_r = r0/(r0 + r1), c_d2 = 1/(r0 + r1),
+ *            D1 = D1_0 + c_r*(D1_0 - D1_1), D2 = c_d2*(D1_0 - D1_1)   c_1 = alpha_t*((exp(-h) - 1)/h + 1),
+ *            x_next = c_x*x - c_0*m0 + c_1*D1 - c_2*D2                c_2 = alpha_t*((exp(-h) - 1 + h)/h^2 - 0.5)
+ * (m1 = model_prev_list[-2], m2 = model_prev_list[-3]; h = lambda_t - lambda_prev_0, r0 = h_0/h, r1 = h_1/h.)  All fp32, every
+ * operation individually rounded (no FMA contraction) in the reference's left-to-right order; the scalars are computed by
+ * the caller.  Coefficients the order does not read are ignored, and so are history pointers.  Outputs, each optional but at
+ * least one: x_next, m0_out = m0 (the history entry the next updates read).  No output may overlap an input or the other
+ * output.  n = number of elements of every operand. */
+int sdb_dpm_solver_step(const float* x, const float* e, const float* e_uncond, float cfg_scale, float sigma_s, float alpha_s,
+                        const float* m1, const float* m2, int order, float c_x, float c_0, float c_1, float c_2, float inv_r0,
+                        float inv_r1, float c_r, float c_d2, float* x_next, float* m0_out, long long n, void* stream);
 /* ---- ancestral (DDPM) update ---------------------------------------------------------------
  * Replaces LatentDiffusion.p_sample's arithmetic (ldm/diffusion/ddpm.py:1528-1793: predict_start_from_noise,
  * x_recon.clamp_, q_posterior, `model_mean + nonzero_mask * (0.5 * model_log_variance).exp() * noise`):

@@ -4,6 +4,7 @@ ProgramerSalar/stable-diffusion-from-scratch, behind the reference's own Python 
     from sdb200.openai_model import UNetModel          # reference: openai_model/model.py:259
     from sdb200.ddim import DDIMSampler                # reference: ldm/diffusion/ddim.py:12
     from sdb200.plms import PLMSSampler                # reference: CompVis ldm/models/diffusion/plms.py
+    from sdb200.dpm_solver import DPMSolverSampler     # reference: CompVis ldm/models/diffusion/dpm_solver/
     from sdb200.autoencoder import AutoencoderKL       # reference: ldm/models/autoencoder.py:292
     from sdb200.ddpm_unet import UNet                  # reference: DDPM/models/unet.py:11
 

@@ -109,6 +109,7 @@ SIGNATURES = {
     "sdb_ddim_step": (_I, [_P, _P, _P, _F, _P, _F, _F, _F, _F, _F, _F, _P, _P, _L, _P]),
     "sdb_ddim_xprev": (_I, [_P, _P, _P, _F, _P, _F, _F, _F, _F, _P, _L, _P]),
     "sdb_plms_step": (_I, [_P, _P, _P, _F, _P, _P, _P, _I, _P, _F, _F, _F, _F, _F, _F, _P, _P, _P, _P, _L, _P]),
+    "sdb_dpm_solver_step": (_I, [_P, _P, _P, _F, _F, _F, _P, _P, _I, _F, _F, _F, _F, _F, _F, _F, _F, _P, _P, _L, _P]),
     "sdb_ddpm_step": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _F, _P, _P, _I, _L, _P]),
     "sdb_inpaint_blend": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _L, _P, _P]),
     "sdb_diag_gaussian": (_I, [_P, _P, _I, _I, _L, _P, _P, _P, _P, _P, _P]),

@@ -446,6 +446,71 @@ plms_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, con
     }
 }
 
+// ---- multistep DPM-Solver++ update (CompVis ldm/models/diffusion/dpm_solver/dpm_solver.py, predict_x0, 'dpm_solver') ------
+//   e   = e_u given ? e_u + cfg * (e - e_u) : e                              (model_wrapper, classifier-free)
+//   m0  = (x - sigma_s * e) / alpha_s                                        (data_prediction_fn at the evaluated time)
+//   order 1: x_t = c_x x - c_0 m0                                            (dpm_solver_first_update)
+//   order 2: D1_0 = inv_r0 (m0 - m1); x_t = c_x x - c_0 m0 - c_1 D1_0        (multistep_dpm_solver_second_update)
+//   order 3: D1_0 = inv_r0 (m0 - m1); D1_1 = inv_r1 (m1 - m2); D1 = D1_0 + c_r (D1_0 - D1_1); D2 = c_d2 (D1_0 - D1_1);
+//            x_t = c_x x - c_0 m0 + c_1 D1 - c_2 D2                          (multistep_dpm_solver_third_update)
+// Separately rounded fp32 operations, left to right as the eager reference evaluates them.
+struct DpmCoef { float sigma_s, alpha_s, c_x, c_0, c_1, c_2, inv_r0, inv_r1, c_r, c_d2; };
+struct DpmOut { float m0, xn; };
+
+__device__ __forceinline__ DpmOut dpm_update_1(int order, float xv, float e, bool has_u, float u, float cfg, float m1, float m2,
+                                               const DpmCoef& k) {
+    if (has_u) e = cfg_combine_1(e, u, cfg);
+    DpmOut r;
+    r.m0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(k.sigma_s, e)), k.alpha_s);
+    r.xn = __fsub_rn(__fmul_rn(k.c_x, xv), __fmul_rn(k.c_0, r.m0));
+    if (order >= 2) {
+        const float d10 = __fmul_rn(k.inv_r0, __fsub_rn(r.m0, m1));
+        if (order == 2) {
+            r.xn = __fsub_rn(r.xn, __fmul_rn(k.c_1, d10));
+        } else {
+            const float d11 = __fmul_rn(k.inv_r1, __fsub_rn(m1, m2));
+            const float dd = __fsub_rn(d10, d11);
+            const float d1 = __fadd_rn(d10, __fmul_rn(k.c_r, dd));
+            const float d2 = __fmul_rn(k.c_d2, dd);
+            r.xn = __fsub_rn(__fadd_rn(r.xn, __fmul_rn(k.c_1, d1)), __fmul_rn(k.c_2, d2));
+        }
+    }
+    return r;
+}
+
+// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, n % 4 == 0), VEC = 1: any alignment.  History pointers the
+// order does not read are NULL (the host clears them), and so is the output not requested.
+template <int VEC>
+__global__ void __launch_bounds__(256)
+dpm_solver_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, const float* __restrict__ e_u, float cfg,
+                       const float* __restrict__ m1, const float* __restrict__ m2, int order, DpmCoef k,
+                       float* __restrict__ x_next, float* __restrict__ m0_out, long long n) {
+    pdl_trigger();
+    pdl_wait();
+    const long long nv = n / VEC;
+    const bool hu = e_u != nullptr;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+        if (VEC == 4) {
+            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+            const float4 x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
+            const float4 e4 = __ldg(reinterpret_cast<const float4*>(e_c) + i);
+            const float4 u4 = hu ? __ldg(reinterpret_cast<const float4*>(e_u) + i) : zero;
+            const float4 a4 = m1 ? __ldg(reinterpret_cast<const float4*>(m1) + i) : zero;
+            const float4 b4 = m2 ? __ldg(reinterpret_cast<const float4*>(m2) + i) : zero;
+            const DpmOut rx = dpm_update_1(order, x4.x, e4.x, hu, u4.x, cfg, a4.x, b4.x, k);
+            const DpmOut ry = dpm_update_1(order, x4.y, e4.y, hu, u4.y, cfg, a4.y, b4.y, k);
+            const DpmOut rz = dpm_update_1(order, x4.z, e4.z, hu, u4.z, cfg, a4.z, b4.z, k);
+            const DpmOut rw = dpm_update_1(order, x4.w, e4.w, hu, u4.w, cfg, a4.w, b4.w, k);
+            if (x_next) reinterpret_cast<float4*>(x_next)[i] = make_float4(rx.xn, ry.xn, rz.xn, rw.xn);
+            if (m0_out) reinterpret_cast<float4*>(m0_out)[i] = make_float4(rx.m0, ry.m0, rz.m0, rw.m0);
+        } else {
+            const DpmOut r = dpm_update_1(order, x[i], e_c[i], hu, hu ? e_u[i] : 0.f, cfg, m1 ? m1[i] : 0.f, m2 ? m2[i] : 0.f, k);
+            if (x_next) x_next[i] = r.xn;
+            if (m0_out) m0_out[i] = r.m0;
+        }
+    }
+}
+
 // ---- ancestral (DDPM) update of LatentDiffusion.p_sample (ldm/diffusion/ddpm.py:1528-1793) -----------------------
 //   x0   = x0_in given ? x0_in : sqrt_recip[t]*x - sqrt_recipm1[t]*eps     (predict_start_from_noise)
 //   x0   = clip ? clamp(x0, -1, 1) : x0                                     (x_recon.clamp_, NaN passes through)
@@ -892,6 +957,35 @@ int sdb_plms_step(const float* x, const float* e, const float* e_uncond, float c
                    e_prime_out, pred_x0, x_prev, n);
     }
     return check_launch("plms_step_kernel");
+}
+
+int sdb_dpm_solver_step(const float* x, const float* e, const float* e_uncond, float cfg_scale, float sigma_s, float alpha_s,
+                        const float* m1, const float* m2, int order, float c_x, float c_0, float c_1, float c_2, float inv_r0,
+                        float inv_r1, float c_r, float c_d2, float* x_next, float* m0_out, long long n, void* stream) {
+    SDB_REQUIRE(x && e && n > 0, "dpm_solver_step: null input or empty problem (n=%lld)", n);
+    SDB_REQUIRE(order >= 1 && order <= 3, "dpm_solver_step: order %d outside 1..3", order);
+    SDB_REQUIRE(order < 2 || m1, "dpm_solver_step: order %d needs m1", order);
+    SDB_REQUIRE(order < 3 || m2, "dpm_solver_step: order 3 needs m2");
+    SDB_REQUIRE(x_next || m0_out, "dpm_solver_step: no output requested");
+    const float* h1 = order >= 2 ? m1 : nullptr;
+    const float* h2 = order >= 3 ? m2 : nullptr;
+    const float* ins[] = {x, e, e_uncond, h1, h2};
+    float* outs[] = {x_next, m0_out};
+    for (int j = 0; j < 2; ++j)
+        for (const float* in : ins) SDB_REQUIRE(!ranges_overlap(outs[j], in, n), "dpm_solver_step: output %d overlaps an input", j);
+    SDB_REQUIRE(!ranges_overlap(x_next, m0_out, n), "dpm_solver_step: outputs x_next and m0_out overlap");
+    const DpmCoef k{sigma_s, alpha_s, c_x, c_0, c_1, c_2, inv_r0, inv_r1, c_r, c_d2};
+    uintptr_t al = 0;
+    for (const float* p : ins) al |= reinterpret_cast<uintptr_t>(p);
+    for (const float* p : outs) al |= reinterpret_cast<uintptr_t>(p);
+    if ((al & 15) == 0 && n % 4 == 0) {
+        launch_pdl(dpm_solver_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond,
+                   cfg_scale, h1, h2, order, k, x_next, m0_out, n);
+    } else {
+        launch_pdl(dpm_solver_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond,
+                   cfg_scale, h1, h2, order, k, x_next, m0_out, n);
+    }
+    return check_launch("dpm_solver_step_kernel");
 }
 
 int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const float* noise, const long long* t,

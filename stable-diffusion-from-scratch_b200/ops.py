@@ -327,6 +327,25 @@ def plms_step(x, e, order, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minu
     return tuple(outs)
 
 
+def dpm_solver_step(x, e, order, coef, e_uncond=None, cfg_scale=1.0, m1=None, m2=None, want_x_next=True, want_m0=True):
+    """One fused multistep DPM-Solver++ update (see include/sdb200.h sdb_dpm_solver_step): guidance combine, the data
+    prediction m0 at the evaluated time and the order-`order` update.  coef = the ten fp32 scalars (sigma_s, alpha_s, c_x, c_0,
+    c_1, c_2, inv_r0, inv_r1, c_r, c_d2) in that order; m1 / m2 = model_prev_list[-2] / [-3] as far as the order reads them.
+    Every tensor operand must be contiguous fp32 with x's element count.  Returns (x_next, m0), each None unless requested."""
+    require_cuda(x, e, e_uncond, m1, m2)
+    _f32c("x", x)
+    for name, t in (("e", e), ("e_uncond", e_uncond), ("m1", m1), ("m2", m2)):
+        _f32c(name, t, x)
+    coef = [float(v) for v in coef]
+    if len(coef) != 10:
+        raise ValueError("dpm_solver_step: coef has %d scalars, expected 10" % len(coef))
+    outs = [torch.empty_like(x) if w else None for w in (want_x_next, want_m0)]
+    check(_L().sdb_dpm_solver_step(ptr(x), ptr(e), ptr(e_uncond), float(cfg_scale), coef[0], coef[1], ptr(m1), ptr(m2),
+                                   int(order), *coef[2:], *[ptr(o) for o in outs], x.numel(), stream_ptr()),
+          "dpm_solver_step")
+    return tuple(outs)
+
+
 def ddpm_step(x, t, table, eps=None, x0=None, noise=None, clip=False, temperature=1.0, want_x_prev=True, want_x0=False):
     """One fused ancestral update (LatentDiffusion.p_sample arithmetic, see include/sdb200.h sdb_ddpm_step).
     x / eps / x0 / noise: contiguous fp32 [B, ...] with x's element count; t: int64 [B] on the device; table: fp32 [5, T]

@@ -16,6 +16,7 @@ from torch import nn
 from . import engine, ops
 from .autoencoder import AutoencoderKL, DiagonalGaussianDistribution, VQModelInterface
 from .ddim import DDIMSampler
+from .dpm_solver import DPMSolverSampler
 from .openai_model import UNetModel
 from .plms import PLMSSampler
 
@@ -406,12 +407,15 @@ class LatentDiffusion(nn.Module):
 
     @torch.no_grad()
     def txt2img(self, cond, batch_size, ddim_steps=50, shape=(4, 64, 64), x_T=None, eta=0.0,
-                unconditional_guidance_scale=1.0, unconditional_conditioning=None, plms=False):
-        """DDIM-`ddim_steps` (plms=True: PLMS-`ddim_steps`, as scripts/txt2img.py --plms; eta must be 0) + VAE decode:
-        latents and [-1,1] images."""
+                unconditional_guidance_scale=1.0, unconditional_conditioning=None, plms=False, dpm_solver=False):
+        """DDIM-`ddim_steps` (plms=True: PLMS-`ddim_steps`, as scripts/txt2img.py --plms; eta must be 0.  dpm_solver=True:
+        DPM-Solver++(2M) with `ddim_steps` model evaluations, as --dpm_solver, eta ignored; it wins over plms, as in
+        txt2img.py) + VAE decode: latents and [-1,1] images."""
         kw = dict(x_T=x_T, eta=eta, unconditional_guidance_scale=unconditional_guidance_scale,
                   unconditional_conditioning=unconditional_conditioning)
-        if plms:
+        if dpm_solver:
+            z, _ = DPMSolverSampler(self).sample(ddim_steps, batch_size, shape, cond, verbose=False, **kw)
+        elif plms:
             z, _ = PLMSSampler(self).sample(ddim_steps, batch_size, shape, cond, verbose=False, **kw)
         else:
             z, _ = self.sample_log(cond, batch_size, ddim=True, ddim_steps=ddim_steps, shape=shape, **kw)
