@@ -172,13 +172,15 @@ int sdb_skinny_linear_bf16w(const float* x, int M, int K, const void* W /* bf16 
  * all fp32, every operation individually rounded (no FMA contraction) like the eager reference.
  * The caller passes the derived per-step scalars sqrt_at = a_t.sqrt(), sqrt_aprev = a_prev.sqrt(),
  * dir_coef = (1 - a_prev - sigma_t**2).sqrt() (ddim.py:197-205) so that it can evaluate them with the
- * reference's own expressions.  noise may be NULL when sigma_t == 0.  n = number of elements. */
+ * reference's own expressions.  noise may be NULL when sigma_t == 0.  No output may overlap an input or the other
+ * output.  n = number of elements. */
 int sdb_ddim_step(const float* x, const float* e_cond, const float* e_uncond, float cfg_scale,
                   const float* noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
                   float sqrt_one_minus_at, float temperature, float* x_prev, float* pred_x0, long long n,
                   void* stream);
 /* Second half of the same update for the quantize_denoised branch (ldm/diffusion/ddim.py:198-205): pred_x0 is GIVEN
- * (the caller replaced it by first_stage_model.quantize(pred_x0)), x_prev = sqrt_aprev*pred_x0 + dir_coef*e + sigma_t*noise*temperature. */
+ * (the caller replaced it by first_stage_model.quantize(pred_x0)), x_prev = sqrt_aprev*pred_x0 + dir_coef*e + sigma_t*noise*temperature.
+ * x_prev may not overlap an input. */
 int sdb_ddim_xprev(const float* pred_x0, const float* e_cond, const float* e_uncond, float cfg_scale, const float* noise,
                    float sqrt_aprev, float dir_coef, float sigma_t, float temperature, float* x_prev, long long n, void* stream);
 /* ---- PLMS update ---------------------------------------------------------------------------
@@ -233,7 +235,8 @@ int sdb_dpm_solver_step(const float* x, const float* e, const float* e_uncond, f
  * sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod, posterior_mean_coef1, posterior_mean_coef2 and
  * posterior_std = exp(0.5 * posterior_log_variance_clipped), gathered per sample inside the kernel.  eps may be NULL
  * when x0_in is given; x_prev and x0_out are each optional, not both (x0_out only: predict_start_from_noise; no noise:
- * the posterior mean).  A t[b] outside [0, T) writes NaN into sample b and is never used as an index. */
+ * the posterior mean).  eps is ignored when x0_in is given.  No output may overlap an input the call reads or the other output.
+ * A t[b] outside [0, T) writes NaN into sample b and is never used as an index. */
 int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const float* noise, const long long* t,
                   const float* table, int T, int clip, float temperature, float* x_prev, float* x0_out, int B, long long per,
                   void* stream);

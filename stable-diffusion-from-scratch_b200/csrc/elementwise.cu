@@ -310,6 +310,44 @@ __global__ void skinny_linear_kernel(const float* __restrict__ x, int M, int K, 
     }
 }
 
+// ---- fused sampler updates: one pointwise driver, one op per update ------------------------------------------------------
+// sampler_update_kernel<VEC, Op> runs Op over n fp32 elements.  VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned
+// and n % 4 == 0; DdpmStep also needs per % 4 == 0, so that a vector never straddles two samples), VEC = 1: any alignment.
+// An op names its NIN elementwise inputs in `ins` and its NOUT outputs in `outs`.  The first NREQ inputs are never NULL.  The
+// kernel reads exactly the inputs that are non-NULL (a NULL one reads as 0; the host sets to NULL every input the call does not
+// read) and stores exactly the outputs that are non-NULL.  op.apply(in, out, i0) maps the VEC elements of every input that start
+// at element i0 to those of every output.
+// At SD-1.x sizes a launch is latency-bound (about 2.5 us on a B200; figures in DESIGN.md §0, sampler-update driver).  Two
+// choices here bring PLMS close to the 2.58 us per launch of its former kernel: 2.60 us with both, 2.77 with a NULL test on the
+// NREQ inputs, 2.64 without __grid_constant__.  __grid_constant__ costs the DDIM and DDPM updates 0.02-0.06 us; they stay
+// faster than their former kernels.
+template <int VEC, class Op>
+__global__ void __launch_bounds__(256) sampler_update_kernel(const __grid_constant__ Op op, long long n) {
+    pdl_trigger();
+    pdl_wait();
+    const long long nv = n / VEC;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+        float in[Op::NIN][VEC], out[Op::NOUT][VEC];
+#pragma unroll
+        for (int k = 0; k < Op::NIN; ++k) {
+            const bool read = k < Op::NREQ || op.ins[k];
+            if constexpr (VEC == 4) {
+                const float4 a = read ? __ldg(reinterpret_cast<const float4*>(op.ins[k]) + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+                in[k][0] = a.x; in[k][1] = a.y; in[k][2] = a.z; in[k][3] = a.w;
+            } else {
+                in[k][0] = read ? __ldg(op.ins[k] + i) : 0.f;
+            }
+        }
+        op.apply(in, out, i * VEC);
+#pragma unroll
+        for (int k = 0; k < Op::NOUT; ++k) {
+            if (!op.outs[k]) continue;
+            if constexpr (VEC == 4) reinterpret_cast<float4*>(op.outs[k])[i] = make_float4(out[k][0], out[k][1], out[k][2], out[k][3]);
+            else op.outs[k][i] = out[k][0];
+        }
+    }
+}
+
 // ---- DDIM update (reference ldm/diffusion/ddim.py:175-205) --------------------------------------
 // Every operation is a separately rounded fp32 op (__f*_rn blocks FMA contraction) so that, given
 // the same eps, x_prev / pred_x0 are bit-identical to the eager reference arithmetic.
@@ -318,7 +356,7 @@ __device__ __forceinline__ float cfg_combine_1(float e, float u, float cfg) {
     return __fadd_rn(u, __fmul_rn(cfg, __fsub_rn(e, u)));
 }
 
-// One element of the update; `p0_in` != NULL: pred_x0 is given (quantize_denoised branch, ddim.py:198-199) and only x_prev is formed.
+// One element of the update; `p0_given`: pred_x0 is given (quantize_denoised branch, ddim.py:198-199) and only x_prev is formed.
 __device__ __forceinline__ void ddim_update_1(float xv, float e, bool has_u, float u, float cfg, bool has_nz, float nzv,
                                               float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
                                               float sqrt_one_minus_at, float temperature, bool p0_given, float& p0, float& xp) {
@@ -330,41 +368,23 @@ __device__ __forceinline__ void ddim_update_1(float xv, float e, bool has_u, flo
     xp = __fadd_rn(__fadd_rn(__fmul_rn(sqrt_aprev, p0), dir), nz);
 }
 
-// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, n % 4 == 0), VEC = 1: any alignment.  HBM-bound:
-// 16 B / element at eta = 0 (x, e in; x_prev, pred_x0 out), + 4 with noise, + 4 with classifier-free guidance.
-template <int VEC>
-__global__ void __launch_bounds__(256)
-ddim_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, const float* __restrict__ e_u, float cfg,
-                 const float* __restrict__ noise, const float* __restrict__ p0_in, float sqrt_at, float sqrt_aprev, float dir_coef,
-                 float sigma_t, float sqrt_one_minus_at, float temperature, float* __restrict__ x_prev,
-                 float* __restrict__ pred_x0, long long n) {
-    pdl_trigger();
-    pdl_wait();
-    const long long nv = n / VEC;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
-        if (VEC == 4) {
-            const float4 e4 = __ldg(reinterpret_cast<const float4*>(e_c) + i);
-            float4 u4 = make_float4(0.f, 0.f, 0.f, 0.f), n4 = u4, x4 = u4, p4 = u4, o4;
-            if (e_u) u4 = __ldg(reinterpret_cast<const float4*>(e_u) + i);
-            if (noise) n4 = __ldg(reinterpret_cast<const float4*>(noise) + i);
-            if (p0_in) p4 = __ldg(reinterpret_cast<const float4*>(p0_in) + i);
-            else x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
-            const bool hu = e_u != nullptr, hn = noise != nullptr, pg = p0_in != nullptr;
-            ddim_update_1(x4.x, e4.x, hu, u4.x, cfg, hn, n4.x, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, pg, p4.x, o4.x);
-            ddim_update_1(x4.y, e4.y, hu, u4.y, cfg, hn, n4.y, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, pg, p4.y, o4.y);
-            ddim_update_1(x4.z, e4.z, hu, u4.z, cfg, hn, n4.z, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, pg, p4.z, o4.z);
-            ddim_update_1(x4.w, e4.w, hu, u4.w, cfg, hn, n4.w, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, pg, p4.w, o4.w);
-            reinterpret_cast<float4*>(x_prev)[i] = o4;
-            if (pred_x0) reinterpret_cast<float4*>(pred_x0)[i] = p4;
-        } else {
-            float p0 = p0_in ? p0_in[i] : 0.f, xp;
-            ddim_update_1(p0_in ? 0.f : x[i], e_c[i], e_u != nullptr, e_u ? e_u[i] : 0.f, cfg, noise != nullptr, noise ? noise[i] : 0.f,
-                          sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, p0_in != nullptr, p0, xp);
-            x_prev[i] = xp;
-            if (pred_x0) pred_x0[i] = p0;
+// HBM-bound: 16 B / element at eta = 0 (x, e in; x_prev, pred_x0 out), + 4 with noise, + 4 with classifier-free guidance.
+// p0_in given: the quantize_denoised branch (ddim.py:198-205); x is not read and pred_x0 is not written.
+struct DdimStep {
+    static constexpr int NIN = 5, NOUT = 2, NREQ = 1;
+    const float* ins[NIN];   // e_cond, x, e_uncond, noise, p0_in
+    float* outs[NOUT];       // x_prev, pred_x0
+    float cfg, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature;
+    template <int VEC>
+    __device__ __forceinline__ void apply(const float (&in)[NIN][VEC], float (&out)[NOUT][VEC], long long) const {
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) {
+            out[1][j] = in[4][j];
+            ddim_update_1(in[1][j], in[0][j], ins[2] != nullptr, in[2][j], cfg, ins[3] != nullptr, in[3][j], sqrt_at, sqrt_aprev,
+                          dir_coef, sigma_t, sqrt_one_minus_at, temperature, ins[4] != nullptr, out[1][j], out[0][j]);
         }
     }
-}
+};
 
 // ---- PLMS update (ldm/models/diffusion/plms.py, p_sample_plms) ------------------------------------------------------------
 //   e  = e_u given ? e_u + cfg * (e - e_u) : e                       (written to e_out: what the eps history keeps)
@@ -399,52 +419,24 @@ __device__ __forceinline__ PlmsOut plms_update_1(int order, float xv, float e, b
     return r;
 }
 
-// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, n % 4 == 0), VEC = 1: any alignment.  History pointers the
-// order does not read are NULL (the host clears them), and so are the outputs not requested.
-template <int VEC>
-__global__ void __launch_bounds__(256)
-plms_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, const float* __restrict__ e_u, float cfg,
-                 const float* __restrict__ o1, const float* __restrict__ o2, const float* __restrict__ o3, int order,
-                 const float* __restrict__ noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
-                 float sqrt_one_minus_at, float temperature, float* __restrict__ e_out, float* __restrict__ ep_out,
-                 float* __restrict__ pred_x0, float* __restrict__ x_prev, long long n) {
-    pdl_trigger();
-    pdl_wait();
-    const long long nv = n / VEC;
-    const bool hu = e_u != nullptr, hn = noise != nullptr;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
-        if (VEC == 4) {
-            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-            const float4 x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
-            const float4 e4 = __ldg(reinterpret_cast<const float4*>(e_c) + i);
-            const float4 u4 = hu ? __ldg(reinterpret_cast<const float4*>(e_u) + i) : zero;
-            const float4 a4 = o1 ? __ldg(reinterpret_cast<const float4*>(o1) + i) : zero;
-            const float4 b4 = o2 ? __ldg(reinterpret_cast<const float4*>(o2) + i) : zero;
-            const float4 c4 = o3 ? __ldg(reinterpret_cast<const float4*>(o3) + i) : zero;
-            const float4 n4 = hn ? __ldg(reinterpret_cast<const float4*>(noise) + i) : zero;
-            const PlmsOut rx = plms_update_1(order, x4.x, e4.x, hu, u4.x, cfg, a4.x, b4.x, c4.x, hn, n4.x, sqrt_at, sqrt_aprev,
-                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
-            const PlmsOut ry = plms_update_1(order, x4.y, e4.y, hu, u4.y, cfg, a4.y, b4.y, c4.y, hn, n4.y, sqrt_at, sqrt_aprev,
-                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
-            const PlmsOut rz = plms_update_1(order, x4.z, e4.z, hu, u4.z, cfg, a4.z, b4.z, c4.z, hn, n4.z, sqrt_at, sqrt_aprev,
-                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
-            const PlmsOut rw = plms_update_1(order, x4.w, e4.w, hu, u4.w, cfg, a4.w, b4.w, c4.w, hn, n4.w, sqrt_at, sqrt_aprev,
-                                             dir_coef, sigma_t, sqrt_one_minus_at, temperature);
-            if (e_out) reinterpret_cast<float4*>(e_out)[i] = make_float4(rx.e, ry.e, rz.e, rw.e);
-            if (ep_out) reinterpret_cast<float4*>(ep_out)[i] = make_float4(rx.ep, ry.ep, rz.ep, rw.ep);
-            if (pred_x0) reinterpret_cast<float4*>(pred_x0)[i] = make_float4(rx.p0, ry.p0, rz.p0, rw.p0);
-            if (x_prev) reinterpret_cast<float4*>(x_prev)[i] = make_float4(rx.xp, ry.xp, rz.xp, rw.xp);
-        } else {
-            const PlmsOut r = plms_update_1(order, x[i], e_c[i], hu, hu ? e_u[i] : 0.f, cfg, o1 ? o1[i] : 0.f, o2 ? o2[i] : 0.f,
-                                            o3 ? o3[i] : 0.f, hn, hn ? noise[i] : 0.f, sqrt_at, sqrt_aprev, dir_coef, sigma_t,
-                                            sqrt_one_minus_at, temperature);
-            if (e_out) e_out[i] = r.e;
-            if (ep_out) ep_out[i] = r.ep;
-            if (pred_x0) pred_x0[i] = r.p0;
-            if (x_prev) x_prev[i] = r.xp;
+struct PlmsStep {
+    static constexpr int NIN = 7, NOUT = 4, NREQ = 2;
+    const float* ins[NIN];   // x, e, e_uncond, o1, o2, o3, noise
+    float* outs[NOUT];       // e_out, ep_out, pred_x0, x_prev
+    float cfg;
+    int order;
+    float sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature;
+    template <int VEC>
+    __device__ __forceinline__ void apply(const float (&in)[NIN][VEC], float (&out)[NOUT][VEC], long long) const {
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) {
+            const PlmsOut r = plms_update_1(order, in[0][j], in[1][j], ins[2] != nullptr, in[2][j], cfg, in[3][j], in[4][j], in[5][j],
+                                            ins[6] != nullptr, in[6][j], sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at,
+                                            temperature);
+            out[0][j] = r.e; out[1][j] = r.ep; out[2][j] = r.p0; out[3][j] = r.xp;
         }
     }
-}
+};
 
 // ---- multistep DPM-Solver++ update (CompVis ldm/models/diffusion/dpm_solver/dpm_solver.py, predict_x0, 'dpm_solver') ------
 //   e   = e_u given ? e_u + cfg * (e - e_u) : e                              (model_wrapper, classifier-free)
@@ -478,38 +470,22 @@ __device__ __forceinline__ DpmOut dpm_update_1(int order, float xv, float e, boo
     return r;
 }
 
-// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, n % 4 == 0), VEC = 1: any alignment.  History pointers the
-// order does not read are NULL (the host clears them), and so is the output not requested.
-template <int VEC>
-__global__ void __launch_bounds__(256)
-dpm_solver_step_kernel(const float* __restrict__ x, const float* __restrict__ e_c, const float* __restrict__ e_u, float cfg,
-                       const float* __restrict__ m1, const float* __restrict__ m2, int order, DpmCoef k,
-                       float* __restrict__ x_next, float* __restrict__ m0_out, long long n) {
-    pdl_trigger();
-    pdl_wait();
-    const long long nv = n / VEC;
-    const bool hu = e_u != nullptr;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
-        if (VEC == 4) {
-            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-            const float4 x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
-            const float4 e4 = __ldg(reinterpret_cast<const float4*>(e_c) + i);
-            const float4 u4 = hu ? __ldg(reinterpret_cast<const float4*>(e_u) + i) : zero;
-            const float4 a4 = m1 ? __ldg(reinterpret_cast<const float4*>(m1) + i) : zero;
-            const float4 b4 = m2 ? __ldg(reinterpret_cast<const float4*>(m2) + i) : zero;
-            const DpmOut rx = dpm_update_1(order, x4.x, e4.x, hu, u4.x, cfg, a4.x, b4.x, k);
-            const DpmOut ry = dpm_update_1(order, x4.y, e4.y, hu, u4.y, cfg, a4.y, b4.y, k);
-            const DpmOut rz = dpm_update_1(order, x4.z, e4.z, hu, u4.z, cfg, a4.z, b4.z, k);
-            const DpmOut rw = dpm_update_1(order, x4.w, e4.w, hu, u4.w, cfg, a4.w, b4.w, k);
-            if (x_next) reinterpret_cast<float4*>(x_next)[i] = make_float4(rx.xn, ry.xn, rz.xn, rw.xn);
-            if (m0_out) reinterpret_cast<float4*>(m0_out)[i] = make_float4(rx.m0, ry.m0, rz.m0, rw.m0);
-        } else {
-            const DpmOut r = dpm_update_1(order, x[i], e_c[i], hu, hu ? e_u[i] : 0.f, cfg, m1 ? m1[i] : 0.f, m2 ? m2[i] : 0.f, k);
-            if (x_next) x_next[i] = r.xn;
-            if (m0_out) m0_out[i] = r.m0;
+struct DpmSolverStep {
+    static constexpr int NIN = 5, NOUT = 2, NREQ = 2;
+    const float* ins[NIN];   // x, e, e_uncond, m1, m2
+    float* outs[NOUT];       // x_next, m0_out
+    float cfg;
+    int order;
+    DpmCoef k;
+    template <int VEC>
+    __device__ __forceinline__ void apply(const float (&in)[NIN][VEC], float (&out)[NOUT][VEC], long long) const {
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) {
+            const DpmOut r = dpm_update_1(order, in[0][j], in[1][j], ins[2] != nullptr, in[2][j], cfg, in[3][j], in[4][j], k);
+            out[0][j] = r.xn; out[1][j] = r.m0;
         }
     }
-}
+};
 
 // ---- ancestral (DDPM) update of LatentDiffusion.p_sample (ldm/diffusion/ddpm.py:1528-1793) -----------------------
 //   x0   = x0_in given ? x0_in : sqrt_recip[t]*x - sqrt_recipm1[t]*eps     (predict_start_from_noise)
@@ -527,53 +503,33 @@ __device__ __forceinline__ void ddpm_update_1(float xv, float e, float x0v, bool
     xp = has_nz ? __fadd_rn(mean, __fmul_rn(s, __fmul_rn(nzv, temperature))) : mean;
 }
 
-// VEC = 4: 128-bit loads / stores (every pointer 16-byte aligned, per % 4 == 0, so a vector never straddles two
-// samples), VEC = 1: any alignment.  x_prev / x0_out may each be NULL (not both).
-template <int VEC>
-__global__ void __launch_bounds__(256)
-ddpm_step_kernel(const float* __restrict__ x, const float* __restrict__ eps, const float* __restrict__ x0_in,
-                 const float* __restrict__ noise, const long long* __restrict__ t, const float* __restrict__ table, int T,
-                 int clip, float temperature, float* __restrict__ x_prev, float* __restrict__ x0_out, long long per, long long n) {
-    pdl_trigger();
-    pdl_wait();
-    const long long nv = n / VEC, pv = per / VEC;
-    const bool xg = x0_in != nullptr, cl = clip != 0, hn = noise != nullptr;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
-        const long long tb = __ldg(t + i / pv);
-        const bool ok = tb >= 0 && tb < T;
-        const float qnan = __int_as_float(0x7fc00000);
-        float sr = qnan, srm1 = qnan, c1 = qnan, c2 = qnan, s = qnan;
-        if (ok) {
-            sr = __ldg(table + tb);
-            srm1 = __ldg(table + T + tb);
-            c1 = __ldg(table + 2 * (long long)T + tb);
-            c2 = __ldg(table + 3 * (long long)T + tb);
-            s = __fmul_rn(tb != 0 ? 1.f : 0.f, __ldg(table + 4 * (long long)T + tb));   // nonzero_mask * std
+// The five coefficients are gathered once per vector: every element of a vector belongs to the same sample.
+struct DdpmStep {
+    static constexpr int NIN = 4, NOUT = 2, NREQ = 1;
+    const float* ins[NIN];   // x, eps, x0_in, noise
+    float* outs[NOUT];       // x_prev, x0_out
+    const long long* t;
+    const float* table;
+    int T, clip;
+    float temperature;
+    long long per;
+    template <int VEC>
+    __device__ __forceinline__ void apply(const float (&in)[NIN][VEC], float (&out)[NOUT][VEC], long long i0) const {
+        const long long tb = __ldg(t + i0 / per);
+        if (tb < 0 || tb >= T) {
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) out[0][j] = out[1][j] = __int_as_float(0x7fc00000);
+            return;
         }
-        if (VEC == 4) {
-            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-            const float4 x4 = __ldg(reinterpret_cast<const float4*>(x) + i);
-            const float4 e4 = xg ? zero : __ldg(reinterpret_cast<const float4*>(eps) + i);
-            const float4 g4 = xg ? __ldg(reinterpret_cast<const float4*>(x0_in) + i) : zero;
-            const float4 n4 = hn ? __ldg(reinterpret_cast<const float4*>(noise) + i) : zero;
-            float4 p4, o4;
-            ddpm_update_1(x4.x, e4.x, g4.x, xg, cl, hn, n4.x, sr, srm1, c1, c2, s, temperature, p4.x, o4.x);
-            ddpm_update_1(x4.y, e4.y, g4.y, xg, cl, hn, n4.y, sr, srm1, c1, c2, s, temperature, p4.y, o4.y);
-            ddpm_update_1(x4.z, e4.z, g4.z, xg, cl, hn, n4.z, sr, srm1, c1, c2, s, temperature, p4.z, o4.z);
-            ddpm_update_1(x4.w, e4.w, g4.w, xg, cl, hn, n4.w, sr, srm1, c1, c2, s, temperature, p4.w, o4.w);
-            if (!ok) p4 = o4 = make_float4(qnan, qnan, qnan, qnan);
-            if (x_prev) reinterpret_cast<float4*>(x_prev)[i] = o4;
-            if (x0_out) reinterpret_cast<float4*>(x0_out)[i] = p4;
-        } else {
-            float p0, xp;
-            ddpm_update_1(x[i], xg ? 0.f : eps[i], xg ? x0_in[i] : 0.f, xg, cl, hn, hn ? noise[i] : 0.f, sr, srm1, c1, c2, s,
-                          temperature, p0, xp);
-            if (!ok) p0 = xp = qnan;
-            if (x_prev) x_prev[i] = xp;
-            if (x0_out) x0_out[i] = p0;
-        }
+        const float sr = __ldg(table + tb), srm1 = __ldg(table + T + tb);
+        const float c1 = __ldg(table + 2 * (long long)T + tb), c2 = __ldg(table + 3 * (long long)T + tb);
+        const float s = __fmul_rn(tb != 0 ? 1.f : 0.f, __ldg(table + 4 * (long long)T + tb));   // nonzero_mask * std
+#pragma unroll
+        for (int j = 0; j < VEC; ++j)
+            ddpm_update_1(in[0][j], in[1][j], in[2][j], ins[2] != nullptr, clip != 0, ins[3] != nullptr, in[3][j], sr, srm1, c1, c2,
+                          s, temperature, out[1][j], out[0][j]);
     }
-}
+};
 
 // ---- inpainting blend of ddim_sampling (ldm/diffusion/ddim.py:144-149) with q_sample (ldm/diffusion/ddpm.py:407-412) fused:
 //   img_orig = a[b] * x0 + c[b] * noise;   out = img_orig * mask + (1 - mask) * img
@@ -741,6 +697,32 @@ static int launch_skinny(const float* x, int M, int K, const void* W, const floa
     return check_launch("skinny_linear_kernel");
 }
 
+// [a, a + n) and [b, b + n) (fp32 elements) share an element; NULL never overlaps.
+static bool ranges_overlap(const float* a, const float* b, long long n) {
+    if (!a || !b) return false;
+    const uintptr_t pa = reinterpret_cast<uintptr_t>(a), pb = reinterpret_cast<uintptr_t>(b), len = (uintptr_t)n * sizeof(float);
+    return pa < pb + len && pb < pa + len;
+}
+
+// Launches sampler_update_kernel over n elements.  It first rejects any output that overlaps an input or another output: the
+// kernel reads its inputs through the read-only data cache (__ldg), which needs them unwritten while it runs.  VEC 4 needs every
+// pointer 16-byte aligned and `unit` a multiple of 4.  Every error message starts with "<entry>: ".
+template <class Op>
+static int launch_sampler_update(const char* entry, const Op& op, long long n, long long unit, void* stream) {
+    for (int j = 0; j < Op::NOUT; ++j) {
+        for (const float* in : op.ins) SDB_REQUIRE(!ranges_overlap(op.outs[j], in, n), "%s: output %d overlaps an input", entry, j);
+        for (int k = 0; k < j; ++k) SDB_REQUIRE(!ranges_overlap(op.outs[j], op.outs[k], n), "%s: outputs %d and %d overlap", entry, k, j);
+    }
+    uintptr_t al = 0;
+    for (const float* p : op.ins) al |= reinterpret_cast<uintptr_t>(p);
+    for (const float* p : op.outs) al |= reinterpret_cast<uintptr_t>(p);
+    if ((al & 15) == 0 && unit % 4 == 0)
+        launch_pdl(sampler_update_kernel<4, Op>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream, op, n);
+    else
+        launch_pdl(sampler_update_kernel<1, Op>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream, op, n);
+    return check_launch(entry);
+}
+
 extern "C" {
 
 int sdb_nchw_concat_to_nhwc(const float* src0, int C0, const float* src1, int C1, void* dst, int dst_dtype, int dst_C, int split,
@@ -882,45 +864,24 @@ int sdb_skinny_linear_bf16w(const float* x, int M, int K, const void* W, const f
     return launch_skinny<true>(x, M, K, W, bias, N, act_in, act_out, y, stream);
 }
 
-static int launch_ddim(const float* x, const float* e_cond, const float* e_uncond, float cfg_scale, const float* noise,
-                       const float* p0_in, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t, float sqrt_one_minus_at,
-                       float temperature, float* x_prev, float* pred_x0, long long n, void* stream) {
-    const uintptr_t al = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(e_cond) | reinterpret_cast<uintptr_t>(e_uncond) |
-                         reinterpret_cast<uintptr_t>(noise) | reinterpret_cast<uintptr_t>(p0_in) | reinterpret_cast<uintptr_t>(x_prev) |
-                         reinterpret_cast<uintptr_t>(pred_x0);
-    if ((al & 15) == 0 && n % 4 == 0) {
-        launch_pdl(ddim_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream,
-            x, e_cond, e_uncond, cfg_scale, noise, p0_in, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, x_prev, pred_x0, n);
-    } else {
-        launch_pdl(ddim_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream,
-            x, e_cond, e_uncond, cfg_scale, noise, p0_in, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, x_prev, pred_x0, n);
-    }
-    return check_launch("ddim_step_kernel");
-}
-
 int sdb_ddim_step(const float* x, const float* e_cond, const float* e_uncond, float cfg_scale,
                   const float* noise, float sqrt_at, float sqrt_aprev, float dir_coef, float sigma_t,
                   float sqrt_one_minus_at, float temperature, float* x_prev, float* pred_x0, long long n,
                   void* stream) {
     SDB_REQUIRE(x && e_cond && x_prev && pred_x0 && n > 0, "ddim_step: bad args");
     SDB_REQUIRE(noise || sigma_t == 0.0f, "ddim_step: sigma_t != 0 needs a noise tensor");
-    return launch_ddim(x, e_cond, e_uncond, cfg_scale, noise, nullptr, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at,
-                       temperature, x_prev, pred_x0, n, stream);
+    const DdimStep op{{e_cond, x, e_uncond, noise, nullptr}, {x_prev, pred_x0}, cfg_scale, sqrt_at, sqrt_aprev, dir_coef, sigma_t,
+                      sqrt_one_minus_at, temperature};
+    return launch_sampler_update("ddim_step", op, n, n, stream);
 }
 
 int sdb_ddim_xprev(const float* pred_x0, const float* e_cond, const float* e_uncond, float cfg_scale, const float* noise,
                    float sqrt_aprev, float dir_coef, float sigma_t, float temperature, float* x_prev, long long n, void* stream) {
     SDB_REQUIRE(pred_x0 && e_cond && x_prev && n > 0, "ddim_xprev: bad args");
     SDB_REQUIRE(noise || sigma_t == 0.0f, "ddim_xprev: sigma_t != 0 needs a noise tensor");
-    return launch_ddim(nullptr, e_cond, e_uncond, cfg_scale, noise, pred_x0, 1.0f, sqrt_aprev, dir_coef, sigma_t, 0.0f,
-                       temperature, x_prev, nullptr, n, stream);
-}
-
-// [a, a + n) and [b, b + n) (fp32 elements) share an element; NULL never overlaps.
-static bool ranges_overlap(const float* a, const float* b, long long n) {
-    if (!a || !b) return false;
-    const uintptr_t pa = reinterpret_cast<uintptr_t>(a), pb = reinterpret_cast<uintptr_t>(b), len = (uintptr_t)n * sizeof(float);
-    return pa < pb + len && pb < pa + len;
+    const DdimStep op{{e_cond, nullptr, e_uncond, noise, pred_x0}, {x_prev, nullptr}, cfg_scale, 1.0f, sqrt_aprev, dir_coef, sigma_t, 0.0f,
+                      temperature};
+    return launch_sampler_update("ddim_xprev", op, n, n, stream);
 }
 
 int sdb_plms_step(const float* x, const float* e, const float* e_uncond, float cfg_scale, const float* e_old1, const float* e_old2,
@@ -938,25 +899,9 @@ int sdb_plms_step(const float* x, const float* e, const float* e_uncond, float c
     const float* o1 = (order == 0 || order >= 2) ? e_old1 : nullptr;
     const float* o2 = order >= 3 ? e_old2 : nullptr;
     const float* o3 = order >= 4 ? e_old3 : nullptr;
-    const float* ins[] = {x, e, e_uncond, o1, o2, o3, noise};
-    float* outs[] = {e_out, e_prime_out, pred_x0, x_prev};
-    for (int j = 0; j < 4; ++j) {
-        for (const float* in : ins) SDB_REQUIRE(!ranges_overlap(outs[j], in, n), "plms_step: output %d overlaps an input", j);
-        for (int k = 0; k < j; ++k) SDB_REQUIRE(!ranges_overlap(outs[j], outs[k], n), "plms_step: outputs %d and %d overlap", k, j);
-    }
-    uintptr_t al = 0;
-    for (const float* p : ins) al |= reinterpret_cast<uintptr_t>(p);
-    for (const float* p : outs) al |= reinterpret_cast<uintptr_t>(p);
-    if ((al & 15) == 0 && n % 4 == 0) {
-        launch_pdl(plms_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond, cfg_scale,
-                   o1, o2, o3, order, noise, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, e_out,
-                   e_prime_out, pred_x0, x_prev, n);
-    } else {
-        launch_pdl(plms_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond, cfg_scale,
-                   o1, o2, o3, order, noise, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature, e_out,
-                   e_prime_out, pred_x0, x_prev, n);
-    }
-    return check_launch("plms_step_kernel");
+    const PlmsStep op{{x, e, e_uncond, o1, o2, o3, noise}, {e_out, e_prime_out, pred_x0, x_prev}, cfg_scale, order, sqrt_at,
+                      sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, temperature};
+    return launch_sampler_update("plms_step", op, n, n, stream);
 }
 
 int sdb_dpm_solver_step(const float* x, const float* e, const float* e_uncond, float cfg_scale, float sigma_s, float alpha_s,
@@ -969,23 +914,9 @@ int sdb_dpm_solver_step(const float* x, const float* e, const float* e_uncond, f
     SDB_REQUIRE(x_next || m0_out, "dpm_solver_step: no output requested");
     const float* h1 = order >= 2 ? m1 : nullptr;
     const float* h2 = order >= 3 ? m2 : nullptr;
-    const float* ins[] = {x, e, e_uncond, h1, h2};
-    float* outs[] = {x_next, m0_out};
-    for (int j = 0; j < 2; ++j)
-        for (const float* in : ins) SDB_REQUIRE(!ranges_overlap(outs[j], in, n), "dpm_solver_step: output %d overlaps an input", j);
-    SDB_REQUIRE(!ranges_overlap(x_next, m0_out, n), "dpm_solver_step: outputs x_next and m0_out overlap");
-    const DpmCoef k{sigma_s, alpha_s, c_x, c_0, c_1, c_2, inv_r0, inv_r1, c_r, c_d2};
-    uintptr_t al = 0;
-    for (const float* p : ins) al |= reinterpret_cast<uintptr_t>(p);
-    for (const float* p : outs) al |= reinterpret_cast<uintptr_t>(p);
-    if ((al & 15) == 0 && n % 4 == 0) {
-        launch_pdl(dpm_solver_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond,
-                   cfg_scale, h1, h2, order, k, x_next, m0_out, n);
-    } else {
-        launch_pdl(dpm_solver_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream, x, e, e_uncond,
-                   cfg_scale, h1, h2, order, k, x_next, m0_out, n);
-    }
-    return check_launch("dpm_solver_step_kernel");
+    const DpmSolverStep op{{x, e, e_uncond, h1, h2}, {x_next, m0_out}, cfg_scale, order,
+                           {sigma_s, alpha_s, c_x, c_0, c_1, c_2, inv_r0, inv_r1, c_r, c_d2}};
+    return launch_sampler_update("dpm_solver_step", op, n, n, stream);
 }
 
 int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const float* noise, const long long* t,
@@ -995,17 +926,8 @@ int sdb_ddpm_step(const float* x, const float* eps, const float* x0_in, const fl
     SDB_REQUIRE(eps || x0_in, "ddpm_step: needs eps or a given x0");
     SDB_REQUIRE(x_prev || x0_out, "ddpm_step: no output requested");
     SDB_REQUIRE(T > 0 && B > 0 && per > 0, "ddpm_step: bad shape B=%d per=%lld T=%d", B, per, T);
-    const long long n = (long long)B * per;
-    const uintptr_t al = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(eps) | reinterpret_cast<uintptr_t>(x0_in) |
-                         reinterpret_cast<uintptr_t>(noise) | reinterpret_cast<uintptr_t>(x_prev) | reinterpret_cast<uintptr_t>(x0_out);
-    if ((al & 15) == 0 && per % 4 == 0) {
-        launch_pdl(ddpm_step_kernel<4>, dim3(grid_for(n / 4, 256)), dim3(256), 0, (cudaStream_t)stream,
-            x, eps, x0_in, noise, t, table, T, clip, temperature, x_prev, x0_out, per, n);
-    } else {
-        launch_pdl(ddpm_step_kernel<1>, dim3(grid_for(n, 256)), dim3(256), 0, (cudaStream_t)stream,
-            x, eps, x0_in, noise, t, table, T, clip, temperature, x_prev, x0_out, per, n);
-    }
-    return check_launch("ddpm_step_kernel");
+    const DdpmStep op{{x, x0_in ? nullptr : eps, x0_in, noise}, {x_prev, x0_out}, t, table, T, clip, temperature, per};
+    return launch_sampler_update("ddpm_step", op, (long long)B * per, per, stream);
 }
 
 int sdb_inpaint_blend(const float* x0, const float* noise, const float* a, const float* c, const float* mask, const float* img,

@@ -276,15 +276,20 @@ def _f32c(name, t, like=None):
         raise _lib.SdbError("%s has %d elements, expected %d" % (name, t.numel(), like.numel()))
 
 
+def _sampler_operands(*others, **named):
+    """The fused sampler updates read n fp32 values from every named operand: each one (None = absent) must be a contiguous
+    fp32 tensor with as many elements as the first.  `others` are further operands that only have to be on the device."""
+    require_cuda(*named.values(), *others)
+    like = next(iter(named.values()))
+    for name, t in named.items():
+        _f32c(name, t, like)
+
+
 def ddim_step(x, e_cond, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_at, e_uncond=None, cfg_scale=1.0,
               noise=None, temperature=1.0):
     """One fused DDIM update; the five scalars are the fp32 per-step coefficients (see DDIMSampler.derived_coefficients).
     Every tensor operand must be contiguous fp32 with x's element count (the kernel reads n fp32 values from each)."""
-    require_cuda(x, e_cond, e_uncond, noise)
-    _f32c("x", x)
-    _f32c("e_cond", e_cond, x)
-    _f32c("e_uncond", e_uncond, x)
-    _f32c("noise", noise, x)
+    _sampler_operands(x=x, e_cond=e_cond, e_uncond=e_uncond, noise=noise)
     x_prev = torch.empty_like(x)
     pred_x0 = torch.empty_like(x)
     check(_L().sdb_ddim_step(ptr(x), ptr(e_cond), ptr(e_uncond), float(cfg_scale), ptr(noise), float(sqrt_at), float(sqrt_aprev),
@@ -295,11 +300,7 @@ def ddim_step(x, e_cond, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minus_
 
 def ddim_xprev(pred_x0, e_cond, sqrt_aprev, dir_coef, sigma_t, e_uncond=None, cfg_scale=1.0, noise=None, temperature=1.0):
     """x_prev from a GIVEN pred_x0 (quantize_denoised branch of p_sample_ddim, ldm/diffusion/ddim.py:198-205)."""
-    require_cuda(pred_x0, e_cond, e_uncond, noise)
-    _f32c("pred_x0", pred_x0)
-    _f32c("e_cond", e_cond, pred_x0)
-    _f32c("e_uncond", e_uncond, pred_x0)
-    _f32c("noise", noise, pred_x0)
+    _sampler_operands(pred_x0=pred_x0, e_cond=e_cond, e_uncond=e_uncond, noise=noise)
     x_prev = torch.empty_like(pred_x0)
     check(_L().sdb_ddim_xprev(ptr(pred_x0), ptr(e_cond), ptr(e_uncond), float(cfg_scale), ptr(noise), float(sqrt_aprev),
                               float(dir_coef), float(sigma_t), float(temperature), ptr(x_prev), pred_x0.numel(), stream_ptr()),
@@ -314,11 +315,7 @@ def plms_step(x, e, order, sqrt_at, sqrt_aprev, dir_coef, sigma_t, sqrt_one_minu
     order 0 takes the first evaluation of the step as e_old[0].  Every tensor operand must be contiguous fp32 with x's element
     count.  Returns (e, e', pred_x0, x_prev), each None unless requested."""
     e_old = tuple(e_old) + (None,) * (3 - len(e_old))
-    require_cuda(x, e, e_uncond, noise, *e_old)
-    _f32c("x", x)
-    for name, t in (("e", e), ("e_uncond", e_uncond), ("e_old1", e_old[0]), ("e_old2", e_old[1]), ("e_old3", e_old[2]),
-                    ("noise", noise)):
-        _f32c(name, t, x)
+    _sampler_operands(x=x, e=e, e_uncond=e_uncond, e_old1=e_old[0], e_old2=e_old[1], e_old3=e_old[2], noise=noise)
     outs = [torch.empty_like(x) if w else None for w in (want_e, want_e_prime, want_pred_x0, want_x_prev)]
     check(_L().sdb_plms_step(ptr(x), ptr(e), ptr(e_uncond), float(cfg_scale), ptr(e_old[0]), ptr(e_old[1]), ptr(e_old[2]),
                              int(order), ptr(noise), float(sqrt_at), float(sqrt_aprev), float(dir_coef), float(sigma_t),
@@ -332,10 +329,7 @@ def dpm_solver_step(x, e, order, coef, e_uncond=None, cfg_scale=1.0, m1=None, m2
     prediction m0 at the evaluated time and the order-`order` update.  coef = the ten fp32 scalars (sigma_s, alpha_s, c_x, c_0,
     c_1, c_2, inv_r0, inv_r1, c_r, c_d2) in that order; m1 / m2 = model_prev_list[-2] / [-3] as far as the order reads them.
     Every tensor operand must be contiguous fp32 with x's element count.  Returns (x_next, m0), each None unless requested."""
-    require_cuda(x, e, e_uncond, m1, m2)
-    _f32c("x", x)
-    for name, t in (("e", e), ("e_uncond", e_uncond), ("m1", m1), ("m2", m2)):
-        _f32c(name, t, x)
+    _sampler_operands(x=x, e=e, e_uncond=e_uncond, m1=m1, m2=m2)
     coef = [float(v) for v in coef]
     if len(coef) != 10:
         raise ValueError("dpm_solver_step: coef has %d scalars, expected 10" % len(coef))
@@ -351,11 +345,7 @@ def ddpm_step(x, t, table, eps=None, x0=None, noise=None, clip=False, temperatur
     x / eps / x0 / noise: contiguous fp32 [B, ...] with x's element count; t: int64 [B] on the device; table: fp32 [5, T]
     (LatentDiffusion.ddpm_table).  x0 given replaces predict_start_from_noise (eps is then unused).  noise None: x_prev is
     the posterior mean.  Returns (x_prev or None, x0 or None)."""
-    require_cuda(x, t, table, eps, x0, noise)
-    _f32c("x", x)
-    _f32c("eps", eps, x)
-    _f32c("x0", x0, x)
-    _f32c("noise", noise, x)
+    _sampler_operands(t, table, x=x, eps=eps, x0=x0, noise=noise)
     _f32c("table", table)
     B = x.shape[0]
     if t.dtype != torch.int64 or t.numel() != B or not t.is_contiguous():

@@ -15,7 +15,7 @@ from torch import nn
 
 from . import engine, ops
 from .autoencoder import AutoencoderKL, DiagonalGaussianDistribution, VQModelInterface
-from .ddim import DDIMSampler
+from .ddim import DDIMSampler, _f32_contiguous
 from .dpm_solver import DPMSolverSampler
 from .openai_model import UNetModel
 from .plms import PLMSSampler
@@ -453,10 +453,6 @@ class LatentDiffusion(nn.Module):
         posterior_mean_coef1, posterior_mean_coef2, posterior_std."""
         return self._ddpm_cache()[1]
 
-    @staticmethod
-    def _f32(t):
-        return t if (t is None or (t.dtype == torch.float32 and t.is_contiguous())) else t.float().contiguous()
-
     def _timesteps(self, t, x):
         return t if (t.dtype == torch.long and t.device == x.device and t.is_contiguous()) else t.to(x.device, torch.long).contiguous()
 
@@ -468,23 +464,23 @@ class LatentDiffusion(nn.Module):
     @torch.no_grad()
     def predict_start_from_noise(self, x_t, t, noise):
         """sqrt_recip_alphas_cumprod[t] * x_t - sqrt_recipm1_alphas_cumprod[t] * noise, one kernel."""
-        x = self._f32(x_t)
-        _, x0 = ops.ddpm_step(x, self._timesteps(t, x), self.ddpm_table(), eps=self._f32(noise), want_x_prev=False, want_x0=True)
+        x = _f32_contiguous(x_t)
+        _, x0 = ops.ddpm_step(x, self._timesteps(t, x), self.ddpm_table(), eps=_f32_contiguous(noise), want_x_prev=False, want_x0=True)
         return x0
 
     @torch.no_grad()
     def q_posterior(self, x_start, x_t, t):
         """(posterior mean coef1[t] * x_start + coef2[t] * x_t, posterior_variance[t], posterior_log_variance_clipped[t])."""
-        x = self._f32(x_t)
+        x = _f32_contiguous(x_t)
         t = self._timesteps(t, x)
-        mean, _ = ops.ddpm_step(x, t, self.ddpm_table(), x0=self._f32(x_start))
+        mean, _ = ops.ddpm_step(x, t, self.ddpm_table(), x0=_f32_contiguous(x_start))
         return mean, self._extract(self.posterior_variance, t, x.shape), self._extract(self.posterior_log_variance_clipped, t, x.shape)
 
     def _model_eps(self, x, c, t, score_corrector, corrector_kwargs):
         model_out = self.apply_model(x, t, c)
         if score_corrector is not None:
             model_out = score_corrector.modify_score(self, model_out, x, t, c, **corrector_kwargs)
-        return self._f32(model_out)
+        return _f32_contiguous(model_out)
 
     def _ancestral_update(self, x, t, eps, clip, quantize_denoised, draw=None):
         """x0 -> (clamp) -> (first_stage_model.quantize) -> posterior mean (+ the noise `draw()` returns, drawn after quantize
@@ -492,7 +488,7 @@ class LatentDiffusion(nn.Module):
         table = self.ddpm_table()
         if quantize_denoised:
             _, x0 = ops.ddpm_step(x, t, table, eps=eps, clip=clip, want_x_prev=False, want_x0=True)
-            x0 = self._f32(self.first_stage_model.quantize(x0)[0])
+            x0 = _f32_contiguous(self.first_stage_model.quantize(x0)[0])
             noise, temperature = draw() if draw is not None else (None, 1.)
             x_prev, _ = ops.ddpm_step(x, t, table, x0=x0, noise=noise, temperature=temperature)
             return x_prev, x0
@@ -506,7 +502,7 @@ class LatentDiffusion(nn.Module):
         self._ancestral_supported()
         if return_codebook_ids:
             raise NotImplementedError("return_codebook_ids is not supported")
-        xf = self._f32(x)
+        xf = _f32_contiguous(x)
         t = self._timesteps(t, xf)
         eps = self._model_eps(x, c, t, score_corrector, corrector_kwargs)
         mean, x_recon = self._ancestral_update(xf, t, eps, clip_denoised, quantize_denoised)
@@ -522,7 +518,7 @@ class LatentDiffusion(nn.Module):
         self._ancestral_supported()
         if return_codebook_ids:
             raise NotImplementedError("return_codebook_ids is not supported")
-        xf = self._f32(x)
+        xf = _f32_contiguous(x)
         t = self._timesteps(t, xf)
         eps = self._model_eps(x, c, t, score_corrector, corrector_kwargs)
 

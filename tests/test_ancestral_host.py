@@ -109,3 +109,32 @@ def test_ddpm_step_no_cpu_fallback_and_host_checks():
     assert lib.sdb_ddpm_step(fake, fake, None, None, fake, fake, 0, 1, 1.0, fake, None, 2, 16, None) == -1        # T = 0
     assert lib.sdb_ddpm_step(fake, fake, None, None, fake, fake, 1000, 1, 1.0, fake, None, 0, 16, None) == -1     # B = 0
     assert b"ddpm_step" in lib.sdb_last_error_string()
+
+
+@pytest.fixture(scope="module")
+def lib():
+    import __graft_entry__ as ge
+    ge.build()
+    from sdb200 import _lib
+    return _lib.load()
+
+
+# fake device addresses, 4 KB apart: never dereferenced, the checks reject the call first
+X, EPS, G, NZ, TS, TAB, XP, X0 = (0x100000 + 0x1000 * k for k in range(8))
+B, PER = 2, 8
+N = B * PER
+
+
+def _ddpm(lib, x=X, eps=EPS, x0=None, noise=NZ, xp=XP, x0_out=X0):
+    return lib.sdb_ddpm_step(x, eps, x0, noise, TS, TAB, 1000, 1, 1.0, xp, x0_out, B, PER, None)
+
+
+@pytest.mark.parametrize("case", [
+    dict(xp=X), dict(x0_out=EPS), dict(xp=NZ), dict(eps=None, x0=G, x0_out=G),      # output == input
+    dict(xp=X + 4 * (N - 1)), dict(x0_out=NZ - 4 * (N - 1)),                        # output overlaps an input
+    dict(x0_out=XP), dict(x0_out=XP + 8),                                           # the two outputs overlap
+])
+def test_ddpm_step_outputs_must_not_overlap(lib, case):
+    assert _ddpm(lib, **case) == -1, case
+    err = lib.sdb_last_error_string()
+    assert err.startswith(b"ddpm_step: ") and b"overlap" in err, (case, err)      # rejected by the check, not by a launch

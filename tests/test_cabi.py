@@ -62,3 +62,31 @@ def test_argument_validation_without_gpu(lib):
     assert rc == -1 and b"null" in lib.sdb_last_error_string()
     rc = lib.sdb_ddim_step(None, None, None, 1.0, None, 0.5, 0.6, 0.3, 0.0, 0.7, 1.0, None, None, 0, None)
     assert rc == -1
+
+
+# fake device addresses, 4 KB apart: never dereferenced, the checks reject the call first
+X, E, U, NZ, XP, P0 = (0x100000 + 0x1000 * k for k in range(6))
+N = 16
+
+
+def _ddim_step(lib, x=X, e=E, u=U, noise=NZ, xp=XP, p0=P0):
+    return lib.sdb_ddim_step(x, e, u, 7.5, noise, 0.9, 0.95, 0.3, 0.5, 0.4, 1.0, xp, p0, N, None)
+
+
+def _ddim_xprev(lib, p0=P0, e=E, u=U, noise=NZ, xp=XP):
+    return lib.sdb_ddim_xprev(p0, e, u, 7.5, noise, 0.95, 0.3, 0.5, 1.0, xp, N, None)
+
+
+@pytest.mark.parametrize("entry, call, case", [
+    *[("ddim_step", _ddim_step, c) for c in (
+        dict(xp=X), dict(p0=E), dict(xp=U), dict(p0=NZ),                              # output == input
+        dict(xp=X + 4 * (N - 1)), dict(p0=NZ - 4 * (N - 1)),                          # output overlaps an input
+        dict(p0=XP), dict(p0=XP + 8))],                                               # the two outputs overlap
+    *[("ddim_xprev", _ddim_xprev, c) for c in (
+        dict(xp=P0), dict(xp=E), dict(xp=U), dict(xp=NZ),                             # output == input
+        dict(xp=P0 + 4 * (N - 1)), dict(xp=E - 4 * (N - 1)))],                        # output overlaps an input
+])
+def test_ddim_outputs_must_not_overlap(lib, entry, call, case):
+    assert call(lib, **case) == -1, case
+    err = lib.sdb_last_error_string()
+    assert err.startswith(entry.encode() + b": ") and b"overlap" in err, (case, err)   # rejected by the check, not by a launch

@@ -196,6 +196,26 @@ def test_ddpm_step_kernel_bit_exact(cuda, per_sample):
     assert torch.equal(xp[:1].cpu(), good_xp) and torch.equal(p0[:1].cpu(), good_x0)
 
 
+@pytest.mark.parametrize("per_sample", [(4, 8, 8), (3, 7, 5)])       # VEC = 4 and VEC = 1
+def test_ddpm_step_unread_eps_may_alias_the_output(cuda, per_sample):
+    """With x0_in given the kernel does not read eps, so an eps that is the x_prev buffer is accepted and changes no bit."""
+    from sdb200 import _lib
+    from sdb200._lib import ptr, stream_ptr
+    from sdb200.pipeline import LatentDiffusion
+    lib = _lib.load()
+    table = LatentDiffusion(first_stage_config=False, unet=torch.nn.Linear(1, 1)).cuda().ddpm_table()
+    B = 3
+    x, noise, x0_in = randn(B, *per_sample, seed=1), randn(B, *per_sample, seed=3), randn(B, *per_sample, seed=4, scale=2.0)
+    t = torch.tensor([999, 500, 0], device="cuda")
+    per = x.numel() // B
+    want, got = torch.empty_like(x), torch.full_like(x, 123.0)
+    for eps, out in ((None, want), (got, got)):
+        assert lib.sdb_ddpm_step(ptr(x), ptr(eps), ptr(x0_in), ptr(noise), ptr(t), ptr(table), table.shape[1], 0, 0.7, ptr(out),
+                                 None, B, per, stream_ptr()) == 0, lib.sdb_last_error_string()
+    assert torch.equal(got, want)
+    assert torch.equal(want.cpu(), cpu_step(x.cpu(), t.cpu(), x0=x0_in.cpu(), noise=noise.cpu(), temperature=0.7)[0])
+
+
 # ---- 2. the loops with a stub eps-model ---------------------------------------------------------------------------------
 def test_p_sample_loop_and_progressive_denoising_bit_exact(cuda):
     ld = _toy_ld()

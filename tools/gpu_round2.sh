@@ -47,5 +47,5 @@ cap attn_d80_S1024_Sk77                    tc_attention_kv1 attn 8 8 1024 77 80
 cap attn_wide_d512_S4096                   tc_attention_wide attnw 8 4096 4096 512
 cap gn_cluster_N8_HW4096_C320              gn_ gn 8 4096 320 1
 cap layernorm_rows32768_C320               layernorm_kernel ln 32768 320
-cap ddim_step_n131072                      ddim_step_kernel ddim 131072
+cap ddim_step_n131072                      sampler_update_kernel ddim 131072
 ls gpurun_out/*.raw.csv | wc -l; du -sh gpurun_out
